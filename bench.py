@@ -4,6 +4,7 @@ plus every other named config and the communicating (frame-sharded) path in a `c
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (torchrun launches N ranks)
     python bench.py --impl reference --gpus N --steps K ...  # the unmodified reference on the host CPUs
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's output (see dump_outputs)
 
 Headline: a *step* is one whole griffin_lim job over one batch of synthetic magnitudes,
     griffin_lim(mag, max_iter=64, alpha=0.99, tol=0, eva_iter=10, hop_length=256, window=hann(1024))
@@ -343,6 +344,21 @@ def synth_mag(cx, w, B, seed, length=None):
     return win, mag
 
 
+DUMP_BYTES = 32 << 20
+
+
+def dump_outputs(directory, signal):
+    """--dump-outputs: the signal the last timed step returned, as DIR/signal.npy (float32, one row per signal).  The
+    inputs are seeded, so two builds of the library run with the same arguments can be compared output for output.
+    A batch larger than DUMP_BYTES is sampled: whole rows, drawn with a fixed seed, in ascending order."""
+    os.makedirs(directory, exist_ok=True)
+    y = signal.reshape(-1, signal.shape[-1])
+    B, L = y.shape
+    n = max(1, min(B, DUMP_BYTES // (L * y.element_size())))
+    rows = np.sort(np.random.RandomState(0).choice(B, n, replace=False))
+    np.save(os.path.join(directory, "signal.npy"), y[rows.tolist()].cpu().numpy())
+
+
 def make_job(cx, w, mag, win, loop_ms=None):
     """One whole public call on device-resident input, step by step like methods.griffin_lim / ADMM so that events
     can bracket the iteration loop (-> ms per fused launch)."""
@@ -655,6 +671,8 @@ def run_ours(args, w):
     total_ms = s.elapsed_time(e)
     it_ms = sum(a.elapsed_time(b) for a, b in loop_ms) / (len(loop_ms) * iters)
     sc_gpu = final_sc_db(cx, w, mag, win, y)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, y)
     del y
 
     # ---- e2e through the public API with host buffers: every step timed on its own (host buffers in, host buffers
@@ -663,7 +681,7 @@ def run_ours(args, w):
     for _ in range(max(3, min(args.warmup, 5))):
         yh = job_e2e()      # keep the result alive like the timed loop does (pinned-buffer cache warm)
     cx.barrier()
-    n_e2e = max(args.steps, 5)
+    n_e2e = args.steps
     marks = [cx.ev() for _ in range(n_e2e + 1)]
     marks[0].record()
     for k in range(n_e2e):
@@ -809,7 +827,14 @@ def main():
     ap.add_argument("--configs", default="all", help="extra configs reported in `configs`: all | none | cfg1,cfg3,...")
     ap.add_argument("--batch", type=int, default=0, help="override the per-GPU batch (debugging only)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline / parity / reference_cuda legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the signal the last one returned (a seeded sample of its rows "
+                         "when larger than 32 MiB) to DIR/signal.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what this library's path computed (--impl ours)")
     w = WORKLOADS[args.workload]
     if args.impl == "reference":
         run_reference(args, w)

@@ -172,6 +172,39 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and "workload" in line["config"]
 
 
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--warmup", "-1"],
+                                  ["--impl", "reference", "--dump-outputs", "unused"]])
+def test_bench_rejects_bad_arguments(argv, tmp_path):
+    import subprocess
+    import sys
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *argv], capture_output=True, text=True,
+                       timeout=120, cwd=tmp_path)
+    assert r.returncode == 2 and "error:" in r.stderr, r.stderr[-2000:]
+    assert not (tmp_path / "unused").exists()
+
+
+@pytest.mark.gpu
+def test_bench_dumps_the_same_outputs_on_every_run(tmp_path):
+    """`bench.py --dump-outputs DIR`: the last timed step's signal, a seeded row sample once the batch exceeds
+    32 MiB (40 signals of 239872 samples: 34 rows), identical from run to run; --steps sets the timed steps."""
+    import json
+    import subprocess
+    import sys
+    got = []
+    for run in ("a", "b"):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--batch",
+                            "40", "--configs", "none", "--no-cpu", "--dump-outputs", str(tmp_path / run)],
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads(r.stdout.strip().splitlines()[-1])
+        assert line["steps"] == 2 and len(line["e2e"]["ms_per_step_all"]) == 2
+        assert sorted(os.listdir(tmp_path / run)) == ["signal.npy"]
+        got.append(np.load(tmp_path / run / "signal.npy"))
+    assert got[0].dtype == np.float32 and got[0].shape == (34, 937 * 256)
+    assert np.isfinite(got[0]).all() and np.abs(got[0]).max() > 0
+    assert np.array_equal(got[0], got[1])
+
+
 def test_every_custom_op_has_a_fake_kernel():
     """SURVEY.md section 8b: each specinv_b200:: op carries a register_fake implementation, so FakeTensorMode /
     torch.compile can trace through callers without a device (the ops mutate caller-owned buffers, return nothing)."""
