@@ -238,16 +238,25 @@ def metric_from_sums(name: str, d: float, e: float, g: float) -> float:
 # --------------------------------------------------------------------------- #
 # one-shot phase initialiser (methods.py:572-615)
 # --------------------------------------------------------------------------- #
-def phase_init(mag: np.ndarray, **stft_kwargs) -> np.ndarray:
-    """Simplified SPSI: strict local maxima along freq for 1<=k<=F-2 (:597-598),
-    parabolic offset p (:604), omega = 2 pi (k+p)/n_fft*hop (:605), written to bins
-    k, k-1, k+1 in that order so later writes win (:607-609), cumulative sum over
-    time (:611), C = mag * exp(i phi) (:612-614)."""
-    shape = mag.shape
+def phase_init_phase(mag: np.ndarray, bins: Optional[Tuple[int, int]] = None, **stft_kwargs
+                     ) -> Tuple[np.ndarray, np.ndarray]:
+    """The running phase of ``phase_init`` for a (B, F, T) or (F, T) magnitude: ``(phase, phase_f64)``,
+    the reference's phase rounded to the magnitude's real dtype and the float64 running sum it was
+    rounded from.
+
+    ``bins=(k0, k1)`` computes bins [k0, k1) only, shape (B, k1-k0, T): a bin's frequency comes from
+    peaks at k-1 .. k+1, which look at magnitudes k-2 .. k+2, so only bins [k0-2, k1+2) are read and
+    k stays absolute in omega.  The result equals the same bins of the whole-spectrum call."""
     m = mag[None] if mag.ndim == 2 else mag
     a = args_helper(m.shape[-2], m.dtype, **stft_kwargs)
     rdt = m.dtype
-    phase = np.zeros_like(m)
+    F = m.shape[1]
+    k0, k1 = (0, F) if bins is None else (int(bins[0]), int(bins[1]))
+    assert 0 <= k0 < k1 <= F, (k0, k1, F)
+    lo, hi = max(k0 - 2, 0), min(k1 + 2, F)
+    m = m[:, lo:hi]
+    phase = np.zeros(m.shape, dtype=rdt)
+    # strict local maxima of the window's interior: absolute bins lo+1 .. hi-2, inside 1 .. F-2 (:597-598)
     mask = np.zeros(m.shape, dtype=bool)
     mask[:, 1:-1] = (m[:, 1:-1] > m[:, 2:]) & (m[:, 1:-1] > m[:, :-2])
     i1, i2, i3 = np.nonzero(mask)
@@ -256,13 +265,25 @@ def phase_init(mag: np.ndarray, **stft_kwargs) -> np.ndarray:
     r = m[i1, i2 + 1, i3]
     p = rdt.type(0.5) * (av - r) / (av - rdt.type(2) * b + r)
     # methods.py:605: idx2.float() + p promotes to the dtype of p (= spec dtype)
-    omega = rdt.type(2 * math.pi) * (i2.astype(rdt) + p) / rdt.type(a.n_fft) * rdt.type(a.hop_length)
+    k = (i2 + lo).astype(rdt)
+    omega = rdt.type(2 * math.pi) * (k + p) / rdt.type(a.n_fft) * rdt.type(a.hop_length)
     phase[i1, i2, i3] = omega
     phase[i1, i2 - 1, i3] = omega
     phase[i1, i2 + 1, i3] = omega
     # torch's CPU cumsum accumulates float32 inputs in float64 (acc_type) and rounds every output
-    phase = np.cumsum(phase.astype(np.float64), axis=2).astype(rdt)
-    cdt = np.result_type(rdt, np.complex64)
+    phase_f64 = np.cumsum(phase[:, k0 - lo:k1 - lo].astype(np.float64), axis=2)
+    return phase_f64.astype(rdt), phase_f64
+
+
+def phase_init(mag: np.ndarray, **stft_kwargs) -> np.ndarray:
+    """Simplified SPSI: strict local maxima along freq for 1<=k<=F-2 (:597-598),
+    parabolic offset p (:604), omega = 2 pi (k+p)/n_fft*hop (:605), written to bins
+    k, k-1, k+1 in that order so later writes win (:607-609), cumulative sum over
+    time (:611), C = mag * exp(i phi) (:612-614)."""
+    shape = mag.shape
+    m = mag[None] if mag.ndim == 2 else mag
+    phase, _ = phase_init_phase(m, **stft_kwargs)
+    cdt = np.result_type(m.dtype, np.complex64)
     out = m * np.exp(phase.astype(cdt) * cdt.type(1j))
     return out.reshape(shape)
 

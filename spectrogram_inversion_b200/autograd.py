@@ -119,19 +119,25 @@ class _IstftFn(torch.autograd.Function):
 # ---------------------------------------------------------------------------------------------------------
 def phase_init_diff(spec: torch.Tensor, n_fft: int, hop: int) -> torch.Tensor:
     """phase_init (methods.py:572-615) as dense differentiable tensor expressions: a bin takes the frequency of
-    the peak below it, else of the peak above it, else its own (the reference's write order :607-609)."""
+    the peak below it, else of the peak above it, else its own (the reference's write order :607-609).
+
+    The arithmetic is the reference's CPU arithmetic: a true division by n_fft (a CUDA tensor divided by a
+    Python number is a multiplication by its reciprocal, which differs in the last bit when n_fft is not a
+    power of two), and the running phase summed in float64 and rounded to the input dtype (torch's CPU cumsum
+    accumulates float32 in float64; a float32 sum drifts by radians over a few thousand frames)."""
     lo, mid, hi = spec[:, :-2], spec[:, 1:-1], spec[:, 2:]
     peak = (mid > hi) & (mid > lo)
     den = torch.where(peak, lo - 2 * mid + hi, torch.ones_like(mid))
     p = 0.5 * (lo - hi) / den
     k = torch.arange(1, spec.shape[1] - 1, device=spec.device, dtype=spec.dtype)[None, :, None]
-    own = torch.where(peak, pi2 * (k + p) / n_fft * hop, torch.zeros_like(mid))
+    n = torch.tensor(n_fft, device=spec.device, dtype=spec.dtype)
+    own = torch.where(peak, pi2 * (k + p) / n * hop, torch.zeros_like(mid))
     own = F.pad(own, [0, 0, 1, 1])
     pk = F.pad(peak, [0, 0, 1, 1])
     up, pk_up = F.pad(own[:, 1:], [0, 0, 0, 1]), F.pad(pk[:, 1:], [0, 0, 0, 1])        # the bin above
     dn, pk_dn = F.pad(own[:, :-1], [0, 0, 1, 0]), F.pad(pk[:, :-1], [0, 0, 1, 0])      # the bin below
     omega = torch.where(pk_dn, dn, torch.where(pk_up, up, own))
-    phase = torch.cumsum(omega, 2)
+    phase = torch.cumsum(omega.double(), 2).to(spec.dtype)
     return spec * torch.exp(phase * 1j)
 
 

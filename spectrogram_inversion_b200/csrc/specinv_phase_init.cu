@@ -12,8 +12,8 @@
 namespace specinv {
 
 template <typename T> __device__ __forceinline__ void sincos_t(T x, T* s, T* c);
-// The running phase reaches 1e5..1e6 rad (omega = pi/2 * k per frame at hop = n_fft/4), far into the slow
-// (Payne-Hanek) range of sincosf.  The float phase is exactly representable in double, so reduce it modulo 2 pi
+// The running phase reaches 1e5..1e6 rad (omega = pi/2 * k per frame at hop = n_fft/4), ~5e8 rad after one hour at
+// n_fft = 4096: far into the slow (Payne-Hanek) range of sincosf.  The float phase is exactly representable in double, so reduce it modulo 2 pi
 // there (two-term 2 pi, error < 1e-10 rad) and take the fast path on the remainder.
 template <> __device__ __forceinline__ void sincos_t<float>(float x, float* s, float* c) {
     const double xd = (double)x;
@@ -45,8 +45,11 @@ __device__ __forceinline__ T mag_at(const T* __restrict__ main, const T* __restr
 //   scan  : an exclusive scan over the chunks of every (signal, bin), in place;
 //   MODE 2: the warp reads ITS start phase from that slot and then writes C for its frames (the slot is overwritten
 //           by the first of them).
-// The double accumulation is then associated per chunk instead of strictly left to right: ~1e-16 relative, which
-// the rounding of the phase to the real type absorbs.
+// The double accumulation is then associated per chunk instead of strictly left to right.  For float32 magnitudes
+// that changes nothing: the omegas of one bin come from peaks at k-1 .. k+1 and lie within a factor 7 of each other,
+// so every partial sum is a multiple of the smallest float ulp u among them and below 7 * 2^24 * T * u: exact in
+// double for T < 2^26, and the chunked phase is bit-identical to the left-to-right sum.  In float64 the sums re-associate
+// (<= T * 2^-53 * |phi|).
 constexpr int PI_SEG = 30;
 
 template <typename T>
@@ -54,9 +57,12 @@ __device__ __forceinline__ double* chunk_slot(const Dims& dm, cx_t<T>* c_main, c
     return reinterpret_cast<double*>((dm.onesided && k == dm.M) ? c_nyq + fr : c_main + fr * dm.row + k);
 }
 
-template <typename T, int MODE>
+// POW2: n_fft is a power of two, where x * (1 / n_fft) IS the IEEE quotient x / n_fft (1 / n_fft is exact); the
+// division costs 6 % of the kernel's time at cfg2 (1.73 vs 1.63 ms on a B200 at 1000 W), so it is only paid where
+// it changes the result.
+template <typename T, int MODE, bool POW2>
 __global__ void __launch_bounds__(128) phase_init_kernel(Dims dm, int F, int segs, int chunks, int chunk_len, T hop,
-                                                         T inv_n_fft, const T* __restrict__ mag_main,
+                                                         T n_fft, const T* __restrict__ mag_main,
                                                          const T* __restrict__ mag_nyq, cx_t<T>* __restrict__ c_main,
                                                          cx_t<T>* __restrict__ c_nyq, const double* __restrict__ phase_in,
                                                          double* __restrict__ phase_out) {
@@ -72,6 +78,7 @@ __global__ void __launch_bounds__(128) phase_init_kernel(Dims dm, int F, int seg
     const bool owner = in_spec && lane >= 1 && lane <= PI_SEG;
     const bool can_peak = k >= 1 && k <= F - 2;       // strict local maxima exist for 1 <= k <= F-2 only (:597-598)
     const T pi2 = (T)6.283185307179586476925286766559;
+    const T inv_n_fft = T(1) / n_fft;                  // exact when POW2
     // torch's CPU cumsum accumulates float32 in float64 and rounds each output; phase_in (frame-range
     // sharding) is the phase accumulated by the frames before this range
     double phase = 0.0;
@@ -94,11 +101,12 @@ __global__ void __launch_bounds__(128) phase_init_kernel(Dims dm, int F, int seg
                 const long long fr = (long long)b * dm.T + t0 + u;
                 const T lo = m[u][0], mid = m[u][1], hi = m[u][2];
                 // own peak: interpolated angular frequency * hop (:604-605), or -1 (omega is never negative).
-                // x / n_fft == x * (1 / n_fft) exactly: n_fft is a power of two.
+                // The operations and their order are the reference's: 2 pi * (k + p), an IEEE division by n_fft
+                // (a multiplication by 1 / n_fft differs in the last bit when n_fft is not a power of two), * hop.
                 T own = T(-1);
                 if (can_peak && mid > hi && mid > lo) {
                     const T p = T(0.5) * (lo - hi) / (lo - T(2) * mid + hi);
-                    own = pi2 * ((T)k + p) * inv_n_fft * hop;
+                    own = POW2 ? pi2 * ((T)k + p) * inv_n_fft * hop : pi2 * ((T)k + p) / n_fft * hop;
                 }
                 const T up = __shfl_down_sync(0xffffffffu, own, 1);      // bin k + 1
                 const T dn = __shfl_up_sync(0xffffffffu, own, 1);        // bin k - 1
@@ -149,6 +157,24 @@ __global__ void spec_abs_kernel(const cx_t<T>* __restrict__ c, T* __restrict__ m
     }
 }
 
+template <typename T, bool POW2>
+static void phase_init_launch(const Dims& dm, int F, int segs, long long chunks, int chunk_len, long long blocks,
+                              const T* mm, const T* mn, cx_t<T>* cm, cx_t<T>* cn, const double* phase_in,
+                              double* phase_out, cudaStream_t st) {
+    const T hop = (T)dm.hop, n_fft = (T)dm.N;
+    if (chunks == 1) {
+        phase_init_kernel<T, 0, POW2><<<(unsigned)blocks, 128, 0, st>>>(dm, F, segs, 1, dm.T, hop, n_fft, mm, mn, cm, cn,
+                                                                        phase_in, phase_out);
+    } else {
+        phase_init_kernel<T, 1, POW2><<<(unsigned)blocks, 128, 0, st>>>(dm, F, segs, (int)chunks, chunk_len, hop, n_fft, mm,
+                                                                        mn, cm, cn, nullptr, nullptr);
+        const long long nbf = (long long)dm.B * F;
+        phase_scan_kernel<T><<<(unsigned)((nbf + 127) / 128), 128, 0, st>>>(dm, F, (int)chunks, chunk_len, cm, cn, phase_in);
+        phase_init_kernel<T, 2, POW2><<<(unsigned)blocks, 128, 0, st>>>(dm, F, segs, (int)chunks, chunk_len, hop, n_fft, mm,
+                                                                        mn, cm, cn, nullptr, phase_out);
+    }
+}
+
 template <typename T>
 static int phase_init_t(const Dims& dm, const void* mag_main, const void* mag_nyq, void* c_main, void* c_nyq,
                         const double* phase_in, double* phase_out, cudaStream_t st) {
@@ -164,20 +190,12 @@ static int phase_init_t(const Dims& dm, const void* mag_main, const void* mag_ny
     chunks = (dm.T + chunk_len - 1) / chunk_len;
     const long long blocks = (pairs * chunks + 3) / 4;                  // 4 warps per block
     if (blocks > 0x7fffffffLL) return SPECINV_ERR_UNSUPPORTED;
-    const T hop = (T)dm.hop, inv_n = (T)(1.0 / dm.N);
     const T* mm = (const T*)mag_main; const T* mn = (const T*)mag_nyq;
     cx_t<T>* cm = (cx_t<T>*)c_main; cx_t<T>* cn = (cx_t<T>*)c_nyq;
-    if (chunks == 1) {
-        phase_init_kernel<T, 0><<<(unsigned)blocks, 128, 0, st>>>(dm, F, segs, 1, dm.T, hop, inv_n, mm, mn, cm, cn, phase_in,
-                                                                  phase_out);
-    } else {
-        phase_init_kernel<T, 1><<<(unsigned)blocks, 128, 0, st>>>(dm, F, segs, (int)chunks, chunk_len, hop, inv_n, mm, mn, cm,
-                                                                  cn, nullptr, nullptr);
-        const long long nbf = (long long)dm.B * F;
-        phase_scan_kernel<T><<<(unsigned)((nbf + 127) / 128), 128, 0, st>>>(dm, F, (int)chunks, chunk_len, cm, cn, phase_in);
-        phase_init_kernel<T, 2><<<(unsigned)blocks, 128, 0, st>>>(dm, F, segs, (int)chunks, chunk_len, hop, inv_n, mm, mn, cm,
-                                                                  cn, nullptr, phase_out);
-    }
+    if ((dm.N & (dm.N - 1)) == 0)
+        phase_init_launch<T, true>(dm, F, segs, chunks, chunk_len, blocks, mm, mn, cm, cn, phase_in, phase_out, st);
+    else
+        phase_init_launch<T, false>(dm, F, segs, chunks, chunk_len, blocks, mm, mn, cm, cn, phase_in, phase_out, st);
     return (int)cudaGetLastError();
 }
 
