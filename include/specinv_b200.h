@@ -166,6 +166,41 @@ int specinv_rtisi_la_steps(const specinv_desc* d, const void* plan, const void* 
                            int max_iter, double alpha, double synth_coeff, int step_begin, int step_end, void* state,
                            void* stream);
 
+/* Streaming RTISI-LA: the same outer steps on magnitude frames that arrive a few at a time, with windows of frames and
+ * samples instead of whole-signal buffers, so neither the final frame count T nor the output length L is needed
+ * before the last call.  d->n_frames = frames received so far (the total when `final`); pad_mode is not used.
+ *   magnitudes  mag_main [B][n_rows][row], mag_nyq [B][n_rows]: row r of a signal is frame frame0 + r.  The rows must
+ *               reach from max(0, step_begin - LA) -- a resume re-reads the LA older active frames -- to the newest
+ *               frame the steps read, min(step_end, n_frames) - 1; frame0 <= max(0, step_begin - LA).
+ *   x_out       [B][x_len]: column c of a signal is output sample x0 + c.  The window must be exactly the samples
+ *               these steps finish: the commit of step i finishes [(i-LA)*hop - P, (i-LA+1)*hop - P) (P = n_fft/2 when
+ *               centred, else 0; clamped at 0), and a final call also finishes everything up to L = (n_frames-1)*hop
+ *               + n_fft - 2P.  Without `final` the window is not clamped at L: samples past L(n_frames) are final as
+ *               values but belong to the signal only if more frames follow (the caller holds them back).
+ *   inv_env     [x_len]: 1/envelope of samples [x0, x0 + x_len) (specinv_plan_inv_env_window).
+ *   plan        any plan of this n_fft / hop / window / normalized / onesided / dtype: only its T-independent
+ *               tables are read.
+ *   steps       [step_begin, step_end): step i reads frame i, so step_end <= n_frames without `final` and
+ *               step_end <= n_frames + LA with it.  Only the final call may be empty (step_begin == step_end ==
+ *               n_frames + LA, look_ahead = 0): it releases the carry the commit of frame n_frames-1 left behind.
+ *   final       0/1: n_frames is the total; frames past it have zero magnitude (methods.py:339), the commit of frame
+ *               n_frames-1 flushes the whole carry and no state is saved after step n_frames + LA.
+ *   state       as for specinv_rtisi_la_steps (its bytes do not depend on n_frames); always required.
+ * Every argument is checked before any launch (SPECINV_ERR_INVALID).  The kernel is chosen as for specinv_rtisi_la,
+ * and the concatenated windows of any sequence of calls are bit-identical to one specinv_rtisi_la run. */
+int specinv_rtisi_la_stream(const specinv_desc* d, const void* plan, const void* window, const void* mag_main,
+                            const void* mag_nyq, int frame0, int n_rows, void* x_out, const void* inv_env, int64_t x0,
+                            int64_t x_len, void* scratch, int look_ahead, int asymmetric_window, int max_iter,
+                            double alpha, double synth_coeff, int step_begin, int step_end, int final, void* state,
+                            void* stream);
+/* out[j] = 1/envelope of sample x0 + j of a signal with total_frames frames (< 0: not known yet; then only samples
+ * whose covering frames all exist may be asked for), gathered from a plan of d->n_frames = T0 frames.  The envelope
+ * sums w^2 over the covering frames in ascending order, so a sample's value depends only on (m + P) mod hop and on
+ * which end clips its frame range: head, interior and tail of any signal are bitwise equal to the plan's.  Needs
+ * (T0 - 1) * hop >= n_fft, and total_frames >= T0 or < 0; total_frames == T0 reads the plan as it is. */
+int specinv_plan_inv_env_window(const specinv_desc* d, const void* plan, int64_t x0, int64_t len,
+                                int64_t total_frames, void* out, void* stream);
+
 /* ---- frame-range sharding helpers (single long signal over several GPUs) --------------------------
  * specinv_halo_sum    : out = left + right over rows x n strided views -- the per-iteration combination of
  *                       the two partial overlap-add sums of the (n_fft - hop)-sample region two neighbouring

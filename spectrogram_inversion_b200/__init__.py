@@ -3,7 +3,8 @@ phase-retrieval hot path of torch_specinv 0.2.1 (griffin_lim, RTISI_LA, ADMM, sc
 from . import methods, metrics
 from .methods import ADMM, L_BFGS, RTISI_LA, griffin_lim, phase_init
 from .metrics import sc, ser, snr, spectral_convergence
+from .streaming import RTISIStream
 
 __version__ = "0.1.0"
-__all__ = ["griffin_lim", "RTISI_LA", "ADMM", "L_BFGS", "phase_init", "sc", "snr", "ser", "spectral_convergence",
+__all__ = ["griffin_lim", "RTISI_LA", "RTISIStream", "ADMM", "L_BFGS", "phase_init", "sc", "snr", "ser", "spectral_convergence",
            "methods", "metrics"]

@@ -27,7 +27,7 @@ EXPORTS = (
     "specinv_halo_area_bytes", "specinv_ipc_alloc", "specinv_ipc_open", "specinv_ipc_close", "specinv_ipc_free",
     "specinv_halo_exchange", "specinv_halo_status",
     "specinv_gl_run_workspace_bytes", "specinv_gl_run", "specinv_gl_run_status",
-    "specinv_rtisi_state_bytes", "specinv_rtisi_la_steps",
+    "specinv_rtisi_state_bytes", "specinv_rtisi_la_steps", "specinv_rtisi_la_stream", "specinv_plan_inv_env_window",
 )
 
 
@@ -75,6 +75,9 @@ def _declare(lib: C.CDLL) -> None:
         "specinv_rtisi_la": [dp, vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, dbl, dbl, vp],
         "specinv_rtisi_state_bytes": [dp, C.c_int, C.POINTER(C.c_size_t)],
         "specinv_rtisi_la_steps": [dp, vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, dbl, dbl, C.c_int, C.c_int, vp, vp],
+        "specinv_rtisi_la_stream": [dp, vp, vp, vp, vp, C.c_int, C.c_int, vp, vp, i64, i64, vp, C.c_int, C.c_int, C.c_int,
+                                    dbl, dbl, C.c_int, C.c_int, C.c_int, vp, vp],
+        "specinv_plan_inv_env_window": [dp, vp, i64, i64, i64, vp, vp],
         "specinv_stft": [dp, vp, vp, vp, vp, vp],
         "specinv_istft": [dp, vp, vp, vp, vp, vp],
         "specinv_gl_iter": [dp, vp, vp, vp, vp, vp, vp, vp, vp, vp, dbl, vp, vp],

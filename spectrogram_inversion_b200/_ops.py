@@ -201,6 +201,34 @@ def rtisi_la_steps(plan: Tensor, window: Tensor, mag_main: Tensor, mag_nyq: Tens
                                               _stream(x_out)), "rtisi_la_steps", 2)
 
 
+@torch.library.custom_op("specinv_b200::rtisi_la_stream", mutates_args=("x_out", "scratch", "state"), device_types="cuda")
+def rtisi_la_stream(plan: Tensor, window: Tensor, mag_main: Tensor, mag_nyq: Tensor, x_out: Tensor, inv_env: Tensor,
+                    scratch: Tensor, state: Tensor, n_frames: int, frame0: int, x0: int, look_ahead: int,
+                    asymmetric: bool, max_iter: int, alpha: float, synth_coeff: float, step_begin: int, step_end: int,
+                    final: bool, n_fft: int, hop: int, center: bool, normalized: bool, onesided: bool) -> None:
+    """Outer steps [step_begin, step_end) of a stream of `n_frames` frames so far: magnitude rows (B, n_rows, .) are
+    frames frame0 + r, x_out (B, x_len) and inv_env (x_len,) are samples x0 + c (include/specinv_b200.h)."""
+    _need_cuda(plan, window, mag_main, mag_nyq, x_out, inv_env, scratch, state)
+    d = _desc(x_out, n_fft, hop, n_frames, x_out.shape[0], center, 1, normalized, onesided)
+    with torch.cuda.device(x_out.device):
+        _ok(_lib.lib().specinv_rtisi_la_stream(
+            C.byref(d), _p(plan), _p(window), _p(mag_main), _p(mag_nyq), int(frame0), mag_main.shape[1], _p(x_out),
+            _p(inv_env), int(x0), x_out.shape[1], _p(scratch), int(look_ahead), int(bool(asymmetric)), int(max_iter),
+            float(alpha), float(synth_coeff), int(step_begin), int(step_end), int(bool(final)), _p(state),
+            _stream(x_out)), "rtisi_la_stream", 2)
+
+
+def plan_inv_env_window(plan: Tensor, out: Tensor, x0: int, total_frames: int, n_fft: int, hop: int, n_frames: int,
+                        center: bool, normalized: bool, onesided: bool) -> None:
+    """out[j] = 1/envelope of sample x0 + j of a signal of total_frames frames (-1: not known yet), from a plan of
+    n_frames frames (specinv_plan_inv_env_window)."""
+    _need_cuda(plan, out)
+    d = _desc(out, n_fft, hop, n_frames, 1, center, 1, normalized, onesided)
+    with torch.cuda.device(plan.device):
+        _ok(_lib.lib().specinv_plan_inv_env_window(C.byref(d), _p(plan), int(x0), out.numel(), int(total_frames),
+                                                   _p(out), _stream(plan)), "plan_inv_env_window")
+
+
 def rtisi_state_bytes(ref: Tensor, n_fft: int, hop: int, n_frames: int, batch: int, normalized: bool, onesided: bool,
                       look_ahead: int) -> int:
     d = _desc(ref, n_fft, hop, n_frames, batch, False, 0, normalized, onesided)
@@ -273,3 +301,14 @@ ALL_OPS = (plan_init, stft, istft, gl_iter, admm_iter, pack, unpack, metric_sums
 for _op in ALL_OPS:
     _op.register_fake(_fake_iter if _op in (gl_iter, admm_iter) else _fake_nothing)
 del _op
+
+
+def _fake_rtisi_la_stream(plan, window, mag_main, mag_nyq, x_out, inv_env, *rest) -> None:
+    if x_out.dim() != 2 or inv_env.shape != (x_out.shape[1],) or mag_main.shape[0] != x_out.shape[0]:
+        raise RuntimeError("specinv_b200: rtisi_la_stream window shapes disagree")
+    return None
+
+
+# the streaming entry (spectrogram_inversion_b200.streaming)
+STREAM_OPS = (rtisi_la_stream,)
+rtisi_la_stream.register_fake(_fake_rtisi_la_stream)

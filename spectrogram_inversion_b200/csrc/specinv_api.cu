@@ -87,6 +87,26 @@ __global__ void plan_envelope_kernel(Dims dm, long long frame_offset, long long 
     inv_env[m] = T(1) / acc;
 }
 
+// 1/envelope of samples [x0, x0 + len) of a signal of `total` frames (total < 0: not known yet, only samples whose
+// covering frames have all been seen are asked for), read from a plan of T0 = dm.T frames.  The envelope kernel above
+// sums w^2 over the covering frames in ascending order, so a sample's value depends only on (m + P) mod hop and on
+// whether its frame range is clipped by the first or by the last frame: the head of the signal is the plan's head,
+// the tail (total >= T0) the plan's tail, and every interior sample equals the plan's interior sample at the same
+// phase.  T0 must satisfy (T0 - 1) * hop >= n_fft unless total == T0.
+template <typename T>
+__global__ void inv_env_window_kernel(Dims dm, const T* __restrict__ inv_env, long long x0, long long len,
+                                      long long total, T* __restrict__ out) {
+    const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= len) return;
+    const long long pp = x0 + j + dm.P;                       // position in the padded signal
+    long long q;
+    if (total == dm.T) q = pp;
+    else if (total >= 0 && pp >= total * dm.hop) q = pp - (total - dm.T) * dm.hop;   // clipped by the last frame
+    else if (pp < dm.N) q = pp;                                                       // clipped by the first frame
+    else q = dm.N + (pp - dm.N) % dm.hop;                                             // interior
+    out[j] = inv_env[q - dm.P];
+}
+
 template <typename T>
 static int plan_init_t(const Dims& dm, const specinv_desc* d, const void* window, void* plan, long long frame_offset,
                        long long total_frames, cudaStream_t st) {
@@ -305,6 +325,29 @@ int specinv_plan_envelope(const specinv_desc* d, const void* plan, void* env_out
     const size_t es = d->dtype == SPECINV_F64 ? 8 : 4;
     return (int)cudaMemcpyAsync(env_out, (const char*)plan + pl.env, (size_t)dm.L * es, cudaMemcpyDeviceToDevice,
                                 (cudaStream_t)stream);
+}
+
+int specinv_plan_inv_env_window(const specinv_desc* d, const void* plan, int64_t x0, int64_t len,
+                                int64_t total_frames, void* out, void* stream) {
+    Dims dm; int rc = make_dims(d, &dm); if (rc) return rc;
+    if (!plan || (len > 0 && !out) || x0 < 0 || len < 0) return SPECINV_ERR_INVALID;
+    if (total_frames != dm.T) {
+        if (total_frames >= 0 && total_frames < dm.T) return SPECINV_ERR_INVALID;    // use a plan of total_frames
+        if ((long long)(dm.T - 1) * dm.hop < dm.N) return SPECINV_ERR_INVALID;       // head and tail would overlap
+        if (total_frames >= 0 && x0 + len > (total_frames - 1) * dm.hop + dm.N - 2LL * dm.P) return SPECINV_ERR_INVALID;
+    } else if (x0 + len > dm.L) {
+        return SPECINV_ERR_INVALID;
+    }
+    if (len == 0) return SPECINV_OK;
+    const PlanLayout pl = plan_layout(dm, d->dtype);
+    const unsigned blocks = (unsigned)((len + 255) / 256);
+    if (d->dtype == SPECINV_F64)
+        inv_env_window_kernel<double><<<blocks, 256, 0, (cudaStream_t)stream>>>(
+            dm, (const double*)((const char*)plan + pl.inv_env), x0, len, total_frames, (double*)out);
+    else
+        inv_env_window_kernel<float><<<blocks, 256, 0, (cudaStream_t)stream>>>(
+            dm, (const float*)((const char*)plan + pl.inv_env), x0, len, total_frames, (float*)out);
+    return (int)cudaGetLastError();
 }
 
 int specinv_plan_unit_envelope(const specinv_desc* d, void* plan, void* stream) {

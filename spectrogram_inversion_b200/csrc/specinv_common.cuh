@@ -78,6 +78,15 @@ struct PlanLayout {
     size_t total;
 };
 
+// Where one RTISI-LA launch reads its magnitudes and writes its samples (include/specinv_b200.h:
+// specinv_rtisi_la_stream).  A whole-signal run is frame0 = 0, n_rows = T, x0 = 0, x_len = L, final = 1.
+struct RtisiWindow {
+    int frame0, n_rows;       // magnitude row r of a signal is spectrogram frame frame0 + r
+    long long x0, x_len;      // x_out column c of a signal is output sample x0 + c; x_len is also the row stride
+    const void* inv_env;      // 1/envelope of samples [x0, x0 + x_len), shared by the batch
+    int final;                // n_frames is the total: zero magnitudes past it, the last frame flushes the carry
+};
+
 inline int ilog2(int v) { int l = 0; while ((1 << l) < v) ++l; return l; }
 
 inline int make_dims(const specinv_desc* d, Dims* o) {

@@ -24,8 +24,8 @@ namespace specinv {
 
 // implemented in specinv_rtisi_fast.cu; returns SPECINV_ERR_UNSUPPORTED when the shape is not its own
 int rtisi_fast(const specinv_desc* d, const Dims& dm, const void* plan, const void* mag_main, const void* mag_nyq,
-               void* x_out, const void* asym1, const void* asym2, int look_ahead, int asymmetric, int max_iter,
-               double alpha, double synth_coeff, int step_begin, int step_end, void* state, cudaStream_t st);
+               void* x_out, const RtisiWindow& win, const void* asym1, const void* asym2, int look_ahead, int asymmetric,
+               int max_iter, double alpha, double synth_coeff, int step_begin, int step_end, void* state, cudaStream_t st);
 
 // Elements (of the real type) of the sliding state of ONE signal between two outer steps, the layout both kernels
 // save / restore (include/specinv_b200.h: specinv_rtisi_la_steps): active frames [NA][N] (logical order, oldest
@@ -39,7 +39,8 @@ size_t rtisi_state_elems(const Dims& dm, int LA) {
 struct RtisiArgs {
     const void* mag_main; const void* mag_nyq;
     void* x_out;
-    const void* tw; const void* twr; const void* wa; const void* ws; const void* inv_env;
+    const void* tw; const void* twr; const void* wa; const void* ws;
+    RtisiWindow win;                          // magnitude / output / 1/envelope windows
     const void* asym1; const void* asym2;     // analysis windows of the newest frame (already * forward scale)
     double synth_coeff;                       // c = hop / (w . w)
     double lr;                                // alpha / (1 + alpha)
@@ -79,8 +80,9 @@ __global__ void __launch_bounds__(256) rtisi_kernel(const RtisiArgs a) {
     const T* asym2 = (const T*)a.asym2;
     const T* mag_main = (const T*)a.mag_main;
     const T* mag_nyq = (const T*)a.mag_nyq;
-    const T* ienv = (const T*)a.inv_env;
-    T* xo = (T*)a.x_out + (long long)b * dm.L;
+    const T* ienv = (const T*)a.win.inv_env;
+    const long long x0 = a.win.x0, x1 = a.win.x0 + a.win.x_len;
+    T* xo = (T*)a.x_out + (long long)b * a.win.x_len;
     const T coef = (T)a.synth_coeff, lr = (T)a.lr;
     T* workf = reinterpret_cast<T*>(work);
     for (int k = tid; k < M; k += NT)
@@ -105,7 +107,7 @@ __global__ void __launch_bounds__(256) rtisi_kernel(const RtisiArgs a) {
     // magnitude of bin kk of spectrogram frame t (zero outside [0, T): the reference pads with zeros, :339)
     auto mag_of = [&](int t, int kk) -> T {
         if (t < 0 || t >= dm.T) return T(0);
-        const long long fr = (long long)b * dm.T + t;
+        const long long fr = (long long)b * a.win.n_rows + (t - a.win.frame0);
         if (dm.onesided && kk == M) return mag_nyq[fr];
         return mag_main[fr * dm.row + kk];
     };
@@ -245,11 +247,11 @@ __global__ void __launch_bounds__(256) rtisi_kernel(const RtisiArgs a) {
             const int t = i - LA;                               // index of the committed frame in the output OLA
             for (int n = tid; n < N; n += NT) carry[n] += wsample(s0, n) * ws[n];
             __syncthreads();
-            const bool last = t == dm.T - 1;
+            const bool last = a.win.final && t == dm.T - 1;
             const int nout = last ? N : hop;                    // the last frame flushes the whole carry
             for (int n = tid; n < nout; n += NT) {
                 const long long m = (long long)t * hop + n - dm.P;
-                if (m >= 0 && m < dm.L) xo[m] = carry[n] * ienv[m];
+                if (m >= x0 && m < x1) xo[m - x0] = carry[n] * ienv[m - x0];
             }
             __syncthreads();
             if (!last) {
@@ -274,7 +276,15 @@ __global__ void __launch_bounds__(256) rtisi_kernel(const RtisiArgs a) {
         for (int n = tid; n < Mp; n += NT) work[(size_t)s0 * Mp + n] = mk<T>(T(0), T(0));
         __syncthreads();
     }
-    if (a.state && a.step_end < dm.T + LA) {
+    if (a.step_begin == a.step_end) {
+        // a final launch with no step left (look_ahead = 0, frame T-1 committed by an earlier launch): release the
+        // carry that commit shifted by one hop -- the values its flush would have written
+        for (int n = tid; n < N - hop; n += NT) {
+            const long long m = (long long)dm.T * hop + n - dm.P;
+            if (m >= x0 && m < x1) xo[m - x0] = carry[n] * ienv[m - x0];
+        }
+    }
+    if (a.state && !(a.win.final && a.step_end == dm.T + LA)) {
         // ---- save the state before outer step step_end (logical order; the newest frame's momentum is not used)
         for (int idx = tid; idx < NA * N; idx += NT) {
             const int aa = idx / N, n = idx - aa * N;
@@ -314,12 +324,13 @@ __global__ void rtisi_windows_kernel(int N, int hop, int K, const T* __restrict_
 
 template <typename T>
 static int rtisi_t(const specinv_desc* d, const Dims& dm, const void* plan, const void* window, const void* mag_main,
-                   const void* mag_nyq, void* x_out, void* scratch, int look_ahead, int asymmetric, int max_iter,
-                   double alpha, double synth_coeff, int step_begin, int step_end, void* state, cudaStream_t st) {
+                   const void* mag_nyq, void* x_out, const RtisiWindow& win, void* scratch, int look_ahead, int asymmetric,
+                   int max_iter, double alpha, double synth_coeff, int step_begin, int step_end, void* state,
+                   cudaStream_t st) {
     RtisiArgs a{};
     const PlanLayout pl = plan_layout(dm, d->dtype);
     const char* p = (const char*)plan;
-    a.tw = p + pl.tw; a.twr = p + pl.twr; a.wa = p + pl.wa; a.ws = p + pl.ws; a.inv_env = p + pl.inv_env;
+    a.tw = p + pl.tw; a.twr = p + pl.twr; a.wa = p + pl.wa; a.ws = p + pl.ws; a.win = win;
     a.dm = dm;
     a.LA = look_ahead < 0 ? dm.K : look_ahead;
     a.max_iter = max_iter; a.asymmetric = asymmetric;
@@ -344,8 +355,8 @@ static int rtisi_t(const specinv_desc* d, const Dims& dm, const void* plan, cons
         // the register-FFT kernel of specinv_rtisi_fast.cu covers n_fft = 1024 / hop = 256 / look_ahead <= 3
         const char* fg = getenv("SPECINV_FORCE_GENERIC");
         if (!(fg && fg[0] == '1')) {
-            const int rf = rtisi_fast(d, dm, plan, mag_main, mag_nyq, x_out, asym, asym + dm.N, look_ahead, asymmetric,
-                                      max_iter, alpha, synth_coeff, step_begin, step_end, state, st);
+            const int rf = rtisi_fast(d, dm, plan, mag_main, mag_nyq, x_out, win, asym, asym + dm.N, look_ahead,
+                                      asymmetric, max_iter, alpha, synth_coeff, step_begin, step_end, state, st);
             if (rf != SPECINV_ERR_UNSUPPORTED) return rf;
         }
     }
@@ -386,11 +397,64 @@ int specinv_rtisi_la_steps(const specinv_desc* d, const void* plan, const void* 
     const int steps = dm.T + (look_ahead < 0 ? dm.K : look_ahead);
     if (step_begin < 0 || step_end > steps || step_begin >= step_end) return SPECINV_ERR_INVALID;
     if ((step_begin > 0 || step_end < steps) && !state) return SPECINV_ERR_INVALID;
+    // the whole signal is the window: every launch addresses all T frames and all L samples
+    const RtisiWindow win{0, dm.T, 0, dm.L, (const char*)plan + plan_layout(dm, d->dtype).inv_env, 1};
     return d->dtype == SPECINV_F64
-               ? rtisi_t<double>(d, dm, plan, window, mag_main, mag_nyq, x_out, scratch, look_ahead, asymmetric_window,
-                                 max_iter, alpha, synth_coeff, step_begin, step_end, state, (cudaStream_t)stream)
-               : rtisi_t<float>(d, dm, plan, window, mag_main, mag_nyq, x_out, scratch, look_ahead, asymmetric_window,
-                                max_iter, alpha, synth_coeff, step_begin, step_end, state, (cudaStream_t)stream);
+               ? rtisi_t<double>(d, dm, plan, window, mag_main, mag_nyq, x_out, win, scratch, look_ahead,
+                                 asymmetric_window, max_iter, alpha, synth_coeff, step_begin, step_end, state,
+                                 (cudaStream_t)stream)
+               : rtisi_t<float>(d, dm, plan, window, mag_main, mag_nyq, x_out, win, scratch, look_ahead,
+                                asymmetric_window, max_iter, alpha, synth_coeff, step_begin, step_end, state,
+                                (cudaStream_t)stream);
+}
+
+int specinv_rtisi_la_stream(const specinv_desc* d, const void* plan, const void* window, const void* mag_main,
+                            const void* mag_nyq, int frame0, int n_rows, void* x_out, const void* inv_env, int64_t x0,
+                            int64_t x_len, void* scratch, int look_ahead, int asymmetric_window, int max_iter,
+                            double alpha, double synth_coeff, int step_begin, int step_end, int final, void* state,
+                            void* stream) {
+    if (!d || d->n_frames < 1) return SPECINV_ERR_INVALID;
+    // RTISI-LA never pads, and one centred frame has no output sample yet (L = 0), which make_dims refuses for a
+    // whole signal: derive the dimensions as for two frames, then put the real frame count back
+    specinv_desc dd = *d;
+    dd.pad_mode = SPECINV_PAD_CONSTANT;
+    if (dd.n_frames < 2) dd.n_frames = 2;
+    Dims dm; int rc = make_dims(&dd, &dm); if (rc) return rc;
+    dm.T = d->n_frames;
+    dm.Lp = (long long)(dm.T - 1) * dm.hop + dm.N;
+    dm.L = dm.Lp - 2LL * dm.P;
+    if (!plan || !window || !scratch || !state) return SPECINV_ERR_INVALID;
+    if (n_rows > 0 && (!mag_main || (dm.onesided && !mag_nyq))) return SPECINV_ERR_INVALID;
+    if (x_len > 0 && (!x_out || !inv_env)) return SPECINV_ERR_INVALID;
+    if (max_iter < 1 || alpha < 0 || (final != 0 && final != 1)) return SPECINV_ERR_INVALID;
+    const int LA = look_ahead < 0 ? dm.K : look_ahead;
+    // steps: step i reads frame i, so a launch that is not final stops at the frames pushed so far
+    if (step_begin < 0 || step_end > dm.T + (final ? LA : 0)) return SPECINV_ERR_INVALID;
+    // an empty range only as the final launch that releases the carry left by an earlier commit of frame T-1
+    if (step_begin > step_end || (step_begin == step_end && !(final && step_end == dm.T + LA))) return SPECINV_ERR_INVALID;
+    // magnitude rows: from the oldest frame a resume re-reads up to the newest one a step reads
+    const int need0 = step_begin - LA > 0 ? step_begin - LA : 0;
+    const int need1 = step_end < dm.T ? step_end : dm.T;
+    if (frame0 < 0 || n_rows < 0 || frame0 > need0 || (long long)frame0 + n_rows > dm.T || frame0 + n_rows < need1)
+        return SPECINV_ERR_INVALID;
+    // samples: exactly those these steps finish (the commit of step i finishes [(i-LA)*hop - P, (i-LA+1)*hop - P);
+    // the final launch also finishes everything up to L)
+    auto block_end = [&](long long i) { const long long e = (i - LA) * dm.hop - dm.P; return e > 0 ? e : 0LL; };
+    long long lo = block_end(step_begin), hi = block_end(step_end);
+    if (final) {
+        const long long L = dm.L > 0 ? dm.L : 0;
+        lo = lo < L ? lo : L;
+        hi = step_end == dm.T + LA || hi > L ? L : hi;
+    }
+    if (x0 != lo || x_len != hi - lo) return SPECINV_ERR_INVALID;
+    const RtisiWindow win{frame0, n_rows, x0, x_len, inv_env, final};
+    return d->dtype == SPECINV_F64
+               ? rtisi_t<double>(d, dm, plan, window, mag_main, mag_nyq, x_out, win, scratch, look_ahead,
+                                 asymmetric_window, max_iter, alpha, synth_coeff, step_begin, step_end, state,
+                                 (cudaStream_t)stream)
+               : rtisi_t<float>(d, dm, plan, window, mag_main, mag_nyq, x_out, win, scratch, look_ahead,
+                                asymmetric_window, max_iter, alpha, synth_coeff, step_begin, step_end, state,
+                                (cudaStream_t)stream);
 }
 
 int specinv_rtisi_la(const specinv_desc* d, const void* plan, const void* window, const void* mag_main,

@@ -35,12 +35,13 @@ struct RArgs {
     const float* mag; const float* mag_nyq;
     float* x_out;
     const float2* tw; const float2* twr;
-    const float* wa; const float* ws; const float* inv_env;
+    const float* wa; const float* ws; const float* inv_env;   // inv_env: samples [x0, x0 + x_len)
     const float* asym1; const float* asym2;   // analysis windows of the newest frame (already x forward scale)
     float coef;                               // c = hop / (w . w)
     float lr;                                 // alpha / (1 + alpha)
     int B, T, P, LA, max_iter, asymmetric;
-    long long L;
+    int frame0, n_rows, final;                // magnitude window and whether T is the total (RtisiWindow)
+    long long x0, x_len;                      // output window: x_out column c of a signal is sample x0 + c
     int step_begin, step_end;                 // outer steps [step_begin, step_end) of the T + LA steps of a run
     float* state;                             // per-signal sliding state in / out (specinv_rtisi.cu: rtisi_state_elems)
     size_t state_elems;
@@ -202,7 +203,7 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
         const int bar_id = 1 + sig;
         const int hi_adj = l == 0 ? -(RC - 1) * LANES : 0;
         const Bins bin{l, l + hi_adj, M - l, M - l - hi_adj, l == 0 ? M / 2 : M - l};
-        float* xo = a.x_out + (long long)b * a.L;
+        float* xo = a.x_out + (long long)b * a.x_len - a.x0;     // indexed by absolute sample
 
         // ---- everything zero (methods.py:353-358)
         float2 v[V];
@@ -245,10 +246,10 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
                 const int t_frame = a.step_begin + la0 - a.LA;
                 float mg[V];
                 const bool inside = t_frame >= 0 && t_frame < a.T;
-                const float* mrow = a.mag + ((long long)b * a.T + (inside ? t_frame : 0)) * M;
+                const float* mrow = a.mag + ((long long)b * a.n_rows + (inside ? t_frame - a.frame0 : 0)) * M;
 #pragma unroll
                 for (int e = 0; e < V; ++e) mg[e] = inside ? __ldg(mrow + bin(e)) : 0.f;
-                mag_nyq = (inside && l == 0) ? __ldg(a.mag_nyq + (long long)b * a.T + t_frame) : 0.f;
+                mag_nyq = (inside && l == 0) ? __ldg(a.mag_nyq + (long long)b * a.n_rows + t_frame - a.frame0) : 0.f;
                 tmem_stw<V>(twarp + TC_MAG, mg);
             }
             const float2* kp = reinterpret_cast<const float2*>(st_kept);
@@ -267,10 +268,10 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
                 // a new frame is born in this warp: fetch its magnitude row (zero outside the spectrogram, :339)
                 float mg[V];
                 const bool inside = t_frame >= 0 && t_frame < a.T;
-                const float* mrow = a.mag + ((long long)b * a.T + (inside ? t_frame : 0)) * M;
+                const float* mrow = a.mag + ((long long)b * a.n_rows + (inside ? t_frame - a.frame0 : 0)) * M;
 #pragma unroll
                 for (int e = 0; e < V; ++e) mg[e] = inside ? __ldg(mrow + bin(e)) : 0.f;
-                mag_nyq = (inside && l == 0) ? __ldg(a.mag_nyq + (long long)b * a.T + t_frame) : 0.f;
+                mag_nyq = (inside && l == 0) ? __ldg(a.mag_nyq + (long long)b * a.n_rows + t_frame - a.frame0) : 0.f;
                 tmem_stw<V>(twarp + TC_MAG, mg);
                 if (i == 0) {
                     // zero-phase start: the newest frame = irfft(first magnitude frame + 0j) (:353-358)
@@ -490,15 +491,15 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
                         const float2 w = s_ws[r * LANES + l];
                         c[r] = pfma(v[r], w, carry[r * LANES + l]);
                     }
-                    const bool last = t == a.T - 1;                 // the last frame flushes the whole carry
+                    const bool last = a.final && t == a.T - 1;      // the last frame flushes the whole carry
 #pragma unroll
                     for (int k = 0; k < 4; ++k) {
                         if (k == 0 || last) {
                             const long long m0 = (long long)(t + k) * HOP - a.P;
-                            if (m0 >= 0 && m0 + HOP <= a.L) {
+                            if (m0 >= a.x0 && m0 + HOP <= a.x0 + a.x_len) {
 #pragma unroll
                                 for (int r = 0; r < HP; ++r) {
-                                    const float2 ie = __ldg(reinterpret_cast<const float2*>(a.inv_env + m0 + 2 * LANES * r + 2 * l));
+                                    const float2 ie = __ldg(reinterpret_cast<const float2*>(a.inv_env + (m0 - a.x0) + 2 * LANES * r + 2 * l));
                                     const float2 val = c[HP * k + r];
                                     *reinterpret_cast<float2*>(xo + m0 + 2 * LANES * r + 2 * l) = pmul(val, ie);
                                 }
@@ -523,7 +524,22 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
             kslot = (kslot + 1) % KEEP;
             sig_sync<LANES>(bar_id, NA);              // the kept ring and the carry are in place for the next step
         }
-        if (a.state && a.step_end < a.T + a.LA) {
+        if (a.step_begin == a.step_end && p == 0) {
+            // a final launch with no step left (look_ahead = 0, frame T-1 committed by an earlier launch): release
+            // the carry that commit shifted by one hop -- the blocks k = 1 .. 3 its flush would have written
+#pragma unroll
+            for (int k = 0; k < 3; ++k) {
+                const long long m0 = (long long)(a.T + k) * HOP - a.P;
+                if (m0 >= a.x0 && m0 + HOP <= a.x0 + a.x_len) {
+#pragma unroll
+                    for (int r = 0; r < HP; ++r) {
+                        const float2 ie = __ldg(reinterpret_cast<const float2*>(a.inv_env + (m0 - a.x0) + 2 * LANES * r + 2 * l));
+                        *reinterpret_cast<float2*>(xo + m0 + 2 * LANES * r + 2 * l) = pmul(carry[(HP * k + r) * LANES + l], ie);
+                    }
+                }
+            }
+        }
+        if (a.state && !(a.final && a.step_end == a.T + a.LA)) {
             // ---- save the state before outer step step_end
             int la1 = (p - a.step_end) % NA; if (la1 < 0) la1 += NA;
             float2* fr = reinterpret_cast<float2*>(st_frames + (size_t)la1 * N);
@@ -567,8 +583,8 @@ static int launch(const RArgs& a, cudaStream_t st) {
 
 // Returns SPECINV_ERR_UNSUPPORTED when the shape is not the one this kernel is specialised for.
 int rtisi_fast(const specinv_desc* d, const Dims& dm, const void* plan, const void* mag_main, const void* mag_nyq,
-               void* x_out, const void* asym1, const void* asym2, int look_ahead, int asymmetric, int max_iter,
-               double alpha, double synth_coeff, int step_begin, int step_end, void* state, cudaStream_t st) {
+               void* x_out, const RtisiWindow& win, const void* asym1, const void* asym2, int look_ahead, int asymmetric,
+               int max_iter, double alpha, double synth_coeff, int step_begin, int step_end, void* state, cudaStream_t st) {
     if (d->dtype != SPECINV_F32 || !d->onesided || d->hop * 4 != d->n_fft ||
         (d->n_fft != 2048 && d->n_fft != 1024 && d->n_fft != 512))
         return SPECINV_ERR_UNSUPPORTED;
@@ -578,11 +594,12 @@ int rtisi_fast(const specinv_desc* d, const Dims& dm, const void* plan, const vo
     const PlanLayout pl = plan_layout(dm, d->dtype);
     const char* p = (const char*)plan;
     a.tw = (const float2*)(p + pl.tw); a.twr = (const float2*)(p + pl.twr);
-    a.wa = (const float*)(p + pl.wa); a.ws = (const float*)(p + pl.ws); a.inv_env = (const float*)(p + pl.inv_env);
+    a.wa = (const float*)(p + pl.wa); a.ws = (const float*)(p + pl.ws); a.inv_env = (const float*)win.inv_env;
     a.asym1 = (const float*)asym1; a.asym2 = (const float*)asym2;
     a.mag = (const float*)mag_main; a.mag_nyq = (const float*)mag_nyq; a.x_out = (float*)x_out;
     a.coef = (float)synth_coeff; a.lr = (float)(alpha / (1.0 + alpha));
-    a.B = dm.B; a.T = dm.T; a.P = dm.P; a.LA = LA; a.max_iter = max_iter; a.asymmetric = asymmetric; a.L = dm.L;
+    a.B = dm.B; a.T = dm.T; a.P = dm.P; a.LA = LA; a.max_iter = max_iter; a.asymmetric = asymmetric;
+    a.frame0 = win.frame0; a.n_rows = win.n_rows; a.final = win.final; a.x0 = win.x0; a.x_len = win.x_len;
     a.step_begin = step_begin; a.step_end = step_end; a.state = (float*)state;
     a.state_elems = (size_t)(LA + 1) * dm.N + 2 * (size_t)(LA + 1) * (dm.M + 1) + (size_t)dm.K * dm.N + dm.N;
     // Signals per CTA: as few as still fit the batch into one wave of CTAs (the kernel is latency-bound, so a signal

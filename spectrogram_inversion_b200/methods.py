@@ -264,19 +264,26 @@ def ADMM(spec, max_iter=1000, tol=1e-6, rho=0.1, verbose=1, eva_iter=10, metric=
     return _finish(solver.signal, spec)
 
 
-def RTISI_LA(spec, look_ahead=-1, asymmetric_window=False, max_iter=25, alpha=0.99, verbose=1, **stft_kwargs):
-    r"""Real-Time Iterative Spectrogram Inversion with Look-Ahead (drop-in for
-    ``torch_specinv.RTISI_LA``, methods.py:273-412)."""
+def _rtisi_checks(spec, max_iter, alpha, asymmetric_window, stft_kwargs) -> None:
+    """The argument checks of RTISI_LA, shared with RTISIStream (``spec`` None: the options only)."""
     assert max_iter > 0
     assert alpha >= 0
-    assert not spec.is_complex()
-    assert 4 > len(spec.shape) > 1
+    if spec is not None:
+        assert not spec.is_complex()
+        assert 4 > len(spec.shape) > 1
     if not asymmetric_window:
         # the reference hands the caller's kwargs to torch.stft on this path (methods.py:308-310, :385), so an unknown
         # key is a TypeError there (griffin_lim / ADMM and the asymmetric path silently ignore it, :42-46)
         for key in stft_kwargs:
             if key not in _TORCH_STFT_KEYS:
                 raise TypeError(f"stft() got an unexpected keyword argument '{key}'")
+
+
+def RTISI_LA(spec, look_ahead=-1, asymmetric_window=False, max_iter=25, alpha=0.99, verbose=1, **stft_kwargs):
+    r"""Real-Time Iterative Spectrogram Inversion with Look-Ahead (drop-in for
+    ``torch_specinv.RTISI_LA``, methods.py:273-412).  ``RTISIStream`` runs the same algorithm on frames that
+    arrive a few at a time."""
+    _rtisi_checks(spec, max_iter, alpha, asymmetric_window, stft_kwargs)
     if autograd.wants_grad(spec):
         work, args = _diff_setup(spec, stft_kwargs)
         return _diff_finish(autograd.rtisi_diff(work, args, look_ahead, asymmetric_window, max_iter, alpha, verbose), spec)
