@@ -133,6 +133,14 @@ int specinv_istft(const specinv_desc* d, const void* plan, const void* main_in, 
 int specinv_gl_iter(const specinv_desc* d, const void* plan, const void* x_in, void* x_out,
                     const void* q_in_main, const void* q_in_nyq, void* q_out_main, void* q_out_nyq,
                     const void* mag_main, const void* mag_nyq, double lr, double* sums, void* stream);
+/* specinv_gl_rebuilt_iter : one loop pass of torchaudio.functional.griffinlim, whose fast Griffin-Lim takes the
+ *   momentum on the previous REBUILT spectrum instead of the previous momentum spectrum:
+ *      s = STFT(x_in); s_out = s; a = s - m*s_in; x_out = ISTFT(mag*a/(|a|+1e-16))      (m = momentum/(1+momentum))
+ *   Arguments, aliasing rules, the NULL-state plain Griffin-Lim case (all four s pointers NULL, m = 0: the same kernel
+ *   as specinv_gl_iter's) and `sums` as for specinv_gl_iter.  A zero s_in makes the first pass s_out = s, a = s. */
+int specinv_gl_rebuilt_iter(const specinv_desc* d, const void* plan, const void* x_in, void* x_out,
+                            const void* s_in_main, const void* s_in_nyq, void* s_out_main, void* s_out_nyq,
+                            const void* mag_main, const void* mag_nyq, double m, double* sums, void* stream);
 int specinv_admm_iter(const specinv_desc* d, const void* plan, const void* x_in, void* x_out,
                       const void* X_in_main, const void* X_in_nyq, const void* U_in_main, const void* U_in_nyq,
                       void* X_out_main, void* X_out_nyq, void* U_out_main, void* U_out_nyq,

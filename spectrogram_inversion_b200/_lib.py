@@ -28,6 +28,7 @@ EXPORTS = (
     "specinv_halo_exchange", "specinv_halo_status",
     "specinv_gl_run_workspace_bytes", "specinv_gl_run", "specinv_gl_run_status",
     "specinv_rtisi_state_bytes", "specinv_rtisi_la_steps", "specinv_rtisi_la_stream", "specinv_plan_inv_env_window",
+    "specinv_gl_rebuilt_iter",
 )
 
 
@@ -81,6 +82,7 @@ def _declare(lib: C.CDLL) -> None:
         "specinv_stft": [dp, vp, vp, vp, vp, vp],
         "specinv_istft": [dp, vp, vp, vp, vp, vp],
         "specinv_gl_iter": [dp, vp, vp, vp, vp, vp, vp, vp, vp, vp, dbl, vp, vp],
+        "specinv_gl_rebuilt_iter": [dp, vp, vp, vp, vp, vp, vp, vp, vp, vp, dbl, vp, vp],
         "specinv_admm_iter": [dp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, dbl, vp, vp],
         "specinv_metric_sums": [C.c_int, vp, vp, i64, vp, vp],
     }

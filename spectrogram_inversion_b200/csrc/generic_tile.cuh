@@ -6,7 +6,9 @@
 
 namespace specinv {
 
-enum { OP_STFT = 0, OP_ISTFT = 1, OP_GL = 2, OP_ADMM = 3 };
+// OP_GLR: fast Griffin-Lim with the momentum on the previous rebuilt spectrum (torchaudio.functional.griffinlim):
+// state out = s, projection of s - lr * s_prev
+enum { OP_STFT = 0, OP_ISTFT = 1, OP_GL = 2, OP_ADMM = 3, OP_GLR = 4 };
 
 struct TileArgs {
     const void* x_in;
@@ -63,7 +65,7 @@ __device__ __forceinline__ BinIn<T> bin_load(const TileArgs& a, const IO& io, in
     in.s0 = mk<T>(T(0), T(0)); in.s1 = in.s0; in.m = T(0);
     if constexpr (OP == OP_ISTFT) {
         in.s0 = io.ldc(a.s0_in_main, a.s0_in_nyq, kk);
-    } else if constexpr (OP == OP_GL) {
+    } else if constexpr (OP == OP_GL || OP == OP_GLR) {
         in.m = io.ldm(kk);
         if (a.s0_in_main != nullptr) in.s0 = io.ldc(a.s0_in_main, a.s0_in_nyq, kk);
     } else if constexpr (OP == OP_ADMM) {
@@ -82,15 +84,18 @@ __device__ __forceinline__ cx_t<T> bin_apply(const TileArgs& a, const IO& io, in
         return s;
     } else if constexpr (OP == OP_ISTFT) {
         return in.s0;
-    } else if constexpr (OP == OP_GL) {
-        // methods.py:243-247
+    } else if constexpr (OP == OP_GL || OP == OP_GLR) {
+        // methods.py:243-247 (OP_GLR: torchaudio's griffinlim, the state is s itself)
         const T lr = (T)a.coef;
         const bool momentum = a.s0_in_main != nullptr;     // NULL state: plain Griffin-Lim (lr == 0), q_n = s
         const T m = in.m;
+        if constexpr (OP == OP_GLR) {       // the state is s: store it before q is formed (fewer live registers)
+            if (owned && momentum) io.stc(a.s0_out_main, a.s0_out_nyq, kk, s);
+        }
         cx_t<T> q = s;
         if (momentum) q = mk<T>(s.x - in.s0.x * lr, s.y - in.s0.y * lr);
         if (owned) {
-            if (momentum) io.stc(a.s0_out_main, a.s0_out_nyq, kk, q);
+            if (OP == OP_GL && momentum) io.stc(a.s0_out_main, a.s0_out_nyq, kk, q);
             if (want_sums) {
                 T r = fast_sqrt(s.x * s.x + s.y * s.y);
                 dsum += (r - m) * (r - m);

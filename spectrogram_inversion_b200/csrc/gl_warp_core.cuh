@@ -31,8 +31,10 @@ namespace specinv {
 namespace wfast {
 
 // OP_ISTFT: stand-alone inverse transform + overlap-add (methods.py:233); OP_GLP: plain Griffin-Lim (alpha = 0:
-// q_n = STFT(x_{n-1}), so no momentum state is read or written)
-enum { OP_GL = 0, OP_ADMM = 1, OP_ISTFT = 2, OP_GLP = 3 };
+// q_n = STFT(x_{n-1}), so no momentum state is read or written); OP_GLR: fast Griffin-Lim with the momentum taken on
+// the previous REBUILT spectrum (torchaudio.functional.griffinlim): the state is s = STFT(x_{n-1}) itself, the
+// projection gets s - m s_prev.  Same traffic as OP_GL, only the stored value differs.
+enum { OP_GL = 0, OP_ADMM = 1, OP_ISTFT = 2, OP_GLP = 3, OP_GLR = 4 };
 
 // complex products on the packed FP32x2 pipe (fft_regs.cuh): 2 instructions each
 SPX_HD float2 cmulf(float2 a, float2 b) { return cmul2(a, b); }
@@ -227,6 +229,9 @@ SPX_HD float2 bin_update(float2 s, float2 a0, float2 a1, float m, float coef, fl
         const float2 q = pfma(f2(-coef, -coef), a0, s);             // s - lr * q_prev
         o0 = q;
         return project_rsq(q, m);
+    } else if constexpr (OP == OP_GLR) {
+        o0 = s;                                                     // state: the rebuilt spectrum
+        return project_rsq(pfma(f2(-coef, -coef), a0, s), m);       // s - m * s_prev
     } else {
         const float rho = coef, inv = coef2;
         const float2 XU = a0 + a1;

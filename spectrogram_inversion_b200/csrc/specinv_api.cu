@@ -25,12 +25,16 @@ int generic_stft(const specinv_desc*, const void*, const void*, void*, void*, vo
 int generic_istft(const specinv_desc*, const void*, const void*, const void*, void*, void*);
 int generic_gl_iter(const specinv_desc*, const void*, const void*, void*, const void*, const void*, void*, void*,
                     const void*, const void*, double, double*, void*);
+int generic_gl_rebuilt_iter(const specinv_desc*, const void*, const void*, void*, const void*, const void*, void*, void*,
+                            const void*, const void*, double, double*, void*);
 int generic_admm_iter(const specinv_desc*, const void*, const void*, void*, const void*, const void*, const void*,
                       const void*, void*, void*, void*, void*, const void*, const void*, double, double*, void*);
 // implemented in specinv_fastw.cu (the specialised kernels); return SPECINV_ERR_UNSUPPORTED when not applicable
 
 int fastw_gl_iter(const specinv_desc*, const void*, const void*, void*, const void*, const void*, void*, void*,
                   const void*, const void*, double, double*, void*);
+int fastw_gl_rebuilt_iter(const specinv_desc*, const void*, const void*, void*, const void*, const void*, void*, void*,
+                          const void*, const void*, double, double*, void*);
 int fastw_admm_iter(const specinv_desc*, const void*, const void*, void*, const void*, const void*, const void*,
                     const void*, void*, void*, void*, void*, const void*, const void*, double, double*, void*);
 int fastw_istft(const specinv_desc*, const void*, const void*, const void*, void*, void*);
@@ -424,6 +428,24 @@ int specinv_gl_iter(const specinv_desc* d, const void* plan, const void* x_in, v
     }
     return generic_gl_iter(d, plan, x_in, x_out, q_in_main, q_in_nyq, q_out_main, q_out_nyq, mag_main, mag_nyq, lr,
                            sums, stream);
+}
+
+int specinv_gl_rebuilt_iter(const specinv_desc* d, const void* plan, const void* x_in, void* x_out,
+                            const void* s_in_main, const void* s_in_nyq, void* s_out_main, void* s_out_nyq,
+                            const void* mag_main, const void* mag_nyq, double m, double* sums, void* stream) {
+    // without state (m == 0) the update is plain Griffin-Lim, exactly what specinv_gl_iter runs then
+    if (!s_in_main && !s_out_main)
+        return specinv_gl_iter(d, plan, x_in, x_out, nullptr, s_in_nyq, nullptr, s_out_nyq, mag_main, mag_nyq, m, sums,
+                               stream);
+    if (!d || !plan || !x_in || !x_out || !mag_main || x_in == x_out) return SPECINV_ERR_INVALID;
+    if (!s_in_main || !s_out_main || s_in_main == s_out_main) return SPECINV_ERR_INVALID;
+    if (!force_generic() && d->onesided && s_in_nyq && s_out_nyq && mag_nyq) {
+        const int rc = fastw_gl_rebuilt_iter(d, plan, x_in, x_out, s_in_main, s_in_nyq, s_out_main, s_out_nyq, mag_main,
+                                             mag_nyq, m, sums, stream);
+        if (rc != SPECINV_ERR_UNSUPPORTED) return rc;
+    }
+    return generic_gl_rebuilt_iter(d, plan, x_in, x_out, s_in_main, s_in_nyq, s_out_main, s_out_nyq, mag_main, mag_nyq, m,
+                                   sums, stream);
 }
 
 int specinv_admm_iter(const specinv_desc* d, const void* plan, const void* x_in, void* x_out,

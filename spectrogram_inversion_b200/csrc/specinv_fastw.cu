@@ -31,9 +31,10 @@ static void fill_common(wfast::WArgs& a, const Dims& dm, const specinv_desc* d, 
 }
 
 // Return SPECINV_ERR_UNSUPPORTED when the shape is not one these kernels are specialised for.
-int fastw_gl_iter(const specinv_desc* d, const void* plan, const void* x_in, void* x_out,
-                  const void* q_in_main, const void* q_in_nyq, void* q_out_main, void* q_out_nyq,
-                  const void* mag_main, const void* mag_nyq, double lr, double* sums, void* stream) {
+// op = OP_GL (state q = s - lr q_prev) or OP_GLR (state = the rebuilt spectrum s, the projection gets s - lr s_prev).
+static int fastw_momentum_iter(int op, const specinv_desc* d, const void* plan, const void* x_in, void* x_out,
+                               const void* q_in_main, const void* q_in_nyq, void* q_out_main, void* q_out_nyq,
+                               const void* mag_main, const void* mag_nyq, double lr, double* sums, void* stream) {
     if (!fastw_applicable(d)) return SPECINV_ERR_UNSUPPORTED;
     Dims dm; int rc = make_dims(d, &dm); if (rc) return rc;
     wfast::WArgs a{};
@@ -43,7 +44,21 @@ int fastw_gl_iter(const specinv_desc* d, const void* plan, const void* x_in, voi
     a.s0_out = (float2*)q_out_main; a.s0_out_nyq = (float2*)q_out_nyq;
     a.mag = (const float*)mag_main; a.mag_nyq = (const float*)mag_nyq;
     a.coef = (float)lr; a.sums = sums;
-    return wfast::launch_op(wfast::OP_GL, a, d, (cudaStream_t)stream);
+    return wfast::launch_op(op, a, d, (cudaStream_t)stream);
+}
+
+int fastw_gl_iter(const specinv_desc* d, const void* plan, const void* x_in, void* x_out,
+                  const void* q_in_main, const void* q_in_nyq, void* q_out_main, void* q_out_nyq,
+                  const void* mag_main, const void* mag_nyq, double lr, double* sums, void* stream) {
+    return fastw_momentum_iter(wfast::OP_GL, d, plan, x_in, x_out, q_in_main, q_in_nyq, q_out_main, q_out_nyq, mag_main,
+                               mag_nyq, lr, sums, stream);
+}
+
+int fastw_gl_rebuilt_iter(const specinv_desc* d, const void* plan, const void* x_in, void* x_out,
+                          const void* s_in_main, const void* s_in_nyq, void* s_out_main, void* s_out_nyq,
+                          const void* mag_main, const void* mag_nyq, double m, double* sums, void* stream) {
+    return fastw_momentum_iter(wfast::OP_GLR, d, plan, x_in, x_out, s_in_main, s_in_nyq, s_out_main, s_out_nyq,
+                               mag_main, mag_nyq, m, sums, stream);
 }
 
 // Plain Griffin-Lim (alpha = 0, methods.py:243 with lr = 0): x_out = ISTFT(proj(STFT(x_in))), no momentum state.

@@ -579,6 +579,7 @@ static int launch_any(const WArgs& a, int n_fft, cudaStream_t st) {
             case OP_ADMM: return launch_any<OP_ADMM, OV>(a, n_fft, st);                        \
             case OP_ISTFT: return launch_any<OP_ISTFT, OV>(a, n_fft, st);                      \
             case OP_GLP: return launch_any<OP_GLP, OV>(a, n_fft, st);                          \
+            case OP_GLR: return launch_any<OP_GLR, OV>(a, n_fft, st);                          \
             default: return SPECINV_ERR_INVALID;                                               \
         }                                                                                      \
     }

@@ -112,7 +112,7 @@ __global__ void __launch_bounds__(1024) tile_kernel(const TileArgs a) {
         }
     }
 
-    if constexpr (OP == OP_GL || OP == OP_ADMM) {
+    if constexpr (OP == OP_GL || OP == OP_GLR || OP == OP_ADMM) {
         if (want_sums) {   // fused metric epilogue: block reduce, one double atomic pair per CTA
             __shared__ double red[2][32];
             double d = (double)dsum, e = (double)esum;
@@ -226,7 +226,7 @@ __global__ void __launch_bounds__(512) dft_tile_kernel(const TileArgs a) {
         }
         hb[idx] = h;
     }
-    if constexpr (OP == OP_GL || OP == OP_ADMM) {
+    if constexpr (OP == OP_GL || OP == OP_GLR || OP == OP_ADMM) {
         if (want_sums) {
             __shared__ double red[2][32];
             double d = (double)dsum, e = (double)esum;
@@ -398,9 +398,10 @@ int generic_istft(const specinv_desc* d, const void* plan, const void* main_in, 
     return dispatch<OP_ISTFT>(d->dtype, a, (cudaStream_t)stream);
 }
 
-int generic_gl_iter(const specinv_desc* d, const void* plan, const void* x_in, void* x_out,
-                    const void* q_in_main, const void* q_in_nyq, void* q_out_main, void* q_out_nyq,
-                    const void* mag_main, const void* mag_nyq, double lr, double* sums, void* stream) {
+// rebuilt = false: specinv_gl_iter (OP_GL); true: specinv_gl_rebuilt_iter (OP_GLR, the state is the rebuilt spectrum)
+static int generic_momentum_iter(bool rebuilt, const specinv_desc* d, const void* plan, const void* x_in, void* x_out,
+                                 const void* q_in_main, const void* q_in_nyq, void* q_out_main, void* q_out_nyq,
+                                 const void* mag_main, const void* mag_nyq, double lr, double* sums, void* stream) {
     Dims dm; int rc = make_dims(d, &dm); if (rc) return rc;
     if (!plan || !x_in || !x_out || !mag_main || x_in == x_out) return SPECINV_ERR_INVALID;
     if (!q_in_main != !q_out_main || (!q_in_main && lr != 0.0)) return SPECINV_ERR_INVALID;
@@ -410,7 +411,23 @@ int generic_gl_iter(const specinv_desc* d, const void* plan, const void* x_in, v
     a.x_in = x_in; a.x_out = x_out;
     a.s0_in_main = q_in_main; a.s0_in_nyq = q_in_nyq; a.s0_out_main = q_out_main; a.s0_out_nyq = q_out_nyq;
     a.mag_main = mag_main; a.mag_nyq = mag_nyq; a.coef = lr; a.sums = sums;
+    // without state both ops are plain Griffin-Lim: one kernel serves them
+    if (rebuilt && q_in_main) return dispatch<OP_GLR>(d->dtype, a, (cudaStream_t)stream);
     return dispatch<OP_GL>(d->dtype, a, (cudaStream_t)stream);
+}
+
+int generic_gl_iter(const specinv_desc* d, const void* plan, const void* x_in, void* x_out,
+                    const void* q_in_main, const void* q_in_nyq, void* q_out_main, void* q_out_nyq,
+                    const void* mag_main, const void* mag_nyq, double lr, double* sums, void* stream) {
+    return generic_momentum_iter(false, d, plan, x_in, x_out, q_in_main, q_in_nyq, q_out_main, q_out_nyq, mag_main,
+                                 mag_nyq, lr, sums, stream);
+}
+
+int generic_gl_rebuilt_iter(const specinv_desc* d, const void* plan, const void* x_in, void* x_out,
+                            const void* s_in_main, const void* s_in_nyq, void* s_out_main, void* s_out_nyq,
+                            const void* mag_main, const void* mag_nyq, double m, double* sums, void* stream) {
+    return generic_momentum_iter(true, d, plan, x_in, x_out, s_in_main, s_in_nyq, s_out_main, s_out_nyq, mag_main,
+                                 mag_nyq, m, sums, stream);
 }
 
 int generic_admm_iter(const specinv_desc* d, const void* plan, const void* x_in, void* x_out,

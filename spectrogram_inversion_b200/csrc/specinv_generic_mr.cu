@@ -226,7 +226,7 @@ __global__ void __launch_bounds__(sizeof(T) == 8 ? 256 : 512, 2) mr_tile_kernel(
         }
     }
 
-    if constexpr (OP == OP_GL || OP == OP_ADMM) {
+    if constexpr (OP == OP_GL || OP == OP_GLR || OP == OP_ADMM) {
         if (want_sums) {   // fused metric epilogue: warp reduce, one double atomic pair per warp
             double d = (double)dsum, e = (double)esum;
             for (int o = 16; o > 0; o >>= 1) {
@@ -371,6 +371,7 @@ static int launch_mr_op(int op, TileArgs& a, const mr::Plan& mp, cudaStream_t st
         case OP_STFT:  return launch_mr<T, OP_STFT>(a, mp, st);
         case OP_ISTFT: return launch_mr<T, OP_ISTFT>(a, mp, st);
         case OP_GL:    return launch_mr<T, OP_GL>(a, mp, st);
+        case OP_GLR:   return launch_mr<T, OP_GLR>(a, mp, st);
         case OP_ADMM:  return launch_mr<T, OP_ADMM>(a, mp, st);
         default:       return SPECINV_ERR_INVALID;
     }
