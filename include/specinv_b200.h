@@ -257,6 +257,17 @@ int specinv_gl_run(const specinv_desc* d, const void* plan, const void* x_in, vo
                    double* sums, void* workspace, void* stream);
 int specinv_gl_run_status(const specinv_desc* d, const void* workspace, uint32_t* status, void* stream);
 
+/* ---- torchaudio's InverseMelScale (csrc/specinv_mel.cu, spectrogram_inversion_b200.torchaudio_compat) -----------
+ * out[b, f, t] = relu(sum_j P[f, j] * mel[b, j, t]) for f in [f_lo, f_hi), and 0 for every other f (no multiply).
+ *   P    [n_stft][n_mels] row-major: pinv(fb^T), the minimum-norm least-squares operator of the mel filterbank; its
+ *        rows outside [f_lo, f_hi) must be zero (bins no filter covers).  Not read when f_lo == f_hi.
+ *   mel  [batch][n_mels][n_frames] contiguous;  out [batch][n_stft][n_frames] contiguous (torchaudio's layout).
+ * relu is torch.relu's: NaN stays NaN.  Any n_stft >= 1, n_mels >= 1 (the kernel tiles over n_mels); FFMA in fp32,
+ * DFMA in fp64, summed over j in ascending order.  Every argument is checked before any launch (SPECINV_ERR_INVALID:
+ * dtype, sizes, 0 <= f_lo <= f_hi <= n_stft, NULL pointers); n_frames == 0 launches nothing. */
+int specinv_mel_inverse(int dtype, const void* P, int n_stft, int n_mels, int f_lo, int f_hi, const void* mel,
+                        void* out, int batch, int64_t n_frames, void* stream);
+
 /* ---- metrics (metrics.py:4-43, F.mse_loss at methods.py:182) ---------------------------------
  * out[0] += sum (a-b)^2, out[1] += sum a^2, out[2] += sum b^2 over n contiguous reals. */
 int specinv_metric_sums(int dtype, const void* a, const void* b, int64_t n, double* out3, void* stream);

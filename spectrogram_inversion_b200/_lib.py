@@ -28,7 +28,7 @@ EXPORTS = (
     "specinv_halo_exchange", "specinv_halo_status",
     "specinv_gl_run_workspace_bytes", "specinv_gl_run", "specinv_gl_run_status",
     "specinv_rtisi_state_bytes", "specinv_rtisi_la_steps", "specinv_rtisi_la_stream", "specinv_plan_inv_env_window",
-    "specinv_gl_rebuilt_iter",
+    "specinv_gl_rebuilt_iter", "specinv_mel_inverse",
 )
 
 
@@ -85,6 +85,7 @@ def _declare(lib: C.CDLL) -> None:
         "specinv_gl_rebuilt_iter": [dp, vp, vp, vp, vp, vp, vp, vp, vp, vp, dbl, vp, vp],
         "specinv_admm_iter": [dp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, dbl, vp, vp],
         "specinv_metric_sums": [C.c_int, vp, vp, i64, vp, vp],
+        "specinv_mel_inverse": [C.c_int, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, C.c_int, i64, vp],
     }
     for name, args in sigs.items():
         fn = getattr(lib, name)

@@ -312,3 +312,45 @@ def _fake_rtisi_la_stream(plan, window, mag_main, mag_nyq, x_out, inv_env, *rest
 # the streaming entry (spectrogram_inversion_b200.streaming)
 STREAM_OPS = (rtisi_la_stream,)
 rtisi_la_stream.register_fake(_fake_rtisi_la_stream)
+
+
+def _check_mel_inverse(P: Tensor, mel: Tensor, out: Tensor, f_lo: int, f_hi: int) -> None:
+    if P.dim() != 2 or mel.dim() != 3 or out.dim() != 3:
+        raise RuntimeError("specinv_b200: mel_inverse needs P (n_stft, n_mels), mel (B, n_mels, T), out (B, n_stft, T)")
+    F, M = P.shape
+    if tuple(mel.shape[:2]) != (out.shape[0], M) or tuple(out.shape[1:]) != (F, mel.shape[2]):
+        raise RuntimeError(f"specinv_b200: mel_inverse shapes disagree: P {list(P.shape)}, mel {list(mel.shape)}, "
+                           f"out {list(out.shape)}")
+    if not P.dtype == mel.dtype == out.dtype or P.dtype not in (torch.float32, torch.float64):
+        raise RuntimeError("specinv_b200: mel_inverse needs P, mel and out of one dtype, float32 or float64")
+    if not 0 <= f_lo <= f_hi <= F:
+        raise RuntimeError(f"specinv_b200: mel_inverse row range [{f_lo}, {f_hi}) outside [0, {F})")
+
+
+def mel_inverse_direct(P: Tensor, mel: Tensor, out: Tensor, f_lo: int, f_hi: int) -> None:
+    """out[b, f, t] = relu(sum_j P[f, j] mel[b, j, t]) for rows f in [f_lo, f_hi), 0 elsewhere (specinv_mel_inverse),
+    called straight through ctypes: the module's one launch per call skips the custom op's dispatch (see
+    `iter_direct`)."""
+    _need_cuda(P, mel, out)
+    _check_mel_inverse(P, mel, out, f_lo, f_hi)
+    B, F, T = out.shape
+    with torch.cuda.device(out.device):
+        _ok(_lib.lib().specinv_mel_inverse(_DT[out.dtype], _p(P), F, P.shape[1], int(f_lo), int(f_hi), _p(mel),
+                                           _p(out), B, T, _stream(out)), "mel_inverse")
+
+
+@torch.library.custom_op("specinv_b200::mel_inverse", mutates_args=("out",), device_types="cuda")
+def mel_inverse(P: Tensor, mel: Tensor, out: Tensor, f_lo: int, f_hi: int) -> None:
+    """torchaudio's InverseMelScale as one GEMM: out (B, n_stft, T) = relu(P @ mel), P = pinv(fb.T) (n_stft, n_mels),
+    mel (B, n_mels, T); rows of P outside [f_lo, f_hi) are zero and their outputs are written as zeros."""
+    mel_inverse_direct(P, mel, out, f_lo, f_hi)
+
+
+def _fake_mel_inverse(P, mel, out, f_lo, f_hi) -> None:
+    _check_mel_inverse(P, mel, out, f_lo, f_hi)
+    return None
+
+
+# torchaudio_compat.InverseMelScale
+MEL_OPS = (mel_inverse,)
+mel_inverse.register_fake(_fake_mel_inverse)

@@ -9,11 +9,19 @@ The one-shot preprocessing runs on torch ops on the input's device, exactly as t
 ``specgram.pow(1 / power)``, the random (``torch.rand`` of the complex dtype) or all-ones start phases and their
 product.  The same seed therefore gives the same start as torchaudio, for host and CUDA inputs alike.
 
+``InverseMelScale`` is ``torchaudio.transforms.InverseMelScale`` with the same filterbank, bit for bit, so that
+``InverseMelScale`` -> ``GriffinLim`` takes a mel spectrogram to a waveform as torchaudio's Tacotron2 Griffin-Lim
+vocoder does.  torchaudio's ``relu(lstsq(fb.T, mel).solution)`` is ``relu(P @ mel)`` per frame with
+``P = pinv(fb.T)``; ``P`` is computed once per filterbank on the host in float64 and applied by one launch of
+``specinv_mel_inverse``.
+
 These names are not exported at the package's top level: ``griffinlim`` next to ``griffin_lim`` would invite mistakes.
 """
 from __future__ import annotations
 
-from typing import Callable, Optional
+import math
+import warnings
+from typing import Callable, Optional, Tuple
 
 import torch
 from torch import Tensor
@@ -245,3 +253,199 @@ class GriffinLim(torch.nn.Module):
     def forward(self, specgram: Tensor) -> Tensor:
         return griffinlim(specgram, self.window, self.n_fft, self.hop_length, self.win_length, self.power, self.n_iter,
                           self.momentum, self.length, self.rand_init)
+
+
+# ---- InverseMelScale ---------------------------------------------------------------------------------------------
+# torchaudio.functional.melscale_fbanks restated op for op (same float32 linspace, same slopes, same min / max), so
+# that `fb` is bitwise torchaudio's and a state_dict moves between the two modules.
+def _hz_to_mel(freq: float, mel_scale: str = "htk") -> float:
+    if mel_scale not in ["slaney", "htk"]:
+        raise ValueError('mel_scale should be one of "htk" or "slaney".')
+    if mel_scale == "htk":
+        return 2595.0 * math.log10(1.0 + (freq / 700.0))
+    f_min = 0.0
+    f_sp = 200.0 / 3
+    mels = (freq - f_min) / f_sp
+    min_log_hz = 1000.0
+    min_log_mel = (min_log_hz - f_min) / f_sp
+    logstep = math.log(6.4) / 27.0
+    if freq >= min_log_hz:
+        mels = min_log_mel + math.log(freq / min_log_hz) / logstep
+    return mels
+
+
+def _mel_to_hz(mels: Tensor, mel_scale: str = "htk") -> Tensor:
+    if mel_scale not in ["slaney", "htk"]:
+        raise ValueError('mel_scale should be one of "htk" or "slaney".')
+    if mel_scale == "htk":
+        return 700.0 * (10.0 ** (mels / 2595.0) - 1.0)
+    f_min = 0.0
+    f_sp = 200.0 / 3
+    freqs = f_min + f_sp * mels
+    min_log_hz = 1000.0
+    min_log_mel = (min_log_hz - f_min) / f_sp
+    logstep = math.log(6.4) / 27.0
+    log_t = mels >= min_log_mel
+    freqs[log_t] = min_log_hz * torch.exp(logstep * (mels[log_t] - min_log_mel))
+    return freqs
+
+
+def _create_triangular_filterbank(all_freqs: Tensor, f_pts: Tensor) -> Tensor:
+    f_diff = f_pts[1:] - f_pts[:-1]
+    slopes = f_pts.unsqueeze(0) - all_freqs.unsqueeze(1)
+    zero = torch.zeros(1)
+    down_slopes = (-1.0 * slopes[:, :-2]) / f_diff[:-1]
+    up_slopes = slopes[:, 2:] / f_diff[1:]
+    return torch.max(zero, torch.min(down_slopes, up_slopes))
+
+
+def _melscale_fbanks(n_freqs: int, f_min: float, f_max: float, n_mels: int, sample_rate: int,
+                     norm: Optional[str] = None, mel_scale: str = "htk") -> Tensor:
+    """(n_freqs, n_mels) triangular filterbank: ``torchaudio.functional.melscale_fbanks``, bit for bit."""
+    if norm is not None and norm != "slaney":
+        raise ValueError('norm must be one of None or "slaney"')
+    all_freqs = torch.linspace(0, sample_rate // 2, n_freqs)
+    m_min = _hz_to_mel(f_min, mel_scale=mel_scale)
+    m_max = _hz_to_mel(f_max, mel_scale=mel_scale)
+    m_pts = torch.linspace(m_min, m_max, n_mels + 2)
+    f_pts = _mel_to_hz(m_pts, mel_scale=mel_scale)
+    fb = _create_triangular_filterbank(all_freqs, f_pts)
+    if norm is not None and norm == "slaney":
+        enorm = 2.0 / (f_pts[2:n_mels + 2] - f_pts[:n_mels])
+        fb *= enorm.unsqueeze(0)
+    if (fb.max(dim=0).values == 0.0).any():
+        warnings.warn(
+            "At least one mel filterbank has all zero values. "
+            f"The value for `n_mels` ({n_mels}) may be set too high. "
+            f"Or, the value for `n_freqs` ({n_freqs}) may be set too low."
+        )
+    return fb
+
+
+_DRIVERS = ["gels", "gelsy", "gelsd", "gelss"]
+
+
+def _mel_operator(fb: Tensor, driver: str) -> Tuple[Tensor, int, int]:
+    """``(P, f_lo, f_hi)``: ``P = pinv(fb.T)`` of shape (n_stft, n_mels), computed in float64 from the SVD and
+    returned in fb's dtype on fb's device, and the rows ``[f_lo, f_hi)`` outside which ``fb`` (hence ``P``) is zero.
+
+    Singular values ``<= sigma_max * max(n_stft, n_mels) * eps64`` are dropped: the default cutoff of
+    ``torch.linalg.pinv``, ``matrix_rank`` and ``lstsq(driver="gelsd")``.  With ``driver="gels"`` a rank below
+    n_mels raises ``torch.linalg.LinAlgError``, as LAPACK's gels does on the host; the other drivers return the
+    minimum-norm solution.  The product is ``torch.linalg.pinv``'s; the rows of ``P`` that no filter covers are zero
+    in exact arithmetic and are set to exactly zero (the SVD leaves ~1e-16 there)."""
+    A = fb.detach().to("cpu", torch.float64).T                      # fb.T: (n_mels, n_stft)
+    n_mels, n_stft = A.shape
+    covered = torch.nonzero(A.ne(0).any(dim=0)).flatten()
+    f_lo, f_hi = (int(covered[0]), int(covered[-1]) + 1) if covered.numel() else (0, 0)
+    U, S, Vh = torch.linalg.svd(A, full_matrices=False)
+    keep = S > S.max() * max(n_stft, n_mels) * torch.finfo(torch.float64).eps
+    rank = int(keep.sum())
+    P = (Vh.mT * torch.where(keep, 1 / S, torch.zeros_like(S)).unsqueeze(-2)) @ U.mT
+    P[:f_lo] = 0
+    P[f_hi:] = 0
+    if driver == "gels" and rank < n_mels:
+        raise torch.linalg.LinAlgError(
+            "torch.linalg.lstsq: The least squares solution could not be computed because the input matrix does not "
+            f"have full rank (rank {rank} of {n_mels}: the mel filterbank has dependent or all-zero filters; "
+            "driver='gelsd' returns the minimum-norm solution)")
+    return P.to(device=fb.device, dtype=fb.dtype).contiguous(), f_lo, f_hi
+
+
+class InverseMelScale(torch.nn.Module):
+    r"""``torchaudio.transforms.InverseMelScale`` on one sm_100a kernel: same constructor, defaults, ``fb`` buffer and
+    checks.  Estimates the linear magnitude spectrogram as ``relu(pinv(fb.T) @ mel)``, the minimum-norm least-squares
+    solution torchaudio's ``relu(lstsq(fb.T, mel).solution)`` returns.
+
+    Args:
+        n_stft (int): number of STFT bins (``n_fft // 2 + 1``).  n_mels (int): default 128.  sample_rate (int):
+        default 16000.  f_min (float): default 0.  f_max (float or None): default ``sample_rate // 2`` (so does 0).
+        norm (str or None): None or ``"slaney"``.  mel_scale (str): ``"htk"`` (default) or ``"slaney"``.
+        driver (str): ``"gels"`` (default), ``"gelsy"``, ``"gelsd"`` or ``"gelss"``.
+
+    ``pinv(fb.T)`` is computed once per filterbank on the host in float64 and cached on the module, keyed on fb's
+    device, dtype and version, so ``.to()``, ``.double()`` and ``load_state_dict`` take effect; ``state_dict()``
+    holds only ``fb``.  Input and ``fb`` must share dtype and device; ``.double()`` the module for float64.  A host
+    module takes host input, computes on the current CUDA device and returns a host tensor.
+
+    Possible deviations from torchaudio for CUDA inputs: torchaudio documents only ``"gels"`` there and assumes a
+    full-rank ``fb``.  Here the rule is the same on every device: ``"gels"`` raises ``torch.linalg.LinAlgError``
+    when the rank (with ``torch.linalg.pinv``'s cutoff) is below n_mels, as torchaudio's host path does, and the
+    other drivers return the minimum-norm solution.  The result depends only on the values, not on the device.
+
+    There is no gradient: an input that requires grad raises ``NotImplementedError``.  torchaudio's Tacotron2
+    Griffin-Lim vocoder calls ``requires_grad_(True)`` on the mel and detaches the result on the next line, a
+    leftover of the older gradient-descent InverseMelScale; drop that line when switching to this module.
+    """
+    __constants__ = ["n_stft", "n_mels", "sample_rate", "f_min", "f_max"]
+
+    def __init__(self, n_stft: int, n_mels: int = 128, sample_rate: int = 16000, f_min: float = 0.0,
+                 f_max: Optional[float] = None, norm: Optional[str] = None, mel_scale: str = "htk",
+                 driver: str = "gels") -> None:
+        super().__init__()
+        self.n_stft = n_stft
+        self.n_mels = n_mels
+        self.sample_rate = sample_rate
+        self.f_max = f_max or float(sample_rate // 2)
+        self.f_min = f_min
+        self.norm = norm
+        self.mel_scale = mel_scale
+        self.driver = driver
+        if f_min > self.f_max:
+            raise ValueError("Require f_min: {} <= f_max: {}".format(f_min, self.f_max))
+        if driver not in _DRIVERS:
+            raise ValueError(f'driver must be one of ["gels", "gelsy", "gelsd", "gelss"]. Found {driver}.')
+        fb = _melscale_fbanks(self.n_stft, self.f_min, self.f_max, self.n_mels, self.sample_rate, self.norm,
+                              self.mel_scale)
+        self.register_buffer("fb", fb)
+        self._op_cache = None       # (key, P, f_lo, f_hi); deliberately not a buffer
+
+    def operator(self) -> Tuple[Tensor, int, int]:
+        """``(P, f_lo, f_hi)`` of the current ``fb`` (see ``_mel_operator``), recomputed when fb changes."""
+        fb = self.fb
+        key = (fb.device, fb.dtype, fb._version, fb.data_ptr())
+        if self._op_cache is None or self._op_cache[0] != key:
+            self._op_cache = (key, *_mel_operator(fb, self.driver))
+        return self._op_cache[1:]
+
+    def forward(self, melspec: Tensor) -> Tensor:
+        r"""
+        Args:
+            melspec (Tensor): mel spectrogram ``(..., n_mels, time)``, in fb's dtype, on fb's device.
+
+        Returns:
+            Tensor: linear magnitude spectrogram ``(..., n_stft, time)`` on melspec's device.
+        """
+        if melspec.dim() < 2:
+            raise RuntimeError(f"InverseMelScale: expected a (..., n_mels, time) tensor, got shape {list(melspec.shape)}")
+        shape = melspec.size()
+        n_mels, time = shape[-2], shape[-1]
+        freq = self.fb.size(0)
+        if self.n_mels != n_mels:
+            raise ValueError("Expected an input with {} mel bins. Found: {}".format(self.n_mels, n_mels))
+        if melspec.requires_grad:
+            raise NotImplementedError("torchaudio_compat.InverseMelScale has no gradient path: the input must not "
+                                      "require grad")
+        if melspec.dtype != self.fb.dtype:
+            raise RuntimeError("torch.linalg.lstsq: Expected input and other to have the same dtype, but got "
+                               f"input's dtype {self.fb.dtype} and other's dtype {melspec.dtype}")
+        if melspec.device != self.fb.device:
+            raise RuntimeError(f"InverseMelScale: fb is on {self.fb.device} and the input on {melspec.device}: move "
+                               "the module with .to()")
+        if self.fb.dtype not in (torch.float32, torch.float64):
+            raise RuntimeError(f"InverseMelScale: dtype {self.fb.dtype} is not supported (float32 / float64 only)")
+        P, f_lo, f_hi = self.operator()
+        mel = melspec.reshape(math.prod(shape[:-2]), n_mels, time)
+        if mel.numel() == 0 or time == 0:
+            return torch.zeros(shape[:-2] + (freq, time), dtype=melspec.dtype, device=melspec.device)
+        dev = compute_device(mel)
+        mel = mel.to(dev, non_blocking=True).contiguous()
+        out = torch.empty(mel.shape[0], freq, time, dtype=mel.dtype, device=dev)
+        _ops.mel_inverse_direct(P.to(dev), mel, out, f_lo, f_hi)
+        out = out.view(shape[:-2] + (freq, time))
+        if dev == melspec.device:
+            return out
+        y = torch.empty(out.shape, dtype=out.dtype, pin_memory=melspec.is_pinned())
+        y.copy_(out, non_blocking=True)
+        torch.cuda.current_stream(dev).synchronize()
+        return y
