@@ -361,11 +361,9 @@ static int launch_tile(TileArgs& a, cudaStream_t st) {
     if (e != cudaSuccess) return (int)e;
     dim3 grid((dm.T + owned - 1) / owned, dm.B);
     if (grid.y > 65535) return SPECINV_ERR_UNSUPPORTED;
-    // threads per CTA: enough to give every thread a few butterflies per pass; SPECINV_TILE_THREADS overrides
-    static int forced = -1;
-    if (forced < 0) { const char* e = getenv("SPECINV_TILE_THREADS"); forced = e ? atoi(e) : 0; }
+    // threads per CTA: enough to give every thread a few butterflies per pass
     const long long bf = (long long)(owned + halo) * (dm.M >> 2);     // radix-4 butterflies per pass
-    int threads = forced > 0 ? forced : (bf >= 4096 ? 1024 : bf >= 1024 ? 512 : 256);
+    const int threads = bf >= 4096 ? 1024 : bf >= 1024 ? 512 : 256;
     tile_kernel<T, OP><<<grid, threads, smem, st>>>(a);
     return (int)cudaGetLastError();
 }

@@ -14,7 +14,6 @@
 //
 // Replaces, per iteration, torch.stft + ~8 point-wise kernels + fft.irfft + conv_transpose1d with a dense
 // diag(window) weight of the reference (methods.py:241-248, :464-477, :127-132).
-#include <cstdlib>
 
 #include "specinv_common.cuh"
 #include "generic_tile.cuh"
@@ -318,12 +317,9 @@ static int launch_mr(TileArgs& a, const mr::Plan& mp, cudaStream_t st) {
     if (optin <= 0) return SPECINV_ERR_NO_DEVICE;
     const size_t big = (size_t)optin - 1024 - perm_bytes;
     // Two CTAs of 16 warps per SM (1024 threads at 64 registers), each with half of the SM's shared memory (228 KB,
-    // 1 KB reserved per CTA).  SPECINV_MR_CTAS_PER_SM=4 launches four CTAs of 8 warps with a quarter each: measured
-    // within +-6 % of the default (0.305 vs 0.326 ms at 400/100, 1.09 vs 1.05 ms at 256/64, 1.29 vs 0.75 ms at 1536/384
-    // where the smaller tile pays more halo frames), so it stays an experiment switch.
-    static int forced_ctas = -1;
-    if (forced_ctas < 0) { const char* e = getenv("SPECINV_MR_CTAS_PER_SM"); forced_ctas = e ? atoi(e) : 0; }
-    const int ctas = forced_ctas == 4 ? 4 : 2;
+    // 1 KB reserved per CTA).  Four CTAs of 8 warps with a quarter each measured no better (within +-6 %, and 1.29 vs
+    // 0.75 ms at 1536/384, where the smaller tile pays more halo frames).
+    const int ctas = 2;
     size_t budget = (size_t)(228 * 1024 / ctas - 1024) - 256 - perm_bytes;
     if (budget > big) budget = big;
     int cap = (int)(budget / frame_bytes);

@@ -17,11 +17,8 @@
 // warp.  After max_iter iterations the oldest frame is committed: it joins the kept ring and is overlap-added
 // (window w, 1/envelope, centre trimming) into the output (methods.py:401-408).  HBM traffic: the magnitudes once,
 // the signal once.
-#include <cstdlib>
-
 #include "specinv_common.cuh"
 #include "gl_warp_core.cuh"
-#include "gl_warp_core_1c.cuh"
 #include "sm100_ptx.cuh"
 
 namespace specinv {
@@ -76,24 +73,11 @@ __device__ __forceinline__ void frame_sync(int bar_id) {
     else asm volatile("bar.sync %0, %1;" ::"r"(bar_id), "n"(LANES) : "memory");
 }
 
-// Shape constants of a (LANES, VV) variant.  <64, 8> is the "one residue class per lane" scheme of
-// gl_warp_core_1c.cuh (n_fft = 1024 over TWO warps): 4 pair slots and 8-point FFTs in all three passes.
-template <int LANES, int VV> struct Shape {
-    using C = Cfg<LANES, VV>;
-    static constexpr bool ONEC = false;
-    static constexpr int M = C::M, HOP = C::HOP, RC = C::RC, R1 = C::R1, R2 = C::R2, CMASK = C::RC - 1;
-};
-template <> struct Shape<64, 8> {
-    static constexpr bool ONEC = true;
-    static constexpr int M = 512, HOP = 256, RC = 4, R1 = 8, R2 = 8, CMASK = 7;
-};
-
 // LANES lanes (LANES / 32 warps) per frame and VV complex values per lane: <32, 16> n_fft = 1024, <32, 8> n_fft = 512,
-// <64, 16> n_fft = 2048, <64, 8> n_fft = 1024 on two warps; SIGS signals per CTA (SIGS x 4 frame slots)
+// <64, 16> n_fft = 2048; SIGS signals per CTA (SIGS x 4 frame slots)
 template <int LANES, int VV, int SIGS>
 __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(const RArgs a) {
-    using C = Shape<LANES, VV>;
-    constexpr bool ONEC = C::ONEC;
+    using C = Cfg<LANES, VV>;
     constexpr int V = VV;                          // shadows wfast::V
     constexpr int M = C::M, HOP = C::HOP, RC = C::RC, HP = VV / 4;
     constexpr int ROWS = M;                        // float2 per frame: VV rows of LANES lanes
@@ -108,8 +92,7 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
         int pl, ph, ql, qh, q0;
         __device__ __forceinline__ int operator()(int e) const {
             const int j = e >> 1;
-            if constexpr (ONEC) return (e & 1) ? (j == 0 ? q0 : ql - LANES * j) : pl + LANES * j;      // gl_warp_core_1c.cuh: bin1
-            else return (e & 1) ? (j == 0 ? q0 : (j >= RC / 2 ? qh : ql) - 2 * LANES * j) : (j >= RC / 2 ? ph : pl) + 2 * LANES * j;
+            return (e & 1) ? (j == 0 ? q0 : (j >= RC / 2 ? qh : ql) - 2 * LANES * j) : (j >= RC / 2 ? ph : pl) + 2 * LANES * j;
         }
     };
     extern __shared__ __align__(16) float2 sm[];
@@ -152,14 +135,13 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
         tmem_stw<2 * V>(tlane + TC_TW1, t);
 #pragma unroll
         for (int kb = 0; kb < C::R2; ++kb) {
-            const float2 w = a.tw[(C::R1 * (l & C::CMASK) * kb) & (M - 1)];
+            const float2 w = a.tw[(C::R1 * (l & (C::RC - 1)) * kb) & (M - 1)];
             t[2 * kb] = w.x; t[2 * kb + 1] = w.y;
         }
         tmem_stw<2 * C::R2>(tlane + TC_TW2, t);
 #pragma unroll
         for (int j = 0; j < RC; ++j) {
-            int k;
-            if constexpr (ONEC) k = l + LANES * j; else k = slot_bin_rt<LANES, VV>(l, j);
+            const int k = slot_bin_rt<LANES, VV>(l, j);
             float2 w;
             if (k <= M / 2) w = a.twr[k];
             else { w = a.twr[M - k]; w.x = -w.x; }
@@ -177,7 +159,7 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
         tmem_stw<2 * V>(tlane + TC_TW1C, t);
 #pragma unroll
         for (int kb = 0; kb < C::R2; ++kb) {
-            const float2 w = a.tw[(C::R1 * (l & C::CMASK) * kb) & (M - 1)];
+            const float2 w = a.tw[(C::R1 * (l & (C::RC - 1)) * kb) & (M - 1)];
             t[2 * kb] = w.x; t[2 * kb + 1] = -w.y;
         }
         tmem_stw<2 * C::R2>(tlane + TC_TW2C, t);
@@ -279,39 +261,19 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
                         const float* mg; float mn;
                         __device__ __forceinline__ float2 s0(int e) const { return f2(e < 0 ? mn : mg[e], 0.f); }
                     } io0{mg, mag_nyq};
-                    if constexpr (ONEC) {
-                        float2 A[8], Bv[4], twr[4], twrc[4], tw[8], twc[8];
-                        tmem_ldw<8>(tlane + TC_TWR, reinterpret_cast<float*>(twr));
-                        tmem_ldw<8>(tlane + TC_TWRC, reinterpret_cast<float*>(twrc));
-                        spectrum_pairs1(l, A, Bv, twr, twrc, io0);
-                        pair_return(l, Bv, e1);                     // the mirror lane's upper half goes through E1
-                        frame_sync<LANES>(fbar);
-                        pair_collect(l, e1, A);
-                        inv1_pass3(l, A, e2);
-                        frame_sync<LANES>(fbar);
-                        tmem_ldw<16>(tlane + TC_TW2, reinterpret_cast<float*>(tw));
-                        tmem_ldw<16>(tlane + TC_TW2C, reinterpret_cast<float*>(twc));
-                        inv1_pass2(l, e2, tw, twc, e1);
-                        frame_sync<LANES>(fbar);
-                        tmem_ldw<16>(tlane + TC_TW1, reinterpret_cast<float*>(tw));
-                        tmem_ldw<16>(tlane + TC_TW1C, reinterpret_cast<float*>(twc));
-                        inv1_pass1(l, e1, tw, twc, v);
-                        frame_sync<LANES>(fbar);
-                    } else {
-                        float2 A[RC], Bv[RC], twr[RC];
-                        tmem_ldw<2 * RC>(tlane + TC_TWR, reinterpret_cast<float*>(twr));
-                        spectrum_pairs<VV>(l, A, Bv, twr, io0);
-                        inv_pass3<LANES, VV>(l, A, Bv, e2);
-                        frame_sync<LANES>(fbar);
-                        float2 tw2[C::R2];
-                        tmem_ldw<2 * C::R2>(tlane + TC_TW2, reinterpret_cast<float*>(tw2));
-                        inv_pass2<LANES, VV>(l, e2, tw2, e1);
-                        frame_sync<LANES>(fbar);
-                        float2 tw1[V];
-                        tmem_ldw<2 * V>(tlane + TC_TW1, reinterpret_cast<float*>(tw1));
-                        inv_pass1<LANES, VV>(l, e1, tw1, v);
-                        frame_sync<LANES>(fbar);
-                    }
+                    float2 A[RC], Bv[RC], twr[RC];
+                    tmem_ldw<2 * RC>(tlane + TC_TWR, reinterpret_cast<float*>(twr));
+                    spectrum_pairs<VV>(l, A, Bv, twr, io0);
+                    inv_pass3<LANES, VV>(l, A, Bv, e2);
+                    frame_sync<LANES>(fbar);
+                    float2 tw2[C::R2];
+                    tmem_ldw<2 * C::R2>(tlane + TC_TW2, reinterpret_cast<float*>(tw2));
+                    inv_pass2<LANES, VV>(l, e2, tw2, e1);
+                    frame_sync<LANES>(fbar);
+                    float2 tw1[V];
+                    tmem_ldw<2 * V>(tlane + TC_TW1, reinterpret_cast<float*>(tw1));
+                    inv_pass1<LANES, VV>(l, e1, tw1, v);
+                    frame_sync<LANES>(fbar);
                 }
             }
             // ---- part of this frame's y that comes from the kept frames: constant over the inner iterations.
@@ -375,7 +337,7 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
 #pragma unroll
                     for (int r = 0; r < V; ++r) y[r] = pmul(y[r], w[r]);
                 }
-                // momentum state and magnitudes of this frame's bins (element e of gl_warp_core*.cuh)
+                // momentum state and magnitudes of this frame's bins (element e of gl_warp_core.cuh)
                 struct IO {
                     float2* pre; const float* mg; float2 pn; float mn;
                     __device__ __forceinline__ float2 s0(int e) const { return e < 0 ? pn : pre[e]; }
@@ -384,51 +346,6 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
                     __device__ __forceinline__ void put(int e, float2 q, float2) { if (e < 0) pn = q; else pre[e] = q; }
                 };
                 const bool mom = j > 0 || (i > 0 && !newest);
-                if constexpr (ONEC) {
-                    // ---- one residue class per lane (gl_warp_core_1c.cuh): two warps share the frame
-                    float2 tw[8], twc[8];
-                    tmem_ldw<16>(tlane + TC_TW1, reinterpret_cast<float*>(tw));
-                    tmem_ldw<16>(tlane + TC_TW1C, reinterpret_cast<float*>(twc));
-                    fwd1_pass1(l, y, tw, twc, e1);
-                    frame_sync<LANES>(fbar);
-                    tmem_ldw<16>(tlane + TC_TW2, reinterpret_cast<float*>(tw));
-                    tmem_ldw<16>(tlane + TC_TW2C, reinterpret_cast<float*>(twc));
-                    fwd1_pass2(l, e1, tw, twc, e2);
-                    frame_sync<LANES>(fbar);
-                    float2 A[8], Bv[4];
-                    fwd1_pass3(l, e2, A);
-                    pair_publish(l, A, e1);                       // E1 is idle until the inverse pass 2: the pair exchange
-                    frame_sync<LANES>(fbar);
-                    pair_fetch(l, e1, Bv);
-                    {
-                        float2 pre[V];
-                        float mg[V];
-                        tmem_wait_st();
-                        tmem_ldw<2 * V>(twarp + TC_PRE, reinterpret_cast<float*>(pre));
-                        tmem_ldw<V>(twarp + TC_MAG, mg);
-                        IO io{pre, mg, pre_nyq, mag_nyq};
-                        float2 twr[4], twrc[4];
-                        tmem_ldw<8>(tlane + TC_TWR, reinterpret_cast<float*>(twr));
-                        tmem_ldw<8>(tlane + TC_TWRC, reinterpret_cast<float*>(twrc));
-                        float ds = 0.f, es = 0.f;
-                        pointwise1<OP_GL, false>(l, A, Bv, twr, twrc, io, mom ? a.lr : 0.f, 0.f, ds, es);
-                        pre_nyq = io.pn;
-                        tmem_stw<2 * V>(twarp + TC_PRE, reinterpret_cast<const float*>(pre));
-                    }
-                    pair_return(l, Bv, e1);
-                    frame_sync<LANES>(fbar);
-                    pair_collect(l, e1, A);
-                    inv1_pass3(l, A, e2);
-                    frame_sync<LANES>(fbar);
-                    tmem_ldw<16>(tlane + TC_TW2, reinterpret_cast<float*>(tw));
-                    tmem_ldw<16>(tlane + TC_TW2C, reinterpret_cast<float*>(twc));
-                    inv1_pass2(l, e2, tw, twc, e1);
-                    frame_sync<LANES>(fbar);
-                    tmem_ldw<16>(tlane + TC_TW1, reinterpret_cast<float*>(tw));
-                    tmem_ldw<16>(tlane + TC_TW1C, reinterpret_cast<float*>(twc));
-                    inv1_pass1(l, e1, tw, twc, v);
-                    frame_sync<LANES>(fbar);
-                } else {
                 {
                     float2 tw1[V], tw1c[V];
                     tmem_ldw<2 * V>(tlane + TC_TW1, reinterpret_cast<float*>(tw1));
@@ -478,7 +395,6 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
                     inv_pass1<LANES, VV, HC>(l, e1, tw1, v, tw1c);
                 }
                 frame_sync<LANES>(fbar);
-                }
             }
 
             // ---- commit the oldest active frame (:401-404) and fuse the final overlap-add (:406-408)
@@ -572,7 +488,7 @@ __global__ void __launch_bounds__(SIGS * NAMAX * LANES, 1) rtisi_fast_kernel(con
 
 template <int LANES, int VV, int SIGS>
 static int launch(const RArgs& a, cudaStream_t st) {
-    const size_t smem = (size_t)SIGS * sig_f2(Shape<LANES, VV>::M) * sizeof(float2);
+    const size_t smem = (size_t)SIGS * sig_f2(Cfg<LANES, VV>::M) * sizeof(float2);
     cudaError_t e = cudaFuncSetAttribute(rtisi_fast_kernel<LANES, VV, SIGS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     rtisi_fast_kernel<LANES, VV, SIGS><<<(a.B + SIGS - 1) / SIGS, SIGS * NAMAX * LANES, smem, st>>>(a);
@@ -608,14 +524,9 @@ int rtisi_fast(const specinv_desc* d, const Dims& dm, const void* plan, const vo
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess)
         return SPECINV_ERR_NO_DEVICE;
     if (d->n_fft == 2048) return rfast::launch<64, 16, 1>(a, st);       // two warps per frame, one signal per CTA
-    if (d->n_fft == 1024) {
-        // SPECINV_RTISI_TWO_WARPS=1: two warps per frame, 8 values per lane (gl_warp_core_1c.cuh).  Half the
-        // instructions per lane, but the same FP work per SM plus two more frame barriers and the mirror-lane exchange:
-        // measured 62.6 ms against 57.2 ms at cfg3 (the FMA pipe is 59 % busy either way), so it is not the default.
-        const char* e = getenv("SPECINV_RTISI_TWO_WARPS");
-        if (e && e[0] == '1') return dm.B <= sms ? rfast::launch<64, 8, 1>(a, st) : rfast::launch<64, 8, 2>(a, st);
-        return dm.B <= sms ? rfast::launch<32, 16, 1>(a, st) : rfast::launch<32, 16, 2>(a, st);
-    }
+    // n_fft = 1024 on one warp per frame: two warps at 8 values per lane measured slower (62.6 ms against 57.2 ms at
+    // cfg3, DESIGN.md section 3.3)
+    if (d->n_fft == 1024) return dm.B <= sms ? rfast::launch<32, 16, 1>(a, st) : rfast::launch<32, 16, 2>(a, st);
     return dm.B <= sms ? rfast::launch<32, 8, 1>(a, st) : dm.B <= 2 * sms ? rfast::launch<32, 8, 2>(a, st)
                                                                           : rfast::launch<32, 8, 4>(a, st);
 }

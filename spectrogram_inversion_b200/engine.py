@@ -140,6 +140,11 @@ def spec_sums(a: SplitSpec, b: SplitSpec) -> torch.Tensor:
     return out
 
 
+def evaluates(i: int, eva_iter: int) -> bool:
+    """Whether iteration ``i`` (from 0) of the reference loop evaluates the metric (methods.py:153-190)."""
+    return i % eva_iter == eva_iter - 1
+
+
 class _Solver:
     """Common ping-pong state for the fused iterations."""
 
@@ -153,11 +158,7 @@ class _Solver:
         self.g = float(spec_sums(mag, mag)[2].item())   # sum mag^2 (constant per call)
         self.iterations = 0
         # Iterations are launched straight through ctypes (`_ops.iter_direct`, ~6 us of host time each), which keeps
-        # even the smallest config GPU-bound (cfg1: 24 us of kernel per iteration).  Replaying runs of iterations
-        # from a CUDA graph is available (`use_graphs = True`) for a solver that lives long enough to pay for the
-        # capture: measured 2.6-4 ms per captured graph, more than a whole 100-iteration cfg1 job.
-        self._graphs = {}
-        self.use_graphs = False
+        # even the smallest config GPU-bound (cfg1: 24 us of kernel per iteration).
         self._ptrs = [None, None]      # per ping-pong parity: (tensors, their device pointers)
 
     def _launch_direct(self, what: str, tensors: tuple, coef: float, sums: torch.Tensor) -> None:
@@ -192,55 +193,12 @@ class _Solver:
             return d, e
         return None
 
-
-    def run_plain(self, n: int) -> None:
-        """``n`` iterations without evaluation (no host synchronisation)."""
-        self.run_many(n, self.iterations, 1, evaluate=False)
-
     def run_many(self, n: int, iter0: int, eva_iter: int, evaluate: bool = True) -> None:
         """Iterations iter0 .. iter0 + n - 1 of the reference loop (methods.py:178-190) without host synchronisation:
-        those with ``i % eva_iter == eva_iter - 1`` run the fused metric epilogue when ``evaluate`` (the last pair of
-        sums stays in ``self.sums``)."""
-        if not evaluate:
-            return self.run_pattern((False,) * n)
-        i = 0
-        while i < n:
-            m = min(eva_iter, n - i)
-            self.run_pattern(tuple((iter0 + i + k) % eva_iter == eva_iter - 1 for k in range(m)))
-            i += m
-
-    def run_pattern(self, flags: Tuple[bool, ...]) -> None:
-        """One iteration per flag, evaluating (fused metric sums left on the device, not read) where the flag is
-        set; never synchronises with the host.  Small problems replay the whole pattern from a CUDA graph."""
-        n = len(flags)
-        if n <= 0:
-            return
-        if n == 1 or not self.use_graphs:
-            for f in flags:
-                self.step(evaluate=f, read=False)
-            return
-        key = (flags if any(flags) else n, self.cur)
-        graph = self._graphs.get(key)
-        if graph is None:
-            # record n ping-pong launches starting from the current parity (the buffers are fixed for the
-            # solver's life); nothing executes during capture, so the bookkeeping is rolled back afterwards
-            cur, its, launches = self.cur, self.iterations, _ops.LAUNCHES[0]
-            graph = torch.cuda.CUDAGraph()
-            main = torch.cuda.current_stream(self.plan.device)
-            side = torch.cuda.Stream(self.plan.device)
-            side.wait_stream(main)
-            with torch.cuda.stream(side):
-                graph.capture_begin(capture_error_mode="thread_local")
-                for f in flags:
-                    self.step(evaluate=f, read=False)
-                graph.capture_end()
-            main.wait_stream(side)
-            self.cur, self.iterations, _ops.LAUNCHES[0] = cur, its, launches
-            self._graphs[key] = graph
-        graph.replay()
-        self.cur ^= n & 1
-        self.iterations += n
-        _ops.LAUNCHES[0] += n
+        those that ``evaluates`` run the fused metric epilogue when ``evaluate`` (the last pair of sums stays in
+        ``self.sums``)."""
+        for i in range(iter0, iter0 + n):
+            self.step(evaluate=evaluate and evaluates(i, eva_iter), read=False)
 
 
 class GriffinLimSolver(_Solver):
@@ -264,10 +222,10 @@ class GriffinLimSolver(_Solver):
                 self._resident_ws = torch.empty(nbytes.value, dtype=torch.uint8, device=plan.device)
 
     def run_many(self, n: int, iter0: int, eva_iter: int, evaluate: bool = True) -> None:
-        if self._resident_ws is None or n < 2 or self.use_graphs:
+        if self._resident_ws is None or n < 2:
             return super().run_many(n, iter0, eva_iter, evaluate)
         p, i, o = self.plan, self.cur, self.cur ^ 1
-        n_eval = sum(1 for k in range(n) if (iter0 + k) % eva_iter == eva_iter - 1) if evaluate else 0
+        n_eval = sum(1 for k in range(iter0, iter0 + n) if evaluates(k, eva_iter)) if evaluate else 0
         sums = torch.zeros(2 * n_eval, dtype=torch.float64, device=p.device) if n_eval else None
         stream = torch.cuda.current_stream(p.device).cuda_stream
         with torch.cuda.device(p.device):
@@ -344,7 +302,8 @@ def training_loop(solver, max_iter: int, tol: float, verbose, eva_iter: int, met
                   history: Optional[List] = None, reduce_sums: Optional[Callable] = None) -> int:
     """Host loop with the reference's evaluation cadence and early-stop rule (methods.py:153-190).
 
-    ``solver`` needs ``step(evaluate) -> (d, e) | None``, ``g`` and ``n_bins_total``.  ``reduce_sums``
+    ``solver`` needs ``step(evaluate) -> (d, e) | None``, ``g`` and ``n_bins_total``; with ``run_many`` (every
+    ``_Solver``) the iterations between evaluations run without a host synchronisation.  ``reduce_sums``
     (multi-GPU): maps the local ``(d, e)`` of an evaluation to the global ones (an all-reduce), so that the
     metric, the loss and therefore the stopping decision are those of the whole batch on every rank --
     the reference evaluates over the entire batch (methods.py:181-182); ``solver.g`` / ``n_bins_total`` must
@@ -358,50 +317,41 @@ def training_loop(solver, max_iter: int, tol: float, verbose, eva_iter: int, met
     init_loss = None
     previous_loss = None
     done = 0
-    run_plain = getattr(solver, "run_plain", None)
-    run_pattern = getattr(solver, "run_pattern", None)
-    if tol == 0 and not verbose and history is None and reduce_sums is None and run_pattern is not None:
+    run_many = getattr(solver, "run_many", None)
+    if tol == 0 and not verbose and history is None and reduce_sums is None and run_many is not None:
         # With tol == 0 the stopping rule `(previous - loss) / init < 0 and previous > loss` (methods.py:187) can
         # never fire and nothing displays the metric: the evaluations are still computed at the reference's cadence
         # (the fused epilogue runs on the same iterations) but the host does not wait for the two sums.
-        run_many = getattr(solver, "run_many", None)
-        if run_many is not None:
-            run_many(max_iter, 0, eva_iter)
-            return max_iter
-        i = 0
-        while i < max_iter:
-            n = min(eva_iter, max_iter - i)
-            run_pattern(tuple((i + k) % eva_iter == eva_iter - 1 for k in range(n)))
-            i += n
+        run_many(max_iter, 0, eva_iter)
         return max_iter
     with tqdm(total=max_iter, disable=not verbose) as pbar:
         i = 0
         while i < max_iter:
-            if i % eva_iter != eva_iter - 1 and run_plain is not None:
-                # the iterations up to the next evaluation (or the end) in one go
-                n = min(eva_iter - 1 - i % eva_iter, max_iter - i)
-                run_plain(n)
-                i += n
+            if not evaluates(i, eva_iter):
+                if run_many is None:
+                    solver.step()
+                    i += 1
+                else:
+                    # the iterations up to the next evaluation (or the end) in one go
+                    n = min(eva_iter - 1 - i % eva_iter, max_iter - i)
+                    run_many(n, i, eva_iter, evaluate=False)
+                    i += n
                 done = i
                 continue
-            if i % eva_iter == eva_iter - 1:
-                d, e = solver.step(evaluate=True)
-                if reduce_sums is not None:
-                    d, e = reduce_sums(d, e)
-                done = i + 1
-                bar[metric] = metric_value(metric, d, e, solver.g)
-                l2_loss = d / solver.n_bins_total
-                if history is not None:
-                    history.append((i, bar[metric], l2_loss))
-                pbar.set_postfix(**bar, loss=l2_loss)
-                pbar.update(eva_iter)
-                if not init_loss:
-                    init_loss = l2_loss
-                elif (previous_loss - l2_loss) / init_loss < tol and previous_loss > l2_loss:
-                    break
-                previous_loss = l2_loss
-            else:
-                solver.step()
-                done = i + 1
+            d, e = solver.step(evaluate=True)
+            if reduce_sums is not None:
+                d, e = reduce_sums(d, e)
+            done = i + 1
+            bar[metric] = metric_value(metric, d, e, solver.g)
+            l2_loss = d / solver.n_bins_total
+            if history is not None:
+                history.append((i, bar[metric], l2_loss))
+            pbar.set_postfix(**bar, loss=l2_loss)
+            pbar.update(eva_iter)
+            if not init_loss:
+                init_loss = l2_loss
+            elif (previous_loss - l2_loss) / init_loss < tol and previous_loss > l2_loss:
+                break
+            previous_loss = l2_loss
             i += 1
     return done

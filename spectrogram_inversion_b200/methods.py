@@ -3,7 +3,6 @@
 from __future__ import annotations
 
 import math
-import os
 
 import torch
 from tqdm import tqdm
@@ -89,8 +88,8 @@ def _pipeline_chunks(spec: torch.Tensor, tol: float, verbose, state_arrays: int 
     if spec.is_cuda or len(spec.shape) != 3 or tol != 0 or verbose:
         return 1
     B, F, T = spec.shape
-    cap = int(os.environ.get("SPECINV_HOST_CHUNKS", "4"))         # measured: tools/e2e_chunks.py
-    n = int(max(1, min(cap, B, (B * T) // 60000)))
+    # at most 4 chunks: 4 / 6 / 8 / 16 measured within noise of each other at cfg2 (DESIGN.md section 7)
+    n = int(max(1, min(4, B, (B * T) // 60000)))
     # ... and small enough for the device: a chunk holds its input, the magnitudes, the ping-pong state (two complex
     # arrays for Griffin-Lim, four for ADMM) and two signals; keep that within 80 % of the free memory
     per_signal = F * T * spec.element_size() * (2 if not spec.is_complex() else 1) * (1 + 0.5 + 2 * state_arrays + 1)
@@ -98,7 +97,7 @@ def _pipeline_chunks(spec: torch.Tensor, tol: float, verbose, state_arrays: int 
         return n
     dev = compute_device(spec)
     # cudaMemGetInfo takes a context-wide lock and was measured to stall this call for 15 - 85 ms now and then
-    # (tools/e2e_trace.py: the whole e2e tail of bench.py).  Ask the driver only when the batch could come anywhere
+    # (the whole e2e tail of bench.py).  Ask the driver only when the batch could come anywhere
     # near the device's memory; otherwise the static total minus torch's own live allocations is estimate enough.
     total = _total_memory(dev)
     if B * per_signal / n > 0.25 * (total - torch.cuda.memory_allocated(dev)):
@@ -119,7 +118,6 @@ def _total_memory(dev: torch.device) -> int:
 
 
 _SIDE_STREAMS = {}
-PIPELINE_TRACE = None      # tools/e2e_trace.py sets a list: per chunk (upload start / end, compute start / end, download end) events
 
 
 def _side_streams(dev: torch.device):
@@ -141,48 +139,22 @@ def _run_host_pipelined(spec, n_chunks, make_solver, max_iter, eva_iter, metric,
     s_in.wait_stream(cur)
     B = spec.shape[0]
     bounds = [(B * k) // n_chunks for k in range(n_chunks + 1)]
-    split = os.environ.get("SPECINV_HOST_SPLIT")          # experiment: relative chunk sizes, e.g. "1,3,3,1"
-    if split:
-        wts = [float(v) for v in split.split(",")]
-        acc, bounds = 0.0, [0]
-        for v in wts:
-            acc += v
-            bounds.append(min(B, max(bounds[-1] + 1, int(round(B * acc / sum(wts))))))
-        bounds[-1] = B
-        n_chunks = len(wts)
-
-    trace = PIPELINE_TRACE
-    marks = {}
-    if trace is not None:
-        import time as _time
-        marks["host"] = [("enter", _time.perf_counter())]
-
-    def mark(name, k, stream):
-        if trace is not None:
-            e = torch.cuda.Event(enable_timing=True)
-            e.record(stream)
-            marks[(name, k)] = e
 
     def stage(k):
         with torch.cuda.stream(s_in):
-            mark("up0", k, s_in)
             t = spec[bounds[k]:bounds[k + 1]].detach().to(dev, non_blocking=True)
             ev = torch.cuda.Event()
             ev.record(s_in)
-            mark("up1", k, s_in)
         return t, ev
 
     out, keep = None, []
     nxt = stage(0)
-    if trace is not None:
-        marks["host"].append(("staged 0", _time.perf_counter()))
     for k in range(n_chunks):
         work, ev = nxt
         if k + 1 < n_chunks:
             nxt = stage(k + 1)
         cur.wait_event(ev)
         work.record_stream(cur)
-        mark("c0", k, cur)
         plan, C, mag = _setup(work, stft_kwargs)
         solver = make_solver(plan, C, mag)
         training_loop(solver, max_iter, 0.0, False, eva_iter, metric)
@@ -191,19 +163,12 @@ def _run_host_pipelined(spec, n_chunks, make_solver, max_iter, eva_iter, metric,
             out = torch.empty((B, x.shape[1]), dtype=x.dtype, pin_memory=spec.is_pinned())
         done = torch.cuda.Event()
         done.record(cur)
-        mark("c1", k, cur)
         with torch.cuda.stream(s_out):
             s_out.wait_event(done)
             out[bounds[k]:bounds[k + 1]].copy_(x, non_blocking=True)
-            mark("dn1", k, s_out)
         keep.append(x)                       # alive until the copy stream has drained
         del plan, C, mag, solver, work
-        if trace is not None:
-            marks["host"].append((f"chunk {k} enqueued", _time.perf_counter()))
     s_out.synchronize()
-    if trace is not None:
-        marks["host"].append(("synchronized", _time.perf_counter()))
-        trace.append((n_chunks, marks))
     return out
 
 

@@ -10,6 +10,7 @@ import torch
 
 import cases
 from oracle import specinv_oracle as O
+from spectrogram_inversion_b200 import engine
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -237,23 +238,20 @@ def test_every_custom_op_has_a_fake_kernel():
         assert _ops.halo_sum(f(B, 96), f(B, 96), f(B, 96)) is None and _ops.fill_padding(x0, 0, 64, L, 0) is None
 
 
-class _FakeSolver:
-    """Records what the host loop asks for (no GPU): loss decreases geometrically."""
+class _FakeSolver(engine._Solver):
+    """The real step / run_many over a launch that records whether it evaluates (no GPU): loss decreases
+    geometrically."""
 
     def __init__(self):
         self.g, self.n_bins_total, self.calls, self.loss = 1.0, 10, [], 1.0
+        self.cur, self.iterations = 0, 0
+        self.sums, self._nosums = torch.zeros(2, dtype=torch.float64), torch.empty(0, dtype=torch.float64)
 
-    def step(self, evaluate=False, read=True):
-        self.calls.append(bool(evaluate))
+    def _launch(self, sums):
+        self.calls.append(sums.numel() > 0)
         self.loss *= 0.9
-        return (self.loss, 1.0) if evaluate and read else None
-
-    def run_pattern(self, flags):
-        for f in flags:
-            self.step(evaluate=f, read=False)
-
-    def run_plain(self, n):
-        self.run_pattern((False,) * n)
+        if sums.numel():
+            sums[0], sums[1] = self.loss, 1.0
 
 
 @pytest.mark.parametrize("max_iter,eva_iter", [(23, 4), (10, 10), (7, 10), (30, 1), (1, 1)])

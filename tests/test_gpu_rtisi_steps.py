@@ -115,8 +115,8 @@ def _canonical(su, st, dtype):
 
 STEP_CASES = [
     dict(n_fft=1024, B=3, T=12, la=3, asym=False, dtype="float32"),
-    dict(n_fft=1024, B=3, T=12, la=3, asym=True, dtype="float32", two_warps=True),      # gl_warp_core_1c.cuh
-    dict(n_fft=1024, B=150, T=10, la=2, asym=False, dtype="float32", two_warps=True),   # two signals per CTA
+    dict(n_fft=1024, B=3, T=12, la=3, asym=True, dtype="float32"),
+    dict(n_fft=1024, B=150, T=10, la=2, asym=False, dtype="float32"),                   # two signals per CTA
     dict(n_fft=1024, B=2, T=12, la=3, asym=True, dtype="float32"),
     dict(n_fft=512, B=4, T=12, la=2, asym=False, dtype="float32"),
     dict(n_fft=2048, B=2, T=10, la=3, asym=False, dtype="float32"),
@@ -130,14 +130,13 @@ STEP_CASES = [
 ]
 
 
-@pytest.mark.parametrize("c", STEP_CASES, ids=lambda c: f"n{c['n_fft']}_B{c['B']}_la{c['la']}_asym{int(c['asym'])}_{c['dtype']}{'_generic' if c.get('generic') else ''}{'_legacy' if c.get('legacy') else ''}{'_two_warps' if c.get('two_warps') else ''}")
+@pytest.mark.parametrize("c", STEP_CASES, ids=lambda c: f"n{c['n_fft']}_B{c['B']}_la{c['la']}_asym{int(c['asym'])}_{c['dtype']}{'_generic' if c.get('generic') else ''}{'_legacy' if c.get('legacy') else ''}")
 def test_one_outer_step_from_the_oracles_state(c, monkeypatch):
     """Outer step i (its max_iter inner iterations j = 0 .. max_iter-1 and the commit) from the ORACLE's state, for
     several i (start-up, steady state, tail where the look-ahead runs past the spectrogram) and max_iter = 1, 2:
     frames to 1e-5 absolute (unit-scale signals) x 4 per extra inner iteration, spectra relative to their scale."""
     monkeypatch.setenv("SPECINV_FORCE_GENERIC", "1" if c.get("generic") else "0")
     monkeypatch.setenv("SPECINV_GENERIC_MR", "0" if c.get("legacy") else "1")
-    monkeypatch.setenv("SPECINV_RTISI_TWO_WARPS", "1" if c.get("two_warps") else "0")
     dtype = np.dtype(c["dtype"])
     f32 = dtype == np.float32
     hop = c["n_fft"] // 4

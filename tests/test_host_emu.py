@@ -11,7 +11,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 NVCC = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
 
 
-@pytest.mark.parametrize("name", ["test_fft_regs", "test_warp_core", "test_warp_core_1c", "test_mixed_radix"])
+@pytest.mark.parametrize("name", ["test_fft_regs", "test_warp_core", "test_mixed_radix"])
 def test_host_emulation(name, tmp_path):
     if not os.path.exists(NVCC):
         pytest.skip("nvcc not available")

@@ -58,10 +58,10 @@ for name in names:
     for _ in range(3):
         solver.step()
     n = min(c["iters"], 20)
-    solver.run_plain(n)          # what training_loop does between evaluations (CUDA graph replay for small problems)
+    solver.run_many(n, 0, 1, evaluate=False)      # what training_loop does between evaluations
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     torch.cuda.synchronize(); e0.record()
-    solver.run_plain(n)
+    solver.run_many(n, 0, 1, evaluate=False)
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / n
     per_bin = (20 if c["alpha"] > 0 else 4) if c["algo"] == "gl" else 36

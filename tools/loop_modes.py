@@ -1,5 +1,5 @@
 """Host / device time of engine.training_loop on a small problem (cfg1 shape): synchronising evaluations (history
-given) or not, iterations replayed from CUDA graphs or launched directly.
+given) or not.
 
     python tools/loop_modes.py
 """
@@ -22,12 +22,11 @@ S = plan.stft(x)
 mag = plan.spec_abs(S)
 
 
-def run(label, graphs, hist, reps=3):
+def run(label, hist, reps=3):
     for r in range(reps):
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         solver = GriffinLimSolver(plan, S, mag, 0.3)
-        solver.use_graphs = graphs
         t1 = time.perf_counter()
         training_loop(solver, 100, 0.0, False, 10, "sc", history=[] if hist else None)
         t2 = time.perf_counter()
@@ -41,7 +40,5 @@ def run(label, graphs, hist, reps=3):
         del solver
 
 
-run("sync evals, graphs", True, True)
-run("sync evals, direct", False, True)
-run("blind evals, graphs", True, False)
-run("blind evals, direct", False, False)
+run("sync evals", True)
+run("blind evals", False)
