@@ -55,7 +55,10 @@ enum { SPECINV_PAD_REFLECT = 0, SPECINV_PAD_CONSTANT = 1, SPECINV_PAD_REPLICATE 
 /* Normalised STFT description == the output of the reference's _args_helper
  * (methods.py:21-91) plus the problem size. */
 typedef struct specinv_desc {
-    int32_t n_fft;       /* 16..8192; odd only with onesided = 0 (RTISI-LA: even, n_fft/2 must factor into 2 .. 13) */
+    int32_t n_fft;       /* 16..32768; odd only with onesided = 0 (RTISI-LA: even, n_fft/2 must factor into 2 .. 13).
+                          * Above 8192 the iterations, STFT and ISTFT need an even n_fft whose half factors into
+                          * 2 .. 13, at most 32768 in fp32 and 16384 in fp64 (SPECINV_ERR_UNSUPPORTED otherwise);
+                          * RTISI-LA stops at 8192 */
     int32_t hop;         /* hop_length, 1..n_fft */
     int32_t n_frames;    /* T */
     int32_t batch;       /* B */

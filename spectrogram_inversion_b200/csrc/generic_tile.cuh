@@ -134,5 +134,8 @@ __device__ __forceinline__ cx_t<T> bin_update(const TileArgs& a, const IO& io, i
 
 // implemented in specinv_generic_mr.cu: SPECINV_ERR_UNSUPPORTED when M = n_fft / 2 has a prime factor > 13
 int mr_tile_launch(int dtype, int op, TileArgs& a, cudaStream_t st);
+// implemented in specinv_generic_stream.cu: the shapes no tile kernel holds; SPECINV_ERR_UNSUPPORTED when one frame does
+// not fit in shared memory, n_fft is odd or M has a prime factor > 13
+int stream_tile_launch(int dtype, int op, TileArgs& a, cudaStream_t st);
 
 }  // namespace specinv

@@ -92,7 +92,7 @@ inline int ilog2(int v) { int l = 0; while ((1 << l) < v) ++l; return l; }
 inline int make_dims(const specinv_desc* d, Dims* o) {
     if (!d) return SPECINV_ERR_INVALID;
     const int N = d->n_fft;
-    if (N < 16 || N > 8192) return SPECINV_ERR_INVALID;
+    if (N < 16 || N > 32768) return SPECINV_ERR_INVALID;
     if ((N & 1) && d->onesided) return SPECINV_ERR_INVALID;   // an odd n_fft only exists two-sided (bin count = n_fft): direct DFT
     if (d->hop < 1 || d->hop > N) return SPECINV_ERR_INVALID;
     if (d->n_frames < 1 || d->batch < 1) return SPECINV_ERR_INVALID;

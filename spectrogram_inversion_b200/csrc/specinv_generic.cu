@@ -329,7 +329,7 @@ static int launch_dft_tile(TileArgs& a, cudaStream_t st) {
 }
 
 template <typename T, int OP>
-static int launch_tile(TileArgs& a, cudaStream_t st) {
+static int launch_tile_kernels(TileArgs& a, cudaStream_t st) {
     const Dims& dm = a.dm;
     // the mixed-radix team kernel (specinv_generic_mr.cu) serves every size whose half factors into 2 .. 13;
     // SPECINV_GENERIC_MR=0 keeps the radix-2^2 CTA-wide kernel / the direct DFT (A/B timing, tests of those kernels)
@@ -366,6 +366,17 @@ static int launch_tile(TileArgs& a, cudaStream_t st) {
     const int threads = bf >= 4096 ? 1024 : bf >= 1024 ? 512 : 256;
     tile_kernel<T, OP><<<grid, threads, smem, st>>>(a);
     return (int)cudaGetLastError();
+}
+
+// The tile kernels keep a whole tile (K halo frames and at least one owned frame) in shared memory and stop at
+// n_fft = 8192; the streamed-frame kernel (specinv_generic_stream.cu) takes every shape they refuse.
+template <typename T, int OP>
+static int launch_tile(TileArgs& a, cudaStream_t st) {
+    if (a.dm.N <= 8192) {
+        const int rc = launch_tile_kernels<T, OP>(a, st);
+        if (rc != SPECINV_ERR_UNSUPPORTED) return rc;
+    }
+    return stream_tile_launch(sizeof(T) == 8 ? SPECINV_F64 : SPECINV_F32, OP, a, st);
 }
 
 static void fill_plan(TileArgs& a, const Dims& dm, int dtype, const void* plan) {

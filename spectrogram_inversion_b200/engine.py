@@ -55,9 +55,11 @@ class StftPlan:
         if args.pad_mode not in _lib.PAD_MODES:
             raise NotImplementedError(f"pad_mode {args.pad_mode!r} is not supported")
         n = args.n_fft
-        if n < 16 or n > 8192:
-            raise NotImplementedError(f"n_fft={n}: the sm_100a kernels need an n_fft in [16, 8192] (sizes whose half "
-                                      "factors into 2 .. 13 run the FFT kernels, other sizes the direct-DFT tile kernel)")
+        top = 16384 if dtype == torch.float64 else 32768
+        if n < 16 or n > top:
+            raise NotImplementedError(f"n_fft={n}: the sm_100a kernels need an n_fft in [16, {top}] in {dtype} "
+                                      "(16384 in float64, 32768 in float32; sizes whose half factors into 2 .. 13 run "
+                                      "the FFT kernels, other sizes up to 8192 the direct-DFT tile kernel)")
         self.args, self.T, self.B, self.dtype, self.device = args, int(n_frames), int(batch), dtype, device
         self.cdtype = _CDT[dtype]
         self.pad_mode = _lib.PAD_MODES[args.pad_mode]
