@@ -271,6 +271,21 @@ int specinv_gl_run_status(const specinv_desc* d, const void* workspace, uint32_t
 int specinv_mel_inverse(int dtype, const void* P, int n_stft, int n_mels, int f_lo, int f_hi, const void* mel,
                         void* out, int batch, int64_t n_frames, void* stream);
 
+/* ---- PGHI: phase-gradient heap integration (csrc/specinv_pghi.cu, spectrogram_inversion_b200.pghi) ---------------
+ * A non-iterative phase for a onesided magnitude, the frame-causal heap integration of Prusa and Holighaus (EUSIPCO
+ * 2017) in its scan formulation (tests/golden/pghi_ref.py): out[b][t][f] = mag[b, f, t] * exp(i phi[b, f, t]).
+ *   mag    real [batch][n_bins][n_frames] with element strides (sb, sf, st), n_bins = n_fft / 2 + 1 (any n_fft >= 2);
+ *   out    complex [batch][n_frames][n_bins] contiguous (frame-major, torch.stft's physical layout);
+ *   hop, win_length (<= n_fft) and gamma (> 0) of the analysis; tol in (0, 1): bins at or below tol * max of their
+ *   signal get phase 0.  Arithmetic is float64 in both dtypes; only the output is rounded.
+ * specinv_pghi_workspace_bytes gives the size of `workspace` (device memory, any content) for a shape; it depends on
+ * the current device's shared memory.  batch <= 65535, n_frames <= INT_MAX.  Every argument is checked before any
+ * launch (SPECINV_ERR_INVALID).  Runs are deterministic. */
+int specinv_pghi_workspace_bytes(int dtype, int batch, int n_bins, int64_t n_frames, size_t* bytes);
+int specinv_pghi(int dtype, const void* mag, int64_t sb, int64_t sf, int64_t st, void* out, int batch, int n_bins,
+                 int64_t n_frames, int n_fft, int hop, int win_length, double gamma, double tol, void* workspace,
+                 size_t workspace_bytes, void* stream);
+
 /* ---- metrics (metrics.py:4-43, F.mse_loss at methods.py:182) ---------------------------------
  * out[0] += sum (a-b)^2, out[1] += sum a^2, out[2] += sum b^2 over n contiguous reals. */
 int specinv_metric_sums(int dtype, const void* a, const void* b, int64_t n, double* out3, void* stream);

@@ -354,3 +354,23 @@ def _fake_mel_inverse(P, mel, out, f_lo, f_hi) -> None:
 # torchaudio_compat.InverseMelScale
 MEL_OPS = (mel_inverse,)
 mel_inverse.register_fake(_fake_mel_inverse)
+
+
+def pghi_direct(mag: Tensor, out: Tensor, n_fft: int, hop: int, win_length: int, gamma: float, tol: float) -> None:
+    """out (B, T, F) complex, contiguous = mag (B, F, T) real, any strides, times e^{i phi} of PGHI (specinv_pghi),
+    called straight through ctypes like `mel_inverse_direct`; the workspace comes from torch's allocator."""
+    _need_cuda(out)
+    if not mag.is_cuda:
+        raise RuntimeError("specinv_b200 ops only run on CUDA tensors (no CPU fallback)")
+    B, F, T = mag.shape
+    if tuple(out.shape) != (B, T, F) or out.dtype != {torch.float32: torch.complex64, torch.float64: torch.complex128}.get(mag.dtype):
+        raise RuntimeError(f"specinv_b200: pghi shapes / dtypes disagree: mag {list(mag.shape)} {mag.dtype}, "
+                           f"out {list(out.shape)} {out.dtype}")
+    dt = _DT[mag.dtype]
+    with torch.cuda.device(out.device):
+        n = C.c_size_t(0)
+        _lib.check(_lib.lib().specinv_pghi_workspace_bytes(dt, B, F, T, C.byref(n)), "pghi_workspace_bytes")
+        ws = torch.empty(int(n.value), dtype=torch.uint8, device=out.device)
+        sb, sf, st = mag.stride()
+        _ok(_lib.lib().specinv_pghi(dt, _p(mag), sb, sf, st, _p(out), B, F, T, int(n_fft), int(hop), int(win_length),
+                                    float(gamma), float(tol), _p(ws), ws.numel(), _stream(out)), "pghi")
