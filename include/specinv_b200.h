@@ -286,6 +286,29 @@ int specinv_pghi(int dtype, const void* mag, int64_t sb, int64_t sf, int64_t st,
                  int64_t n_frames, int n_fft, int hop, int win_length, double gamma, double tol, void* workspace,
                  size_t workspace_bytes, void* stream);
 
+/* ---- PGHI on a stream (csrc/specinv_pghi.cu, spectrogram_inversion_b200.PGHIStream) ------------------------------
+ * Finalises frames a few at a time, from a per-signal state carried between calls.  The threshold is causal: the step
+ * that computes frame n uses thr_n = tol * max(mag[b, :, 0 .. min(n + 1, N - 1)]) (N: the frames of the stream) for
+ * the significance of frames n-1 and n and the logs of n-1, n and n+1; otherwise the arithmetic is specinv_pghi's,
+ * and the frames do not depend on how the stream is cut into calls (tests/golden/pghi_stream_ref.py).
+ *   mag     real rows [batch][n_bins][n_rows], element strides (sb, sf, st): row r is frame frame0 + r.  The rows are
+ *           the frame before the first one finalised (absent when that is frame 0), the n_final frames finalised,
+ *           and, unless `final`, one frame of look-ahead.  So the first frame finalised is
+ *           frame0 + n_rows - n_final - (final ? 0 : 1), and it must be the state's frame count.
+ *   final   1: the last row is the stream's last frame (zero time derivative, as specinv_pghi's last frame).
+ *   state   specinv_pghi_stream_state_bytes bytes (device memory, independent of the frame count): per signal the
+ *           running max, the frame count and the running phase of the last frame finalised (F doubles), and the CTA
+ *           working set when it does not fit in shared memory.  Any content before the call that finalises frame 0,
+ *           which initialises it.  A call whose first frame is not the state's count writes NaN frames and leaves the
+ *           state unchanged.
+ *   out     complex [batch][n_final][n_bins] contiguous (frame-major); may be NULL when n_final == 0 (no launch).
+ *   n_fft, hop, win_length, gamma, tol as for specinv_pghi.
+ * Every argument is checked before any launch (SPECINV_ERR_INVALID).  One launch, one CTA per signal. */
+int specinv_pghi_stream_state_bytes(int dtype, int batch, int n_bins, size_t* bytes);
+int specinv_pghi_stream(int dtype, const void* mag, int64_t sb, int64_t sf, int64_t st, int frame0, int n_rows,
+                        int n_final, int final, void* state, size_t state_bytes, void* out, int batch, int n_bins,
+                        int n_fft, int hop, int win_length, double gamma, double tol, void* stream);
+
 /* ---- metrics (metrics.py:4-43, F.mse_loss at methods.py:182) ---------------------------------
  * out[0] += sum (a-b)^2, out[1] += sum a^2, out[2] += sum b^2 over n contiguous reals. */
 int specinv_metric_sums(int dtype, const void* a, const void* b, int64_t n, double* out3, void* stream);

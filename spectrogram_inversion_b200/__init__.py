@@ -4,8 +4,8 @@ from . import methods, metrics, torchaudio_compat
 from .methods import ADMM, L_BFGS, RTISI_LA, griffin_lim, phase_init
 from .metrics import sc, ser, snr, spectral_convergence
 from .pghi import pghi
-from .streaming import RTISIStream
+from .streaming import PGHIStream, RTISIStream
 
 __version__ = "0.1.0"
-__all__ = ["griffin_lim", "RTISI_LA", "RTISIStream", "ADMM", "L_BFGS", "phase_init", "pghi", "sc", "snr", "ser", "spectral_convergence",
+__all__ = ["griffin_lim", "RTISI_LA", "RTISIStream", "PGHIStream", "ADMM", "L_BFGS", "phase_init", "pghi", "sc", "snr", "ser", "spectral_convergence",
            "methods", "metrics", "torchaudio_compat"]

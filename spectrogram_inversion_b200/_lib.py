@@ -29,6 +29,7 @@ EXPORTS = (
     "specinv_gl_run_workspace_bytes", "specinv_gl_run", "specinv_gl_run_status",
     "specinv_rtisi_state_bytes", "specinv_rtisi_la_steps", "specinv_rtisi_la_stream", "specinv_plan_inv_env_window",
     "specinv_gl_rebuilt_iter", "specinv_mel_inverse", "specinv_pghi_workspace_bytes", "specinv_pghi",
+    "specinv_pghi_stream_state_bytes", "specinv_pghi_stream",
 )
 
 
@@ -89,6 +90,9 @@ def _declare(lib: C.CDLL) -> None:
         "specinv_pghi_workspace_bytes": [C.c_int, C.c_int, C.c_int, i64, C.POINTER(C.c_size_t)],
         "specinv_pghi": [C.c_int, vp, i64, i64, i64, vp, C.c_int, C.c_int, i64, C.c_int, C.c_int, C.c_int, dbl, dbl, vp,
                          C.c_size_t, vp],
+        "specinv_pghi_stream_state_bytes": [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)],
+        "specinv_pghi_stream": [C.c_int, vp, i64, i64, i64, C.c_int, C.c_int, C.c_int, C.c_int, vp, C.c_size_t, vp,
+                                C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, dbl, dbl, vp],
     }
     for name, args in sigs.items():
         fn = getattr(lib, name)

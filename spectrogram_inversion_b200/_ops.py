@@ -374,3 +374,30 @@ def pghi_direct(mag: Tensor, out: Tensor, n_fft: int, hop: int, win_length: int,
         sb, sf, st = mag.stride()
         _ok(_lib.lib().specinv_pghi(dt, _p(mag), sb, sf, st, _p(out), B, F, T, int(n_fft), int(hop), int(win_length),
                                     float(gamma), float(tol), _p(ws), ws.numel(), _stream(out)), "pghi")
+
+
+def pghi_stream_state_bytes(dtype: torch.dtype, batch: int, n_bins: int) -> int:
+    n = C.c_size_t(0)
+    _lib.check(_lib.lib().specinv_pghi_stream_state_bytes(_DT[dtype], int(batch), int(n_bins), C.byref(n)),
+               "pghi_stream_state_bytes")
+    return int(n.value)
+
+
+def pghi_stream_direct(mag: Tensor, frame0: int, n_final: int, final: bool, state: Tensor, out: Tensor, n_fft: int,
+                       hop: int, win_length: int, gamma: float, tol: float) -> None:
+    """Finalise n_final frames of a PGHI stream (specinv_pghi_stream): mag (B, F, n_rows) real, any strides, row r is
+    frame frame0 + r; out (B, n_final, F) complex, contiguous; state from `pghi_stream_state_bytes`.  Straight
+    through ctypes like `pghi_direct`."""
+    _need_cuda(state, out)
+    if not mag.is_cuda:
+        raise RuntimeError("specinv_b200 ops only run on CUDA tensors (no CPU fallback)")
+    B, F, R = mag.shape
+    if tuple(out.shape) != (B, n_final, F) or out.dtype != {torch.float32: torch.complex64, torch.float64: torch.complex128}.get(mag.dtype):
+        raise RuntimeError(f"specinv_b200: pghi_stream shapes / dtypes disagree: mag {list(mag.shape)} {mag.dtype}, "
+                           f"out {list(out.shape)} {out.dtype}")
+    sb, sf, st = mag.stride()
+    with torch.cuda.device(out.device):
+        _ok(_lib.lib().specinv_pghi_stream(_DT[mag.dtype], _p(mag), sb, sf, st, int(frame0), R, int(n_final),
+                                           int(bool(final)), _p(state), state.numel(), _p(out), B, F, int(n_fft),
+                                           int(hop), int(win_length), float(gamma), float(tol), _stream(out)),
+            "pghi_stream", 1 if n_final else 0)

@@ -14,6 +14,8 @@
 //   pghi_frames_kernel<T, 1>   compose the per-frame maps of a chunk (all chunks but the last)
 //   pghi_carry_kernel          running phase at the start of every chunk, sequentially over the chunks
 //   pghi_frames_kernel<T, 0>   recompute the per-frame maps, integrate from the chunk's start, write mag * e^{i phi}
+//   pghi_stream_kernel<T>      the stream mode (frames_body<T, 2>): one CTA per signal finalises the frames of one
+//                              push from the state of the last one, with the causal threshold (DESIGN.md section 3.7.1)
 #include <limits.h>
 #include <math.h>
 
@@ -155,24 +157,60 @@ __global__ void __launch_bounds__(NT) pghi_max_kernel(Params p, const T* __restr
     }
 }
 
-// MODE 0: apply (write mag * e^{i phi} for the chunk's frames); MODE 1: compose the chunk's per-frame maps.
+// One call of the stream mode (MODE 2, pghi_stream_kernel): the magnitude rows are frames frame0 + r, r < p.T - frame0
+// (p.T is the end of the frames seen so far); frames [first, first + n_fin) are finalised.  state: StreamHead, then
+// the running phase [F] (StreamState); out: [B][n_fin][F].
+struct Stream { int frame0, first, n_fin; };
+struct StreamHead { double max; long long count; };      // running max of the frames read, frames final so far
+
+__host__ __device__ inline size_t stream_row_bytes(int F) { return al16(sizeof(StreamHead) + (size_t)F * 8); }
+
+// Block-wide max; every thread gets it.  red: NW doubles, free until the next __syncthreads.
+__device__ __forceinline__ double block_max(double v, double* red) {
+#pragma unroll
+    for (int d = 16; d; d >>= 1) v = fmax(v, __shfl_xor_sync(~0u, v, d));
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+    __syncthreads();
+    for (int k = 0; k < NW; ++k) v = fmax(v, red[k]);
+    return v;
+}
+
+// MODE 0: apply (write mag * e^{i phi} for the chunk's frames); MODE 1: compose the chunk's per-frame maps;
+// MODE 2: apply for a stream, with the causal threshold thr_n = tol * max(frames 0 .. n + 1) (DESIGN.md section 3.7.1).
 template <typename T, int MODE>
-__global__ void __launch_bounds__(NT) pghi_frames_kernel(Params p, const T* __restrict__ mag,
-                                                         const unsigned long long* __restrict__ maxbits,
-                                                         const double* __restrict__ phi_start, int* __restrict__ map_g,
-                                                         double* __restrict__ map_c, cx_t<T>* __restrict__ out,
-                                                         char* __restrict__ scratch) {
+__device__ __forceinline__ void frames_body(Params p, const T* __restrict__ mag,
+                                            const unsigned long long* __restrict__ maxbits,
+                                            const double* __restrict__ phi_start, int* __restrict__ map_g,
+                                            double* __restrict__ map_c, cx_t<T>* __restrict__ out,
+                                            char* __restrict__ scratch, Stream sm, char* __restrict__ state) {
     extern __shared__ __align__(16) char smem[];
     __shared__ Reach<T> wrf[NW], wrb[NW];
     __shared__ Seg wsf[NW], wsb[NW];
     const int F = p.F, tid = threadIdx.x;
-    const int per_signal = MODE ? p.chunks - 1 : p.chunks;
+    const int per_signal = MODE == 2 ? 1 : MODE ? p.chunks - 1 : p.chunks;
     const int b = blockIdx.x / per_signal, chunk = blockIdx.x % per_signal;
-    const int ta = chunk * p.chunk_len, tb = min(p.T, ta + p.chunk_len);
+    const int ta = MODE == 2 ? sm.first : chunk * p.chunk_len;
+    const int tb = MODE == 2 ? sm.first + sm.n_fin : min(p.T, ta + p.chunk_len);
     Work<T> wk;
     work_bytes<T>(F, &wk, scratch ? scratch + (size_t)blockIdx.x * p.cta_bytes : smem);
     const T* mb = mag + (long long)b * p.sb;
-    const double thr = p.tol * __longlong_as_double((long long)maxbits[b]);
+    StreamHead* head = nullptr;
+    double* st_phase = nullptr;
+    double runmax = 0.0;
+    __shared__ double red[MODE == 2 ? NW : 1];
+    if (MODE == 2) {
+        head = (StreamHead*)(state + (size_t)b * stream_row_bytes(F));
+        st_phase = (double*)(head + 1);
+        if (ta > 0) {
+            if (head->count != ta) {           // not this stream's next call: refuse visibly, leave the state
+                for (int i = tid; i < sm.n_fin * F; i += NT)
+                    out[(long long)b * sm.n_fin * F + i] = mk<T>(T(NAN), T(NAN));
+                return;
+            }
+            runmax = head->max;
+        }
+    }
+    double thr = MODE == 2 ? 0.0 : p.tol * __longlong_as_double((long long)maxbits[b]);
     const int P = (F + NT - 1) / NT, lo = min(F, tid * P), hi = min(F, lo + P);
     const long long chunk_row = ((long long)b * p.chunks + chunk) * F;
 
@@ -186,18 +224,43 @@ __global__ void __launch_bounds__(NT) pghi_frames_kernel(Params p, const T* __re
             wk.s[r * F + m] = log(fmax((double)v, thr));
         }
     };
+    // stream mode: the magnitudes first (their max moves the threshold), the logs once the threshold is known
+    auto load_mag = [&](int n) {
+        const int r = slot(n);
+        double mx = 0.0;                   // magnitudes are >= 0; NaN never wins a comparison
+        for (int m = tid; m < F; m += NT) {
+            const T v = __ldg(mb + (long long)m * p.sf + (long long)(n - sm.frame0) * p.st);
+            wk.mag[r * F + m] = v;
+            if ((double)v > mx) mx = (double)v;
+        }
+        return mx;
+    };
+    auto relog = [&](int n) {              // own bins only: the same threads wrote them in load_mag
+        const int r = slot(n);
+        for (int m = tid; m < F; m += NT) wk.s[r * F + m] = log(fmax((double)wk.mag[r * F + m], thr));
+    };
     // ping-pong: the phase (apply) or the composed map (compose) up to frame n-1, and the one being built
     double *ph0 = wk.ph[0], *ph1 = wk.ph[1];
     int *g0 = wk.g[0], *g1 = wk.g[1];
     for (int m = tid; m < F; m += NT) {
-        if (MODE) { g0[m] = m; ph0[m] = 0.0; }
+        if (MODE == 2) ph0[m] = ta > 0 ? st_phase[m] : 0.0;
+        else if (MODE) { g0[m] = m; ph0[m] = 0.0; }
         else ph0[m] = p.chunks > 1 ? phi_start[chunk_row + m] : 0.0;
     }
-    if (ta > 0) load(ta - 1);
-    load(ta);
+    if (MODE == 2) {
+        double mx = load_mag(ta);
+        if (ta > 0) mx = fmax(mx, load_mag(ta - 1));
+        runmax = block_max(fmax(runmax, mx), red);
+        thr = p.tol * runmax;
+        if (ta > 0) relog(ta - 1);
+        relog(ta);
+    } else {
+        if (ta > 0) load(ta - 1);
+        load(ta);
+    }
     auto write_out = [&](int n, const double* ph) {
         const T* mg = wk.mag + slot(n) * F;
-        cx_t<T>* o = out + ((long long)b * p.T + n) * F;
+        cx_t<T>* o = MODE == 2 ? out + ((long long)b * sm.n_fin + (n - ta)) * F : out + ((long long)b * p.T + n) * F;
         for (int m = tid; m < F; m += NT) {
             double sn, cs;
             sincos(ph[m], &sn, &cs);
@@ -207,8 +270,20 @@ __global__ void __launch_bounds__(NT) pghi_frames_kernel(Params p, const T* __re
     };
 
     for (int n = ta; n < tb; ++n) {
-        if (!MODE && n > ta) write_out(n - 1, ph0);
-        if (n + 1 < p.T) load(n + 1);
+        if (MODE != 1 && n > ta) write_out(n - 1, ph0);
+        if (MODE == 2) {
+            // thr_n: fold frame n+1 into the running max; the ring's logs change only when the threshold does
+            const double mx = block_max(fmax(runmax, n + 1 < p.T ? load_mag(n + 1) : 0.0), red);
+            if (mx != runmax) {
+                runmax = mx;
+                thr = p.tol * runmax;
+                if (n > 0) relog(n - 1);
+                relog(n);
+            }
+            if (n + 1 < p.T) relog(n + 1);
+        } else if (n + 1 < p.T) {
+            load(n + 1);
+        }
         __syncthreads();
         const T* mp = wk.mag + slot(n - 1) * F;      // not read in frame 0
         const T* mc = wk.mag + slot(n) * F;
@@ -297,7 +372,11 @@ __global__ void __launch_bounds__(NT) pghi_frames_kernel(Params p, const T* __re
         { double* t = ph0; ph0 = ph1; ph1 = t; }
         { int* t = g0; g0 = g1; g1 = t; }
     }
-    if (MODE) {
+    if (MODE == 2) {
+        if (tb > ta) write_out(tb - 1, ph0);
+        for (int m = tid; m < F; m += NT) st_phase[m] = ph0[m];
+        if (tid == 0) *head = StreamHead{runmax, (long long)tb};
+    } else if (MODE) {
         for (int m = tid; m < F; m += NT) {
             map_g[chunk_row + m] = g0[m];
             map_c[chunk_row + m] = ph0[m];
@@ -305,6 +384,23 @@ __global__ void __launch_bounds__(NT) pghi_frames_kernel(Params p, const T* __re
     } else {
         write_out(tb - 1, ph0);
     }
+}
+
+template <typename T, int MODE>
+__global__ void __launch_bounds__(NT) pghi_frames_kernel(Params p, const T* __restrict__ mag,
+                                                         const unsigned long long* __restrict__ maxbits,
+                                                         const double* __restrict__ phi_start, int* __restrict__ map_g,
+                                                         double* __restrict__ map_c, cx_t<T>* __restrict__ out,
+                                                         char* __restrict__ scratch) {
+    frames_body<T, MODE>(p, mag, maxbits, phi_start, map_g, map_c, out, scratch, Stream{}, nullptr);
+}
+
+// One CTA per signal: finalise frames [sm.first, sm.first + sm.n_fin) of a stream (specinv_pghi_stream).
+template <typename T>
+__global__ void __launch_bounds__(NT) pghi_stream_kernel(Params p, const T* __restrict__ mag, Stream sm,
+                                                         char* __restrict__ state, cx_t<T>* __restrict__ out,
+                                                         char* __restrict__ scratch) {
+    frames_body<T, 2>(p, mag, nullptr, nullptr, nullptr, nullptr, out, scratch, sm, state);
 }
 
 // phi_start[b][k] = the running phase of frame k * chunk_len - 1 (zero for k = 0), through the composed maps.
@@ -329,14 +425,23 @@ struct Layout {
     size_t cta_bytes, off_maps_g, off_maps_c, off_phi, off_scratch, total;
 };
 
-template <typename T> static int layout(int B, int F, int T_, Layout* L) {
-    L->cta_bytes = work_bytes<T>(F, nullptr, nullptr);
+// Whether a CTA's working set (cta_bytes) exceeds the current device's shared memory and lives in global memory.
+// static_extra: static shared memory of the kernel beyond the scan buffers (the stream mode's block max).
+template <typename T> static int global_work(int F, size_t static_extra, size_t* cta_bytes, bool* global) {
+    *cta_bytes = work_bytes<T>(F, nullptr, nullptr);
     int dev = 0, smem_optin = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
     if (e != cudaSuccess) return (int)e;
-    const size_t static_smem = 2 * NW * (sizeof(Reach<T>) + sizeof(Seg));
-    L->global_work = L->cta_bytes + static_smem > (size_t)smem_optin;
+    const size_t static_smem = 2 * NW * (sizeof(Reach<T>) + sizeof(Seg)) + static_extra;
+    *global = *cta_bytes + static_smem > (size_t)smem_optin;
+    return 0;
+}
+
+template <typename T> static int layout(int B, int F, int T_, Layout* L) {
+    int rc = global_work<T>(F, 0, &L->cta_bytes, &L->global_work);
+    if (rc) return rc;
+    cudaError_t e;
     int per_sm = 1;
     if (!L->global_work) {
         e = cudaFuncSetAttribute(pghi_frames_kernel<T, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L->cta_bytes);
@@ -405,6 +510,51 @@ static bool valid_sizes(int dtype, int batch, int n_bins, int64_t n_frames) {
            n_frames >= 1 && n_frames <= INT_MAX;
 }
 
+// Stream state: [batch] rows of StreamHead + running phase, then, when the working set does not fit in shared memory,
+// [batch] CTA working sets.
+template <typename T> static int stream_state_bytes(int B, int F, size_t* bytes, size_t* cta_bytes, bool* global) {
+    const int rc = global_work<T>(F, NW * sizeof(double), cta_bytes, global);
+    if (rc) return rc;
+    *bytes = (size_t)B * stream_row_bytes(F) + (*global ? (size_t)B * *cta_bytes : 0);
+    return 0;
+}
+
+template <typename T>
+static int run_stream(Params p, const void* mag, Stream sm, char* state, size_t state_bytes, void* out,
+                      cudaStream_t st) {
+    size_t need = 0;
+    bool global = false;
+    int rc = stream_state_bytes<T>(p.B, p.F, &need, &p.cta_bytes, &global);
+    if (rc) return rc;
+    if (state_bytes < need) return SPECINV_ERR_INVALID;
+    if (sm.n_fin == 0) return SPECINV_OK;
+    char* scratch = global ? state + (size_t)p.B * stream_row_bytes(p.F) : nullptr;
+    const size_t dyn = global ? 0 : p.cta_bytes;
+    if (!global) {
+        const cudaError_t e = cudaFuncSetAttribute(pghi_stream_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                                   (int)dyn);
+        if (e != cudaSuccess) return (int)e;
+    }
+    pghi_stream_kernel<T><<<p.B, NT, dyn, st>>>(p, (const T*)mag, sm, state, (cx_t<T>*)out, scratch);
+    return (int)cudaGetLastError();
+}
+
+static bool valid_analysis(int n_bins, int n_fft, int hop, int win_length, double gamma, double tol) {
+    return n_fft >= 2 && n_fft / 2 + 1 == n_bins && hop >= 1 && win_length >= 1 && win_length <= n_fft &&
+           gamma > 0.0 && gamma < INFINITY && tol > 0.0 && tol < 1.0;
+}
+
+static Params analysis_params(int batch, int n_bins, int n_fft, int hop, int win_length, double gamma, double tol) {
+    Params p{};
+    p.B = batch; p.F = n_bins; p.M = n_fft; p.hop = hop;
+    p.tol = tol;
+    const double c = (n_fft - win_length) / 2 + win_length / 2.0;      // window centre inside the frame
+    p.K0 = 2 * PI * c / n_fft;
+    p.K1 = (double)hop * n_fft / gamma;
+    p.K2 = gamma / ((double)n_fft * hop);
+    return p;
+}
+
 }  // namespace pghi
 }  // namespace specinv
 
@@ -426,20 +576,46 @@ int specinv_pghi(int dtype, const void* mag, int64_t sb, int64_t sf, int64_t st,
                  size_t workspace_bytes, void* stream) {
     using namespace specinv::pghi;
     if (!valid_sizes(dtype, batch, n_bins, n_frames) || !mag || !out || !workspace) return SPECINV_ERR_INVALID;
-    if (n_fft < 2 || n_fft / 2 + 1 != n_bins || hop < 1 || win_length < 1 || win_length > n_fft)
-        return SPECINV_ERR_INVALID;
-    if (!(gamma > 0.0) || !(gamma < INFINITY) || !(tol > 0.0 && tol < 1.0)) return SPECINV_ERR_INVALID;
-    Params p{};
-    p.B = batch; p.F = n_bins; p.T = (int)n_frames; p.M = n_fft; p.hop = hop;
+    if (!valid_analysis(n_bins, n_fft, hop, win_length, gamma, tol)) return SPECINV_ERR_INVALID;
+    Params p = analysis_params(batch, n_bins, n_fft, hop, win_length, gamma, tol);
+    p.T = (int)n_frames;
     p.sb = sb; p.sf = sf; p.st = st;
-    p.tol = tol;
-    const double c = (n_fft - win_length) / 2 + win_length / 2.0;      // window centre inside the frame
-    p.K0 = 2 * PI * c / n_fft;
-    p.K1 = (double)hop * n_fft / gamma;
-    p.K2 = gamma / ((double)n_fft * hop);
     cudaStream_t s = (cudaStream_t)stream;
     return dtype == SPECINV_F64 ? run<double>(p, mag, out, (char*)workspace, workspace_bytes, s)
                                 : run<float>(p, mag, out, (char*)workspace, workspace_bytes, s);
+}
+
+int specinv_pghi_stream_state_bytes(int dtype, int batch, int n_bins, size_t* bytes) {
+    using namespace specinv::pghi;
+    if (!bytes || !valid_sizes(dtype, batch, n_bins, 1)) return SPECINV_ERR_INVALID;
+    size_t cta = 0;
+    bool global = false;
+    return dtype == SPECINV_F64 ? stream_state_bytes<double>(batch, n_bins, bytes, &cta, &global)
+                                : stream_state_bytes<float>(batch, n_bins, bytes, &cta, &global);
+}
+
+int specinv_pghi_stream(int dtype, const void* mag, int64_t sb, int64_t sf, int64_t st, int frame0, int n_rows,
+                        int n_final, int final, void* state, size_t state_bytes, void* out, int batch, int n_bins,
+                        int n_fft, int hop, int win_length, double gamma, double tol, void* stream) {
+    using namespace specinv::pghi;
+    if (!valid_sizes(dtype, batch, n_bins, n_rows) || !mag || !state || (n_final > 0 && !out)) return SPECINV_ERR_INVALID;
+    if (!valid_analysis(n_bins, n_fft, hop, win_length, gamma, tol)) return SPECINV_ERR_INVALID;
+    // rows: the frame before the first one finalised (unless that is frame 0), the n_final frames, and one frame of
+    // look-ahead unless `final`
+    const int ahead = final ? 0 : 1;
+    if ((final != 0 && final != 1) || frame0 < 0 || n_final < 0 || n_rows - n_final - ahead < 0 ||
+        (long long)frame0 + n_rows > INT_MAX)
+        return SPECINV_ERR_INVALID;
+    const int first = frame0 + n_rows - n_final - ahead;
+    if (first > 0 && first - 1 < frame0) return SPECINV_ERR_INVALID;
+    Params p = analysis_params(batch, n_bins, n_fft, hop, win_length, gamma, tol);
+    p.T = frame0 + n_rows;
+    p.chunks = 1;
+    p.sb = sb; p.sf = sf; p.st = st;
+    const Stream sm{frame0, first, n_final};
+    cudaStream_t s = (cudaStream_t)stream;
+    return dtype == SPECINV_F64 ? run_stream<double>(p, mag, sm, (char*)state, state_bytes, out, s)
+                                : run_stream<float>(p, mag, sm, (char*)state, state_bytes, out, s);
 }
 
 }  // extern "C"

@@ -1,16 +1,20 @@
-"""Streaming RTISI-LA: magnitude frames in as they are produced, final samples out as soon as they are final."""
+"""Streaming RTISI-LA and PGHI: magnitude frames in as they are produced, final samples (or frames) out as soon as
+they are final."""
 from __future__ import annotations
 
+import ctypes as C
 import dataclasses
+import math
 
 import torch
 
-from . import _ops
+from . import _lib, _ops
 from .engine import StftPlan, compute_device
 from .methods import _rtisi_checks
+from .pghi import _CDT, _analysis
 from .stft_args import args_helper
 
-__all__ = ["RTISIStream", "emitted_samples"]
+__all__ = ["RTISIStream", "emitted_samples", "PGHIStream", "pghi_emitted_samples"]
 
 
 def emitted_samples(n_frames: int, n_fft: int, hop: int, look_ahead: int, center: bool) -> int:
@@ -187,4 +191,197 @@ class RTISIStream:
         out = self._emit(x, max(0, self._length(self._n)))
         self._closed = True
         self._plan = self._state = self._hist = self._pending = self._scratch = None
+        return out
+
+
+def pghi_emitted_samples(n_frames: int, n_fft: int, hop: int, center: bool) -> int:
+    """E(n) = clamp((n - 1) * hop - P, 0, L(n)): the samples per signal a PGHIStream with ``output="waveform"`` has
+    returned once n frames have been pushed (P = n_fft // 2 when centred, L(n) = (n - 1) * hop + n_fft - 2P)."""
+    P = n_fft // 2 if center else 0
+    return max(0, min((n_frames - 1) * hop - P, (n_frames - 1) * hop + n_fft - 2 * P))
+
+
+class PGHIStream:
+    r"""PGHI on a spectrogram that arrives a few frames at a time: one frame of look-ahead, no iterations.
+
+    ``PGHIStream(gamma=None, tol=1e-5, output="waveform", **stft_kwargs)``: ``gamma``, ``tol`` and ``stft_kwargs``
+    take ``pghi``'s meaning, defaults and checks.
+
+    * ``push(chunk)``: ``chunk`` holds ``k >= 0`` real magnitude frames, ``(F, k)`` or ``(B, F, k)``, float32 or
+      float64; returns what became final.  The first push fixes F, B, the number of dimensions, the dtype and the
+      device; a later chunk that differs is an ``AssertionError``.
+    * ``flush()``: the rest; the stream is closed afterwards.
+    * ``output="spectrum"``: the complex frames that became final, ``(F, k')`` or ``(B, F, k')``.
+      ``output="waveform"``: their samples, ``(n,)`` or ``(B, n)``, the ISTFT of the frames with the same
+      ``stft_kwargs``.
+
+    Semantics:
+
+    * Frame j is final once frame j+1 has been pushed, or at ``flush()``, where the last frame has a zero time
+      derivative like ``pghi``'s.  After n frames ``output="spectrum"`` has returned ``max(0, n - 1)`` frames, and
+      ``output="waveform"`` exactly ``pghi_emitted_samples(n, ...)`` samples per signal: a sample is final when every
+      frame covering it is.  Returned values never change.
+    * The threshold is causal: the step that computes frame n uses ``tol * max`` over frames ``0 .. n + 1`` (``pghi``
+      uses the whole signal's max).  So the frames do not depend on how the stream is cut into chunks, and they
+      equal ``pghi``'s when a signal's loudest bin lies in frame 0 or 1 (DESIGN.md section 3.7.1).
+    * A CUDA chunk is processed on the current stream and the result is a device tensor, without synchronising; a
+      host chunk gives a host tensor.
+    * Device memory does not grow with the number of frames: the per-signal state, the last two frames, the
+      overlap-add carry of ``n_fft - hop`` samples, a plan of ``(n_fft - 1) // hop + 2`` frames and one push's
+      buffers.
+    * The waveform needs an even n_fft (the ISTFT's sizes: up to 32768 in float32, 16384 in float64) and
+      ``hop_length <= win_length``; otherwise ``NotImplementedError``.
+    * No gradients: a chunk that requires grad raises ``NotImplementedError``.  ``flush()`` before any frame, and
+      ``push`` / ``flush`` after ``flush()``, raise ``RuntimeError``.
+    """
+
+    def __init__(self, gamma=None, tol=1e-5, output="waveform", **stft_kwargs):
+        if not (isinstance(tol, (int, float)) and 0 < tol < 1):
+            raise ValueError(f"PGHIStream: tol={tol} must lie in (0, 1)")
+        if gamma is not None and not (float(gamma) > 0 and math.isfinite(float(gamma))):
+            raise ValueError(f"PGHIStream: gamma={gamma} must be positive and finite")
+        if output not in ("waveform", "spectrum"):
+            raise ValueError(f"PGHIStream: output={output!r} must be 'waveform' or 'spectrum'")
+        if stft_kwargs.get("n_fft") is not None:
+            _analysis(int(stft_kwargs["n_fft"]) // 2 + 1, stft_kwargs)        # refuse bad options before any frame
+        self.gamma, self.tol, self.output = gamma, float(tol), output
+        self._stft_kwargs = stft_kwargs
+        self._n = 0                # frames pushed
+        self._final = 0            # frames final
+        self._started = False
+        self._closed = False
+
+    # ---- set-up at the first push ---------------------------------------------------------------------------
+    def _start(self, chunk: torch.Tensor) -> None:
+        self._ndim, self._F, self._dtype, self._in_device = chunk.dim(), chunk.shape[-2], chunk.dtype, chunk.device
+        self._host = not chunk.is_cuda
+        self._B = chunk.shape[0] if chunk.dim() == 3 else 1
+        n_fft, hop, wl = _analysis(self._F, self._stft_kwargs)
+        gamma = 0.25645 * wl ** 2 if self.gamma is None else float(self.gamma)
+        self._an = (n_fft, hop, wl, gamma)
+        if self.output == "waveform":
+            if n_fft % 2:
+                raise NotImplementedError(f"PGHIStream: output='waveform' needs an even n_fft (got {n_fft}); "
+                                          "output='spectrum' takes any")
+            if hop > wl:
+                raise NotImplementedError(f"PGHIStream: output='waveform' needs hop_length <= win_length "
+                                          f"({hop} > {wl}): the envelope would vanish between frames")
+        self._dev = dev = compute_device(chunk)
+        self._state = torch.empty(_ops.pghi_stream_state_bytes(chunk.dtype, self._B, self._F), dtype=torch.uint8,
+                                  device=dev)
+        self._hist = torch.empty(self._B, self._F, 0, dtype=chunk.dtype, device=dev)     # frames [final - 1, n)
+        if self.output == "waveform":
+            kw = {k: v for k, v in self._stft_kwargs.items() if k != "n_fft"}
+            shape_only = torch.empty(self._B, self._F, 0, dtype=chunk.dtype, device=dev)
+            # a constant pad mode keeps short plans valid for make_dims (as RTISIStream)
+            self._args = dataclasses.replace(args_helper(shape_only, **kw), pad_mode="constant")
+            self._P = self._args.pad
+            # shortest plan whose envelope has head, interior and tail apart: (T0 - 1) * hop >= n_fft
+            self._T0 = (n_fft - 1) // hop + 2
+            self._plan = StftPlan(self._args, self._T0, self._B, chunk.dtype, dev)
+            self._ola = None       # (frames, un-centred unit-envelope plan): plain windowed overlap-add
+            self._carry = torch.zeros(self._B, n_fft - hop, dtype=chunk.dtype, device=dev)
+        self._started = True
+
+    # 1/envelope of output samples [x0, x0 + length), from the T0-frame plan (or a plan of the whole signal when it has
+    # fewer frames): the same gather as RTISIStream's, on the same attributes
+    _inv_env_window = RTISIStream._inv_env_window
+
+    def _check_open(self) -> None:
+        if self._closed:
+            raise RuntimeError("PGHIStream: the stream was flushed and is closed")
+
+    # ---- the steps ---------------------------------------------------------------------------------------------
+    def _frames(self, window: torch.Tensor, frame0: int, n_final: int, final: bool) -> torch.Tensor:
+        """Finalise frames [self._final, self._final + n_final) from magnitude rows frame0 + r: (B, n_final, F)."""
+        n_fft, hop, wl, gamma = self._an
+        out = torch.empty(self._B, n_final, self._F, dtype=_CDT[self._dtype], device=self._dev)
+        if n_final:                # nothing final yet (the window may even be empty)
+            _ops.pghi_stream_direct(window, frame0, n_final, final, self._state, out, n_fft, hop, wl, gamma,
+                                    self.tol)
+        return out
+
+    def _samples(self, frames: torch.Tensor, first: int, final: bool) -> torch.Tensor:
+        """The output samples that frames [first, first + k) finish: overlap-add, carry, 1/envelope, trim."""
+        a = self._args
+        n_fft, hop = a.n_fft, a.hop_length
+        k = frames.shape[1]
+        T = max(k, self._T0)
+        if self._ola is None or self._ola[0] != T:
+            plan = StftPlan(dataclasses.replace(a, center=False), T, self._B, self._dtype, self._dev)
+            with torch.cuda.device(self._dev):
+                _lib.check(_lib.lib().specinv_plan_unit_envelope(plan.desc_ref, C.c_void_p(plan.buf.data_ptr()),
+                                                                 _ops._stream(plan.buf)), "plan_unit_envelope")
+            self._ola = (T, plan)
+        plan = self._ola[1]
+        if k < T:
+            frames = torch.cat([frames, frames.new_zeros(self._B, T - k, self._F)], 1)
+        y = plan.istft(plan.pack(frames.transpose(1, 2)))       # padded samples first * hop + j
+        z = y[:, :(k - 1) * hop + n_fft]
+        z[:, :n_fft - hop] += self._carry
+        if not final:
+            self._carry = z[:, k * hop:].clone()
+            z = z[:, :k * hop]
+        o0 = first * hop - self._P                               # output sample of z[:, 0]
+        o1 = o0 + z.shape[1]
+        if final:
+            o1 = min(o1, a.signal_length(self._n))
+        x0 = max(0, o0)
+        if o1 <= x0:
+            return z[:, :0]
+        return z[:, x0 - o0:o1 - o0] * self._inv_env_window(x0, o1 - x0, self._n if final else -1)
+
+    def _run(self, window: torch.Tensor, frame0: int, n_final: int, final: bool) -> torch.Tensor:
+        first = self._final
+        frames = self._frames(window, frame0, n_final, final)
+        self._final += n_final
+        if self.output == "spectrum":
+            out = frames.transpose(1, 2)
+        elif n_final:
+            out = self._samples(frames, first, final)
+        else:
+            out = torch.empty(self._B, 0, dtype=self._dtype, device=self._dev)
+        if self._ndim == 2:
+            out = out[0]
+        if not self._host:
+            return out
+        host = torch.empty(out.shape, dtype=out.dtype)
+        host.copy_(out)
+        return host
+
+    # ---- public ------------------------------------------------------------------------------------------------
+    def push(self, chunk: torch.Tensor) -> torch.Tensor:
+        """Append k >= 0 magnitude frames, (F, k) or (B, F, k); return the frames or samples that became final."""
+        self._check_open()
+        if chunk.requires_grad:
+            raise NotImplementedError("PGHIStream has no gradient path: detach the magnitude")
+        if chunk.is_complex():
+            raise ValueError("PGHIStream: a chunk must be a real magnitude, not a complex spectrum")
+        if chunk.dtype not in _CDT:
+            raise NotImplementedError(f"PGHIStream: dtype {chunk.dtype} is not supported (float32 / float64 only)")
+        if chunk.dim() not in (2, 3):
+            raise ValueError(f"PGHIStream: a chunk must be (F, k) or (B, F, k), got shape {list(chunk.shape)}")
+        if not self._started:
+            self._start(chunk)
+        assert chunk.dim() == self._ndim and chunk.shape[-2] == self._F, (tuple(chunk.shape), self._ndim, self._F)
+        assert (chunk.shape[0] if chunk.dim() == 3 else 1) == self._B, (tuple(chunk.shape), self._B)
+        assert chunk.dtype == self._dtype and chunk.device == self._in_device, (chunk.dtype, chunk.device)
+        work = (chunk if chunk.dim() == 3 else chunk.unsqueeze(0)).detach().to(self._dev)
+        window = torch.cat([self._hist, work], -1) if work.shape[-1] else self._hist
+        frame0 = self._n - self._hist.shape[-1]
+        self._n += work.shape[-1]
+        n_final = max(0, self._n - 1 - self._final)
+        out = self._run(window, frame0, n_final, False)
+        keep = min(self._n - max(0, self._final - 1), window.shape[-1])
+        self._hist = window[..., window.shape[-1] - keep:].clone()
+        return out
+
+    def flush(self) -> torch.Tensor:
+        """The frames or samples not returned yet; closes the stream."""
+        self._check_open()
+        if self._n == 0:
+            raise RuntimeError("PGHIStream.flush: no frame has been pushed")
+        out = self._run(self._hist, self._n - self._hist.shape[-1], self._n - self._final, True)
+        self._closed = True
+        self._state = self._hist = self._plan = self._ola = self._carry = None
         return out
