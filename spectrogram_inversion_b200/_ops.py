@@ -13,6 +13,8 @@ from . import _lib
 LAUNCHES = [0]
 
 _DT = {torch.float32: _lib.F32, torch.float64: _lib.F64, torch.complex64: _lib.F32, torch.complex128: _lib.F64}
+# the complex dtype of each real dtype the kernels take
+CDT = {torch.float32: torch.complex64, torch.float64: torch.complex128}
 
 
 def _ok(code: int, what: str, kernels: int = 1) -> None:
@@ -363,7 +365,7 @@ def pghi_direct(mag: Tensor, out: Tensor, n_fft: int, hop: int, win_length: int,
     if not mag.is_cuda:
         raise RuntimeError("specinv_b200 ops only run on CUDA tensors (no CPU fallback)")
     B, F, T = mag.shape
-    if tuple(out.shape) != (B, T, F) or out.dtype != {torch.float32: torch.complex64, torch.float64: torch.complex128}.get(mag.dtype):
+    if tuple(out.shape) != (B, T, F) or out.dtype != CDT.get(mag.dtype):
         raise RuntimeError(f"specinv_b200: pghi shapes / dtypes disagree: mag {list(mag.shape)} {mag.dtype}, "
                            f"out {list(out.shape)} {out.dtype}")
     dt = _DT[mag.dtype]
@@ -392,7 +394,7 @@ def pghi_stream_direct(mag: Tensor, frame0: int, n_final: int, final: bool, stat
     if not mag.is_cuda:
         raise RuntimeError("specinv_b200 ops only run on CUDA tensors (no CPU fallback)")
     B, F, R = mag.shape
-    if tuple(out.shape) != (B, n_final, F) or out.dtype != {torch.float32: torch.complex64, torch.float64: torch.complex128}.get(mag.dtype):
+    if tuple(out.shape) != (B, n_final, F) or out.dtype != CDT.get(mag.dtype):
         raise RuntimeError(f"specinv_b200: pghi_stream shapes / dtypes disagree: mag {list(mag.shape)} {mag.dtype}, "
                            f"out {list(out.shape)} {out.dtype}")
     sb, sf, st = mag.stride()

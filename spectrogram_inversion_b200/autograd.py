@@ -15,14 +15,12 @@ with wa / ws the analysis / synthesis windows (their scale ratio is N, or 1 when
 spectra use c = 1 (methods.py:145-146)."""
 from __future__ import annotations
 
-import ctypes as C
 import dataclasses
 import math
 import torch
 import torch.nn.functional as F
 from tqdm import tqdm
 
-from . import _lib, _ops
 from .engine import METRIC_NAMES, StftPlan, metric_value
 from .stft_args import StftArgs
 
@@ -31,12 +29,6 @@ pi2 = 2 * math.pi
 
 def wants_grad(spec: torch.Tensor) -> bool:
     return torch.is_grad_enabled() and spec.requires_grad
-
-
-def _desc_of(plan: StftPlan):
-    a = plan.args
-    return _lib.make_desc(a.n_fft, a.hop_length, plan.T, plan.B, a.center, plan.pad_mode, a.normalized, a.onesided,
-                          _ops._DT[plan.dtype])
 
 
 class Transforms:
@@ -49,15 +41,8 @@ class Transforms:
         self.plan = StftPlan(args, n_frames, batch, dtype, device)          # as the caller sees it
         self.plan_nc = StftPlan(nc, n_frames, batch, dtype, device)         # un-centred, over the padded length
         self.plan_raw = StftPlan(nc, n_frames, batch, dtype, device)        # un-centred, unit envelope: plain OLA
-        d = _desc_of(self.plan_raw)
-        stream = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
-        with torch.cuda.device(device):
-            _lib.check(_lib.lib().specinv_plan_unit_envelope(C.byref(d), C.c_void_p(self.plan_raw.buf.data_ptr()),
-                                                             stream), "plan_unit_envelope")
-            self.env = torch.empty(self.plan.length, dtype=dtype, device=device)
-            d2 = _desc_of(self.plan)
-            _lib.check(_lib.lib().specinv_plan_envelope(C.byref(d2), C.c_void_p(self.plan.buf.data_ptr()),
-                                                        C.c_void_p(self.env.data_ptr()), stream), "plan_envelope")
+        self.plan_raw.set_unit_envelope()
+        self.env = self.plan.envelope()
         n = args.n_fft
         self.ratio = 1.0 if args.normalized else float(n)                   # analysis scale / synthesis scale
         F_ = args.n_bins

@@ -16,8 +16,6 @@ from tqdm import tqdm
 from . import _lib, _ops
 from .stft_args import StftArgs
 
-_CDT = {torch.float32: torch.complex64, torch.float64: torch.complex128}
-
 
 def require_cuda() -> None:
     if not torch.cuda.is_available():
@@ -29,6 +27,16 @@ def compute_device(t: torch.Tensor) -> torch.device:
     """CUDA tensors run in place; host tensors are staged through the current CUDA device."""
     require_cuda()
     return t.device if t.is_cuda else torch.device("cuda", torch.cuda.current_device())
+
+
+def host_copy(x: torch.Tensor, pinned: bool) -> torch.Tensor:
+    """A host copy of device tensor ``x`` for a caller whose input was on the host.  With ``pinned`` (that input was
+    pinned) the copy goes to pinned memory and runs asynchronously; it is complete on return either way, the current
+    stream being synchronised."""
+    out = torch.empty(x.shape, dtype=x.dtype, pin_memory=pinned)
+    out.copy_(x, non_blocking=True)
+    torch.cuda.current_stream(x.device).synchronize()
+    return out
 
 
 @dataclass
@@ -50,7 +58,7 @@ class StftPlan:
     def __init__(self, args: StftArgs, n_frames: int, batch: int, dtype: torch.dtype, device: torch.device,
                  tables: bool = True):
         require_cuda()
-        if dtype not in _CDT:
+        if dtype not in _ops.CDT:
             raise NotImplementedError(f"dtype {dtype} is not supported (float32 / float64 only)")
         if args.pad_mode not in _lib.PAD_MODES:
             raise NotImplementedError(f"pad_mode {args.pad_mode!r} is not supported")
@@ -61,7 +69,7 @@ class StftPlan:
                                       "(16384 in float64, 32768 in float32; sizes whose half factors into 2 .. 13 run "
                                       "the FFT kernels, other sizes up to 8192 the direct-DFT tile kernel)")
         self.args, self.T, self.B, self.dtype, self.device = args, int(n_frames), int(batch), dtype, device
-        self.cdtype = _CDT[dtype]
+        self.cdtype = _ops.CDT[dtype]
         self.pad_mode = _lib.PAD_MODES[args.pad_mode]
         self.length = args.signal_length(self.T)
         self.row = n // 2 if args.onesided else n
@@ -131,6 +139,21 @@ class StftPlan:
         out = out if out is not None else self.empty_signal()
         _ops.istft(self.buf, s.main, s.nyq, out, *self._k)
         return out
+
+    # ---- window envelope -------------------------------------------------------------------
+    def envelope(self) -> torch.Tensor:
+        """The window envelope the ISTFT divides by, one value per sample of the plan's signal (``length``)."""
+        env = torch.empty(self.length, dtype=self.dtype, device=self.device)
+        with torch.cuda.device(self.buf.device):
+            _lib.check(_lib.lib().specinv_plan_envelope(self.desc_ref, _ops._p(self.buf), _ops._p(env),
+                                                        _ops._stream(self.buf)), "plan_envelope")
+        return env
+
+    def set_unit_envelope(self) -> None:
+        """Make the envelope 1 everywhere, so that the plan's ISTFT is a plain windowed overlap-add."""
+        with torch.cuda.device(self.buf.device):
+            _lib.check(_lib.lib().specinv_plan_unit_envelope(self.desc_ref, _ops._p(self.buf), _ops._stream(self.buf)),
+                       "plan_unit_envelope")
 
 
 def spec_sums(a: SplitSpec, b: SplitSpec) -> torch.Tensor:

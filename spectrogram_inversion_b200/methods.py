@@ -8,7 +8,7 @@ import torch
 from tqdm import tqdm
 
 from . import _ops, autograd
-from .engine import ADMMSolver, GriffinLimSolver, METRIC_NAMES, StftPlan, compute_device, training_loop
+from .engine import ADMMSolver, GriffinLimSolver, METRIC_NAMES, StftPlan, compute_device, host_copy, training_loop
 from .stft_args import args_helper, real_dtype_of
 
 __all__ = ["griffin_lim", "RTISI_LA", "ADMM", "L_BFGS", "phase_init"]
@@ -70,13 +70,7 @@ def _finish(x: torch.Tensor, spec: torch.Tensor) -> torch.Tensor:
     """methods.py:267-270: drop the batch dim unless the input was (1, F, T)."""
     if not (spec.shape[0] == 1 and len(spec.shape) == 3):
         x = x.squeeze(0)
-    if spec.is_cuda:
-        return x.clone()
-    # host caller: device -> host copy (pinned + asynchronous when the input was pinned)
-    out = torch.empty(x.shape, dtype=x.dtype, pin_memory=spec.is_pinned())
-    out.copy_(x, non_blocking=True)
-    torch.cuda.current_stream(x.device).synchronize()
-    return out
+    return x.clone() if spec.is_cuda else host_copy(x, spec.is_pinned())
 
 
 def _pipeline_chunks(spec: torch.Tensor, tol: float, verbose, state_arrays: int = 1) -> int:

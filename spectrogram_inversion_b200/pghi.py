@@ -17,8 +17,6 @@ from .engine import compute_device
 
 __all__ = ["pghi"]
 
-_CDT = {torch.float32: torch.complex64, torch.float64: torch.complex128}
-
 
 def _analysis(n_bins: int, stft_kwargs: dict):
     """(n_fft, hop, win_length) of a onesided spectrum: the defaults and the onesided rule of ``args_helper``
@@ -71,7 +69,7 @@ def pghi(spec, gamma=None, tol=1e-5, **stft_kwargs):
         raise ValueError("pghi: spec must be a real magnitude, not a complex spectrum")
     if spec.requires_grad and torch.is_grad_enabled():
         raise NotImplementedError("pghi has no gradient path: detach the magnitude or call it under torch.no_grad()")
-    if spec.dtype not in _CDT:
+    if spec.dtype not in _ops.CDT:
         raise NotImplementedError(f"pghi: dtype {spec.dtype} is not supported (float32 / float64 only)")
     if spec.dim() < 2:
         raise ValueError(f"pghi: spec must be (..., F, T), got shape {list(spec.shape)}")
@@ -86,7 +84,7 @@ def pghi(spec, gamma=None, tol=1e-5, **stft_kwargs):
     dev = compute_device(spec)
     m = spec.detach().to(dev).reshape(-1, F, T)
     B = m.shape[0]
-    out = torch.empty(B, T, F, dtype=_CDT[spec.dtype], device=dev)
+    out = torch.empty(B, T, F, dtype=_ops.CDT[spec.dtype], device=dev)
     if B and T:
         _ops.pghi_direct(m, out, n_fft, hop, win_length, gamma, float(tol))
     return out.transpose(1, 2).reshape(shape).to(spec.device)

@@ -2,16 +2,15 @@
 they are final."""
 from __future__ import annotations
 
-import ctypes as C
 import dataclasses
 import math
 
 import torch
 
-from . import _lib, _ops
-from .engine import StftPlan, compute_device
+from . import _ops
+from .engine import StftPlan, compute_device, host_copy
 from .methods import _rtisi_checks
-from .pghi import _CDT, _analysis
+from .pghi import _analysis
 from .stft_args import args_helper
 
 __all__ = ["RTISIStream", "emitted_samples", "PGHIStream", "pghi_emitted_samples"]
@@ -25,7 +24,105 @@ def emitted_samples(n_frames: int, n_fft: int, hop: int, look_ahead: int, center
     return max(0, min((n_frames - LA) * hop - P, (n_frames - 1) * hop + n_fft - 2 * P))
 
 
-class RTISIStream:
+def pghi_emitted_samples(n_frames: int, n_fft: int, hop: int, center: bool) -> int:
+    """E(n) = clamp((n - 1) * hop - P, 0, L(n)): the samples per signal a PGHIStream with ``output="waveform"`` has
+    returned once n frames have been pushed (P = n_fft // 2 when centred, L(n) = (n - 1) * hop + n_fft - 2P).  That is
+    ``emitted_samples`` with a look-ahead of one frame."""
+    return emitted_samples(n_frames, n_fft, hop, 1, center)
+
+
+class _FrameStream:
+    """The push / flush protocol of the frame streams.  The first chunk fixes the number of dimensions, F, B, the dtype
+    and the device of every later one; the frames a step still needs are kept on the compute device between pushes;
+    results go back as the chunks came (host or CUDA, with or without the batch dimension).
+
+    A subclass defines ``_start(chunk)``, its set-up at the first push, which calls ``_capture`` (and
+    ``_start_envelope`` when it needs 1/envelope windows), and ``_last()``, the final step of ``flush()``, which
+    returns what was not returned yet and drops the subclass's own buffers."""
+
+    def __init__(self, stft_kwargs: dict):
+        self._stft_kwargs = stft_kwargs
+        self._n = 0                # frames pushed
+        self._started = False
+        self._closed = False
+
+    def _check_open(self) -> None:
+        if self._closed:
+            raise RuntimeError(f"{type(self).__name__}: the stream was flushed and is closed")
+
+    # ---- set-up at the first push ---------------------------------------------------------------------------
+    def _capture(self, chunk: torch.Tensor) -> None:
+        self._ndim, self._F, self._dtype, self._in_device = chunk.dim(), chunk.shape[-2], chunk.dtype, chunk.device
+        self._B = chunk.shape[0] if chunk.dim() == 3 else 1
+        self._host = not chunk.is_cuda
+        self._pinned = self._host and chunk.is_pinned()
+        self._dev = compute_device(chunk)
+        self._hist = torch.empty(self._B, self._F, 0, dtype=self._dtype, device=self._dev)   # frames kept
+
+    def _start_envelope(self, stft_kwargs: dict) -> None:
+        """The STFT arguments and the plan that ``_inv_env_window`` gathers from."""
+        shape_only = torch.empty(self._B, self._F, 0, dtype=self._dtype, device=self._dev)
+        # no stream pads a signal: a constant pad mode keeps short plans (a flush of a few frames) valid for make_dims
+        self._args = a = dataclasses.replace(args_helper(shape_only, **stft_kwargs), pad_mode="constant")
+        self._P = a.pad
+        # shortest plan whose envelope has head, interior and tail apart: (T0 - 1) * hop >= n_fft
+        self._T0 = (a.n_fft - 1) // a.hop_length + 2
+        self._plan = StftPlan(a, self._T0, self._B, self._dtype, self._dev)
+
+    def _inv_env_window(self, x0: int, length: int, total_frames: int = -1) -> torch.Tensor:
+        """1/envelope of samples [x0, x0 + length) of the signal (total_frames -1: not known yet), gathered from the
+        short plan, or from a plan of the whole signal when it has fewer than T0 frames."""
+        a = self._args
+        out = torch.empty(length, dtype=self._dtype, device=self._dev)
+        if 0 <= total_frames < self._T0:
+            plan = StftPlan(a, total_frames, self._B, self._dtype, self._dev)
+        else:
+            plan = self._plan
+        _ops.plan_inv_env_window(plan.buf, out, x0, total_frames, a.n_fft, a.hop_length, plan.T, a.center,
+                                 a.normalized, a.onesided)
+        return out
+
+    # ---- every push ------------------------------------------------------------------------------------------
+    def _append(self, chunk: torch.Tensor):
+        """Set the stream up at the first chunk, check a later one against it, and append its frames to the kept
+        ones: returns (window, frame0), window (B, F, rows) on the compute device with row r holding frame
+        frame0 + r."""
+        if not self._started:
+            self._start(chunk)
+            self._started = True
+        assert chunk.dim() == self._ndim and chunk.shape[-2] == self._F, (tuple(chunk.shape), self._ndim, self._F)
+        assert (chunk.shape[0] if chunk.dim() == 3 else 1) == self._B, (tuple(chunk.shape), self._B)
+        assert chunk.dtype == self._dtype and chunk.device == self._in_device, (chunk.dtype, chunk.device)
+        work = (chunk if chunk.dim() == 3 else chunk.unsqueeze(0)).detach().to(self._dev, non_blocking=True)
+        frame0 = self._n - self._hist.shape[-1]
+        window = torch.cat([self._hist, work], -1) if work.shape[-1] else self._hist
+        self._n += work.shape[-1]
+        return window, frame0
+
+    def _keep(self, window: torch.Tensor, k: int) -> None:
+        """Keep the last k frames of the window (all of them when it has fewer) for the next push."""
+        self._hist = window[..., window.shape[-1] - min(k, window.shape[-1]):].clone()
+
+    def _result(self, out: torch.Tensor) -> torch.Tensor:
+        """``out`` (B, ...) on the compute device as the caller gets it: without the batch dimension for 2-D chunks,
+        as a host copy for host chunks."""
+        if self._ndim == 2:
+            out = out[0]
+        return host_copy(out, self._pinned) if self._host else out
+
+    # ---- public ------------------------------------------------------------------------------------------------
+    def flush(self) -> torch.Tensor:
+        """What was not returned yet; closes the stream."""
+        self._check_open()
+        if self._n == 0:
+            raise RuntimeError(f"{type(self).__name__}.flush: no frame has been pushed")
+        out = self._last()
+        self._closed = True
+        self._plan = self._hist = None
+        return out
+
+
+class RTISIStream(_FrameStream):
     r"""RTISI-LA on a spectrogram that arrives a few frames at a time (a TTS or vocoder front end).
 
     ``RTISIStream(look_ahead, asymmetric_window, max_iter, alpha, **stft_kwargs)`` takes ``RTISI_LA``'s arguments
@@ -56,69 +153,29 @@ class RTISIStream:
 
     def __init__(self, look_ahead=-1, asymmetric_window=False, max_iter=25, alpha=0.99, **stft_kwargs):
         _rtisi_checks(None, max_iter, alpha, asymmetric_window, stft_kwargs)
+        super().__init__(stft_kwargs)
         self.look_ahead, self.asymmetric_window = int(look_ahead), bool(asymmetric_window)
         self.max_iter, self.alpha = int(max_iter), float(alpha)
-        self._stft_kwargs = stft_kwargs
-        self._n = 0                # frames pushed
         self._steps = 0            # outer steps run
         self._emitted = 0          # samples per signal returned
-        self._started = False
-        self._closed = False
 
-    # ---- set-up at the first push ---------------------------------------------------------------------------
     def _start(self, chunk: torch.Tensor) -> None:
-        self._ndim, self._F, self._dtype, self._in_device = chunk.dim(), chunk.shape[-2], chunk.dtype, chunk.device
-        self._host = not chunk.is_cuda
-        self._pinned = self._host and chunk.is_pinned()
-        work = chunk if chunk.dim() == 3 else chunk.unsqueeze(0)
-        self._B = work.shape[0]
-        self._dev = dev = compute_device(chunk)
-        # RTISI-LA never pads: a constant pad mode keeps short plans (flush of a few frames) valid for make_dims
-        shape_only = torch.empty(work.shape[:-1] + (0,), dtype=work.dtype, device=dev)
-        args = dataclasses.replace(args_helper(shape_only, **self._stft_kwargs), pad_mode="constant")
-        self._args = args
-        n, hop = args.n_fft, args.hop_length
-        K = (n - 1) // hop
-        self._LA = K if self.look_ahead < 0 else self.look_ahead
-        self._P = n // 2 if args.center else 0
-        # shortest plan whose envelope has head, interior and tail apart: (T0 - 1) * hop >= n_fft
-        self._T0 = K + 2
-        self._plan = StftPlan(args, self._T0, self._B, chunk.dtype, dev)
-        self._window = args.window.detach().to(device=dev, dtype=chunk.dtype).contiguous()
+        self._capture(chunk)
+        self._start_envelope(self._stft_kwargs)
+        a, dev = self._args, self._dev
+        n, hop = a.n_fft, a.hop_length
+        self._LA = (n - 1) // hop if self.look_ahead < 0 else self.look_ahead
+        self._window = a.window.detach().to(device=dev, dtype=chunk.dtype).contiguous()
         self._synth_coeff = float(hop / (self._window @ self._window))            # as RTISI_LA (methods.py:318)
         self._scratch = torch.empty(2 * n, dtype=chunk.dtype, device=dev)
-        nbytes = _ops.rtisi_state_bytes(self._scratch, n, hop, 1, self._B, args.normalized, args.onesided, self._LA)
+        nbytes = _ops.rtisi_state_bytes(self._scratch, n, hop, 1, self._B, a.normalized, a.onesided, self._LA)
         self._state = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-        self._hist = torch.empty(self._B, self._F, 0, dtype=chunk.dtype, device=dev)   # last LA frames pushed
         self._pending = torch.empty(self._B, 0, dtype=chunk.dtype, device=dev)         # computed, not yet returned
-        self._started = True
-
-    def _check_open(self) -> None:
-        if self._closed:
-            raise RuntimeError("RTISIStream: the stream was flushed and is closed")
 
     # ---- helpers -----------------------------------------------------------------------------------------------
-    def _length(self, n_frames: int) -> int:
-        """L(n): the reference's output length for n frames."""
-        a = self._args
-        return (n_frames - 1) * a.hop_length + a.n_fft - 2 * self._P
-
     def _block_end(self, step: int) -> int:
         """End of the samples finished by the steps before `step`."""
         return max(0, (step - self._LA) * self._args.hop_length - self._P)
-
-    def _inv_env_window(self, x0: int, length: int, total_frames: int = -1) -> torch.Tensor:
-        """1/envelope of samples [x0, x0 + length) of the signal (total_frames -1: not known yet), gathered from the
-        short plan, or from a plan of the whole signal when it has fewer than T0 frames."""
-        a = self._args
-        out = torch.empty(length, dtype=self._dtype, device=self._dev)
-        if 0 <= total_frames < self._T0:
-            plan = StftPlan(a, total_frames, self._B, self._dtype, self._dev)
-        else:
-            plan = self._plan
-        _ops.plan_inv_env_window(plan.buf, out, x0, total_frames, a.n_fft, a.hop_length, plan.T, a.center,
-                                 a.normalized, a.onesided)
-        return out
 
     def _run(self, mag_ext: torch.Tensor, frame0: int, step_end: int, final: bool):
         """Steps [self._steps, step_end) on magnitude frames [frame0, frame0 + mag_ext.shape[-1]); returns the
@@ -127,7 +184,7 @@ class RTISIStream:
         x0 = self._block_end(self._steps)
         x1 = self._block_end(step_end)
         if final:
-            L = max(0, self._length(self._n))
+            L = max(0, a.signal_length(self._n))
             x0, x1 = min(x0, L), L
         x = torch.empty(self._B, x1 - x0, dtype=self._dtype, device=self._dev)
         if final and x1 == x0:
@@ -149,16 +206,7 @@ class RTISIStream:
         out = avail[:, :take]
         self._pending = avail[:, take:].clone() if take < avail.shape[1] else avail[:, :0]
         self._emitted = upto
-        if self._ndim == 2:
-            out = out[0]
-        if not out.is_contiguous():
-            out = out.contiguous()
-        if not self._host:
-            return out
-        host = torch.empty(out.shape, dtype=out.dtype, pin_memory=self._pinned)
-        host.copy_(out, non_blocking=True)
-        torch.cuda.current_stream(self._dev).synchronize()
-        return host
+        return self._result(out.contiguous())
 
     # ---- public ------------------------------------------------------------------------------------------------
     def push(self, chunk: torch.Tensor) -> torch.Tensor:
@@ -167,41 +215,20 @@ class RTISIStream:
         if chunk.requires_grad:
             raise NotImplementedError("RTISIStream has no gradient path: use RTISI_LA for a differentiable inversion")
         _rtisi_checks(chunk, self.max_iter, self.alpha, self.asymmetric_window, self._stft_kwargs)
-        if not self._started:
-            self._start(chunk)
-        assert chunk.dim() == self._ndim and chunk.shape[-2] == self._F, (tuple(chunk.shape), self._ndim, self._F)
-        assert (chunk.shape[0] if chunk.dim() == 3 else 1) == self._B, (tuple(chunk.shape), self._B)
-        assert chunk.dtype == self._dtype and chunk.device == self._in_device, (chunk.dtype, chunk.device)
-        k = chunk.shape[-1]
-        work = (chunk if chunk.dim() == 3 else chunk.unsqueeze(0)).detach().to(self._dev, non_blocking=True)
-        frame0 = self._n - self._hist.shape[-1]
-        mag_ext = torch.cat([self._hist, work], -1) if k else self._hist
-        self._n += k
-        x = self._run(mag_ext, frame0, self._n, False) if k else self._pending[:, :0]
-        self._hist = mag_ext[..., mag_ext.shape[-1] - min(self._LA, mag_ext.shape[-1]):].clone()
+        mag_ext, frame0 = self._append(chunk)
+        x = self._run(mag_ext, frame0, self._n, False) if chunk.shape[-1] else self._pending[:, :0]
+        self._keep(mag_ext, self._LA)
         a = self._args
         return self._emit(x, emitted_samples(self._n, a.n_fft, a.hop_length, self._LA, a.center))
 
-    def flush(self) -> torch.Tensor:
-        """The samples not returned yet; closes the stream."""
-        self._check_open()
-        if self._n == 0:
-            raise RuntimeError("RTISIStream.flush: no frame has been pushed")
+    def _last(self) -> torch.Tensor:
         x = self._run(self._hist, self._n - self._hist.shape[-1], self._n + self._LA, True)
-        out = self._emit(x, max(0, self._length(self._n)))
-        self._closed = True
-        self._plan = self._state = self._hist = self._pending = self._scratch = None
+        out = self._emit(x, max(0, self._args.signal_length(self._n)))
+        self._state = self._pending = self._scratch = None
         return out
 
 
-def pghi_emitted_samples(n_frames: int, n_fft: int, hop: int, center: bool) -> int:
-    """E(n) = clamp((n - 1) * hop - P, 0, L(n)): the samples per signal a PGHIStream with ``output="waveform"`` has
-    returned once n frames have been pushed (P = n_fft // 2 when centred, L(n) = (n - 1) * hop + n_fft - 2P)."""
-    P = n_fft // 2 if center else 0
-    return max(0, min((n_frames - 1) * hop - P, (n_frames - 1) * hop + n_fft - 2 * P))
-
-
-class PGHIStream:
+class PGHIStream(_FrameStream):
     r"""PGHI on a spectrogram that arrives a few frames at a time: one frame of look-ahead, no iterations.
 
     ``PGHIStream(gamma=None, tol=1e-5, output="waveform", **stft_kwargs)``: ``gamma``, ``tol`` and ``stft_kwargs``
@@ -244,21 +271,13 @@ class PGHIStream:
             raise ValueError(f"PGHIStream: output={output!r} must be 'waveform' or 'spectrum'")
         if stft_kwargs.get("n_fft") is not None:
             _analysis(int(stft_kwargs["n_fft"]) // 2 + 1, stft_kwargs)        # refuse bad options before any frame
+        super().__init__(stft_kwargs)
         self.gamma, self.tol, self.output = gamma, float(tol), output
-        self._stft_kwargs = stft_kwargs
-        self._n = 0                # frames pushed
         self._final = 0            # frames final
-        self._started = False
-        self._closed = False
 
-    # ---- set-up at the first push ---------------------------------------------------------------------------
     def _start(self, chunk: torch.Tensor) -> None:
-        self._ndim, self._F, self._dtype, self._in_device = chunk.dim(), chunk.shape[-2], chunk.dtype, chunk.device
-        self._host = not chunk.is_cuda
-        self._B = chunk.shape[0] if chunk.dim() == 3 else 1
-        n_fft, hop, wl = _analysis(self._F, self._stft_kwargs)
+        n_fft, hop, wl = _analysis(chunk.shape[-2], self._stft_kwargs)
         gamma = 0.25645 * wl ** 2 if self.gamma is None else float(self.gamma)
-        self._an = (n_fft, hop, wl, gamma)
         if self.output == "waveform":
             if n_fft % 2:
                 raise NotImplementedError(f"PGHIStream: output='waveform' needs an even n_fft (got {n_fft}); "
@@ -266,36 +285,20 @@ class PGHIStream:
             if hop > wl:
                 raise NotImplementedError(f"PGHIStream: output='waveform' needs hop_length <= win_length "
                                           f"({hop} > {wl}): the envelope would vanish between frames")
-        self._dev = dev = compute_device(chunk)
+        self._capture(chunk)
+        self._an = (n_fft, hop, wl, gamma)
         self._state = torch.empty(_ops.pghi_stream_state_bytes(chunk.dtype, self._B, self._F), dtype=torch.uint8,
-                                  device=dev)
-        self._hist = torch.empty(self._B, self._F, 0, dtype=chunk.dtype, device=dev)     # frames [final - 1, n)
+                                  device=self._dev)
         if self.output == "waveform":
-            kw = {k: v for k, v in self._stft_kwargs.items() if k != "n_fft"}
-            shape_only = torch.empty(self._B, self._F, 0, dtype=chunk.dtype, device=dev)
-            # a constant pad mode keeps short plans valid for make_dims (as RTISIStream)
-            self._args = dataclasses.replace(args_helper(shape_only, **kw), pad_mode="constant")
-            self._P = self._args.pad
-            # shortest plan whose envelope has head, interior and tail apart: (T0 - 1) * hop >= n_fft
-            self._T0 = (n_fft - 1) // hop + 2
-            self._plan = StftPlan(self._args, self._T0, self._B, chunk.dtype, dev)
+            self._start_envelope({k: v for k, v in self._stft_kwargs.items() if k != "n_fft"})
             self._ola = None       # (frames, un-centred unit-envelope plan): plain windowed overlap-add
-            self._carry = torch.zeros(self._B, n_fft - hop, dtype=chunk.dtype, device=dev)
-        self._started = True
-
-    # 1/envelope of output samples [x0, x0 + length), from the T0-frame plan (or a plan of the whole signal when it has
-    # fewer frames): the same gather as RTISIStream's, on the same attributes
-    _inv_env_window = RTISIStream._inv_env_window
-
-    def _check_open(self) -> None:
-        if self._closed:
-            raise RuntimeError("PGHIStream: the stream was flushed and is closed")
+            self._carry = torch.zeros(self._B, n_fft - hop, dtype=chunk.dtype, device=self._dev)
 
     # ---- the steps ---------------------------------------------------------------------------------------------
     def _frames(self, window: torch.Tensor, frame0: int, n_final: int, final: bool) -> torch.Tensor:
         """Finalise frames [self._final, self._final + n_final) from magnitude rows frame0 + r: (B, n_final, F)."""
         n_fft, hop, wl, gamma = self._an
-        out = torch.empty(self._B, n_final, self._F, dtype=_CDT[self._dtype], device=self._dev)
+        out = torch.empty(self._B, n_final, self._F, dtype=_ops.CDT[self._dtype], device=self._dev)
         if n_final:                # nothing final yet (the window may even be empty)
             _ops.pghi_stream_direct(window, frame0, n_final, final, self._state, out, n_fft, hop, wl, gamma,
                                     self.tol)
@@ -309,9 +312,7 @@ class PGHIStream:
         T = max(k, self._T0)
         if self._ola is None or self._ola[0] != T:
             plan = StftPlan(dataclasses.replace(a, center=False), T, self._B, self._dtype, self._dev)
-            with torch.cuda.device(self._dev):
-                _lib.check(_lib.lib().specinv_plan_unit_envelope(plan.desc_ref, C.c_void_p(plan.buf.data_ptr()),
-                                                                 _ops._stream(plan.buf)), "plan_unit_envelope")
+            plan.set_unit_envelope()
             self._ola = (T, plan)
         plan = self._ola[1]
         if k < T:
@@ -341,13 +342,7 @@ class PGHIStream:
             out = self._samples(frames, first, final)
         else:
             out = torch.empty(self._B, 0, dtype=self._dtype, device=self._dev)
-        if self._ndim == 2:
-            out = out[0]
-        if not self._host:
-            return out
-        host = torch.empty(out.shape, dtype=out.dtype)
-        host.copy_(out)
-        return host
+        return self._result(out)
 
     # ---- public ------------------------------------------------------------------------------------------------
     def push(self, chunk: torch.Tensor) -> torch.Tensor:
@@ -357,31 +352,16 @@ class PGHIStream:
             raise NotImplementedError("PGHIStream has no gradient path: detach the magnitude")
         if chunk.is_complex():
             raise ValueError("PGHIStream: a chunk must be a real magnitude, not a complex spectrum")
-        if chunk.dtype not in _CDT:
+        if chunk.dtype not in _ops.CDT:
             raise NotImplementedError(f"PGHIStream: dtype {chunk.dtype} is not supported (float32 / float64 only)")
         if chunk.dim() not in (2, 3):
             raise ValueError(f"PGHIStream: a chunk must be (F, k) or (B, F, k), got shape {list(chunk.shape)}")
-        if not self._started:
-            self._start(chunk)
-        assert chunk.dim() == self._ndim and chunk.shape[-2] == self._F, (tuple(chunk.shape), self._ndim, self._F)
-        assert (chunk.shape[0] if chunk.dim() == 3 else 1) == self._B, (tuple(chunk.shape), self._B)
-        assert chunk.dtype == self._dtype and chunk.device == self._in_device, (chunk.dtype, chunk.device)
-        work = (chunk if chunk.dim() == 3 else chunk.unsqueeze(0)).detach().to(self._dev)
-        window = torch.cat([self._hist, work], -1) if work.shape[-1] else self._hist
-        frame0 = self._n - self._hist.shape[-1]
-        self._n += work.shape[-1]
-        n_final = max(0, self._n - 1 - self._final)
-        out = self._run(window, frame0, n_final, False)
-        keep = min(self._n - max(0, self._final - 1), window.shape[-1])
-        self._hist = window[..., window.shape[-1] - keep:].clone()
+        window, frame0 = self._append(chunk)
+        out = self._run(window, frame0, max(0, self._n - 1 - self._final), False)
+        self._keep(window, self._n - max(0, self._final - 1))      # frames [final - 1, n)
         return out
 
-    def flush(self) -> torch.Tensor:
-        """The frames or samples not returned yet; closes the stream."""
-        self._check_open()
-        if self._n == 0:
-            raise RuntimeError("PGHIStream.flush: no frame has been pushed")
+    def _last(self) -> torch.Tensor:
         out = self._run(self._hist, self._n - self._hist.shape[-1], self._n - self._final, True)
-        self._closed = True
-        self._state = self._hist = self._plan = self._ola = self._carry = None
+        self._state = self._ola = self._carry = None
         return out

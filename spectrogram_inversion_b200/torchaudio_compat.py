@@ -27,12 +27,10 @@ import torch
 from torch import Tensor
 
 from . import _lib, _ops
-from .engine import SplitSpec, StftPlan, compute_device
+from .engine import SplitSpec, StftPlan, compute_device, host_copy
 from .stft_args import StftArgs
 
 __all__ = ["griffinlim", "GriffinLim"]
-
-_CPLX = {torch.float32: torch.complex64, torch.float64: torch.complex128}
 
 
 def _check(shape, window: Optional[Tensor], n_fft: int, hop_length: int, win_length: int, n_iter: int,
@@ -94,13 +92,7 @@ class _Runner:
         """torch.istft's check: the window envelope over the output must not fall below 1e-11 (one host sync)."""
         if self.n_valid <= 0:
             return
-        p = self.plan
-        env = torch.empty(p.length, dtype=p.dtype, device=self.device)
-        with torch.cuda.device(self.device):
-            _ops._ok(_lib.lib().specinv_plan_envelope(p.desc_ref, _lib.C.c_void_p(p.buf.data_ptr()),
-                                                      _lib.C.c_void_p(env.data_ptr()),
-                                                      _lib.C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)),
-                     "plan_envelope", 0)
+        env = self.plan.envelope()
         low = float(env[self.P:self.P + self.n_valid].abs().min())
         if low < 1e-11:
             raise RuntimeError(f"istft(...): window overlap add min: {low:g} (below 1e-11): the window and hop leave "
@@ -176,7 +168,7 @@ def griffinlim(specgram: Tensor, window: Tensor, n_fft: int, hop_length: int, wi
     shape = specgram.size()
     specgram = specgram.reshape([-1] + list(shape[-2:]))
     specgram = specgram.pow(1 / power)
-    cdt = _CPLX.get(specgram.dtype)
+    cdt = _ops.CDT.get(specgram.dtype)
     if cdt is None:
         raise NotImplementedError(f"dtype {specgram.dtype} is not supported (float32 / float64 only)")
     if rand_init:
@@ -211,12 +203,7 @@ def griffinlim(specgram: Tensor, window: Tensor, n_fft: int, hop_length: int, wi
         cur ^= 1
     y = run.output(x[cur])
     y = y.reshape(shape[:-2] + y.shape[-1:])
-    if y.device == specgram.device:
-        return y
-    out = torch.empty(y.shape, dtype=y.dtype, pin_memory=specgram.is_pinned())
-    out.copy_(y, non_blocking=True)
-    torch.cuda.current_stream(y.device).synchronize()
-    return out
+    return y if y.device == specgram.device else host_copy(y, specgram.is_pinned())
 
 
 class GriffinLim(torch.nn.Module):
@@ -443,9 +430,4 @@ class InverseMelScale(torch.nn.Module):
         out = torch.empty(mel.shape[0], freq, time, dtype=mel.dtype, device=dev)
         _ops.mel_inverse_direct(P.to(dev), mel, out, f_lo, f_hi)
         out = out.view(shape[:-2] + (freq, time))
-        if dev == melspec.device:
-            return out
-        y = torch.empty(out.shape, dtype=out.dtype, pin_memory=melspec.is_pinned())
-        y.copy_(out, non_blocking=True)
-        torch.cuda.current_stream(dev).synchronize()
-        return y
+        return out if dev == melspec.device else host_copy(out, melspec.is_pinned())

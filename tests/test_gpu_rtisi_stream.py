@@ -150,11 +150,7 @@ def _full_inv_env(n_fft, hop, T, center, dtype):
     plan = StftPlan(args, T, 1, dtype, "cuda")
     out = torch.empty(plan.length, dtype=dtype, device="cuda")
     _ops.plan_inv_env_window(plan.buf, out, 0, T, n_fft, hop, T, center, False, True)   # the plan's own values
-    env = torch.empty_like(out)
-    from spectrogram_inversion_b200 import _lib
-    import ctypes as C
-    _lib.check(_lib.lib().specinv_plan_envelope(plan.desc_ref, C.c_void_p(plan.buf.data_ptr()),
-                                                C.c_void_p(env.data_ptr()), None), "plan_envelope")
+    env = plan.envelope()
     torch.cuda.synchronize()
     assert _same_bits(out, 1 / env)               # (an independent read of the same plan)
     return w, out
