@@ -7,7 +7,7 @@ from __future__ import annotations
 
 import math
 import os
-from dataclasses import dataclass
+from dataclasses import dataclass, replace
 from typing import Callable, List, Optional, Tuple
 
 import torch
@@ -17,15 +17,9 @@ from . import _lib, _ops
 from .stft_args import StftArgs
 
 
-def require_cuda() -> None:
-    if not torch.cuda.is_available():
-        raise RuntimeError("spectrogram_inversion_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
-    _lib.lib()
-
-
 def compute_device(t: torch.Tensor) -> torch.device:
     """CUDA tensors run in place; host tensors are staged through the current CUDA device."""
-    require_cuda()
+    _ops.require_cuda()
     return t.device if t.is_cuda else torch.device("cuda", torch.cuda.current_device())
 
 
@@ -53,11 +47,14 @@ class SplitSpec:
 
 
 class StftPlan:
-    """Twiddles, scaled windows and 1/envelope for one (stft args, T, B, dtype, device)."""
+    """Twiddles, scaled windows and 1/envelope for one (stft args, T, B, dtype, device).  With ``total_frames``: for
+    frames [frame_offset, frame_offset + T) of a longer signal, un-centred, with that signal's envelope."""
 
     def __init__(self, args: StftArgs, n_frames: int, batch: int, dtype: torch.dtype, device: torch.device,
-                 tables: bool = True):
-        require_cuda()
+                 tables: bool = True, frame_offset: int = 0, total_frames: Optional[int] = None):
+        _ops.require_cuda()
+        if total_frames is not None:
+            args = replace(args, center=False)
         if dtype not in _ops.CDT:
             raise NotImplementedError(f"dtype {dtype} is not supported (float32 / float64 only)")
         if args.pad_mode not in _lib.PAD_MODES:
@@ -76,17 +73,18 @@ class StftPlan:
         self.n_bins = args.n_bins
         self._k = (n, args.hop_length, args.center, self.pad_mode, args.normalized, args.onesided)
         self.buf = None
-        d = _lib.make_desc(n, args.hop_length, self.T, self.B, args.center, self.pad_mode, args.normalized,
-                           args.onesided, _ops._DT[dtype])
-        self.desc, self.desc_ref = d, _lib.C.byref(d)      # struct specinv_desc of this plan (kept alive here)
+        self.desc_ref = _ops.desc(dtype, n, args.hop_length, self.T, self.B, args.center, self.pad_mode,
+                                  args.normalized, args.onesided)
         if not tables:          # layout conversion / phase_init only
             return
-        nbytes = _lib.C.c_size_t(0)
-        _lib.check(_lib.lib().specinv_plan_bytes(_lib.C.byref(d), _lib.C.byref(nbytes)), "plan_bytes")
-        self.buf = torch.empty(nbytes.value, dtype=torch.uint8, device=device)
+        self.buf = torch.empty(_ops.plan_bytes(self.desc_ref), dtype=torch.uint8, device=device)
         window = args.window.detach().to(device=device, dtype=dtype).contiguous()
-        _ops.plan_init(self.buf, window, n, args.hop_length, self.T, self.B, args.center, self.pad_mode,
-                       args.normalized, args.onesided)
+        if total_frames is None:
+            _ops.plan_init(self.buf, window, n, args.hop_length, self.T, self.B, args.center, self.pad_mode,
+                           args.normalized, args.onesided)
+        else:
+            _ops.plan_init_ranged(self.buf, window, n, args.hop_length, self.T, self.B, args.normalized,
+                                  args.onesided, frame_offset, total_frames)
 
     # ---- buffers ---------------------------------------------------------------------------
     def empty_spec(self, real: bool = False) -> SplitSpec:
@@ -144,16 +142,12 @@ class StftPlan:
     def envelope(self) -> torch.Tensor:
         """The window envelope the ISTFT divides by, one value per sample of the plan's signal (``length``)."""
         env = torch.empty(self.length, dtype=self.dtype, device=self.device)
-        with torch.cuda.device(self.buf.device):
-            _lib.check(_lib.lib().specinv_plan_envelope(self.desc_ref, _ops._p(self.buf), _ops._p(env),
-                                                        _ops._stream(self.buf)), "plan_envelope")
+        _ops.plan_envelope(self.buf, self.desc_ref, env)
         return env
 
     def set_unit_envelope(self) -> None:
         """Make the envelope 1 everywhere, so that the plan's ISTFT is a plain windowed overlap-add."""
-        with torch.cuda.device(self.buf.device):
-            _lib.check(_lib.lib().specinv_plan_unit_envelope(self.desc_ref, _ops._p(self.buf), _ops._stream(self.buf)),
-                       "plan_unit_envelope")
+        _ops.plan_unit_envelope(self.buf, self.desc_ref)
 
 
 def spec_sums(a: SplitSpec, b: SplitSpec) -> torch.Tensor:
@@ -186,11 +180,11 @@ class _Solver:
         # even the smallest config GPU-bound (cfg1: 24 us of kernel per iteration).
         self._ptrs = [None, None]      # per ping-pong parity: (tensors, their device pointers)
 
-    def _launch_direct(self, what: str, tensors: tuple, coef: float, sums: torch.Tensor) -> None:
+    def _launch_direct(self, entry: str, tensors: tuple, coef: float, sums: torch.Tensor) -> None:
         c = self._ptrs[self.cur]
         if c is None or len(c[0]) != len(tensors) or any(a is not b for a, b in zip(c[0], tensors)):
             c = self._ptrs[self.cur] = (tensors, _ops.pointers(tensors))      # (re)built when a buffer was replaced
-        _ops.iter_direct(self._fn, what, self.plan.device, self.plan.desc_ref, c[1], coef,
+        _ops.iter_direct(entry, entry, self.plan.device, self.plan.desc_ref, c[1], coef,
                          sums.data_ptr() if sums.numel() else None)
 
     @property
@@ -236,15 +230,14 @@ class GriffinLimSolver(_Solver):
         # alpha = 0 is plain Griffin-Lim: q_n = STFT(x_{n-1}) needs no momentum state, so none is kept or moved
         self.plain = self.lr == 0
         self.q = None if self.plain else [C, C.like()]
-        self._fn = _lib.lib().specinv_gl_iter
         plan.istft(C, self.x[0])                          # methods.py:233
         # Small problems (B * T frames fit the SMs' shared memory): runs of iterations go through ONE persistent kernel
         # with the state resident on chip (csrc/specinv_resident.cu) instead of one launch per iteration.
         self._resident_ws = None
         if not self.plain and plan.dtype == torch.float32 and os.environ.get("SPECINV_RESIDENT", "1") != "0":
-            nbytes = _lib.C.c_size_t(0)
-            if _lib.lib().specinv_gl_run_workspace_bytes(plan.desc_ref, _lib.C.byref(nbytes)) == 0:
-                self._resident_ws = torch.empty(nbytes.value, dtype=torch.uint8, device=plan.device)
+            nbytes = _ops.gl_run_workspace_bytes(plan.desc_ref)
+            if nbytes is not None:
+                self._resident_ws = torch.empty(nbytes, dtype=torch.uint8, device=plan.device)
 
     def run_many(self, n: int, iter0: int, eva_iter: int, evaluate: bool = True) -> None:
         if self._resident_ws is None or n < 2:
@@ -252,14 +245,9 @@ class GriffinLimSolver(_Solver):
         p, i, o = self.plan, self.cur, self.cur ^ 1
         n_eval = sum(1 for k in range(iter0, iter0 + n) if evaluates(k, eva_iter)) if evaluate else 0
         sums = torch.zeros(2 * n_eval, dtype=torch.float64, device=p.device) if n_eval else None
-        stream = torch.cuda.current_stream(p.device).cuda_stream
-        with torch.cuda.device(p.device):
-            code = _lib.lib().specinv_gl_run(
-                p.desc_ref, p.buf.data_ptr(), self.x[i].data_ptr(), self.x[o].data_ptr(), self.q[i].main.data_ptr(),
-                self.q[i].nyq.data_ptr(), self.q[o].main.data_ptr(), self.q[o].nyq.data_ptr(), self.mag.main.data_ptr(),
-                self.mag.nyq.data_ptr(), self.lr, int(n), int(iter0), int(eva_iter),
-                sums.data_ptr() if sums is not None else None, self._resident_ws.data_ptr(), stream)
-        _ops._ok(code, "gl_run")
+        _ops.gl_run(p.desc_ref, (p.buf, self.x[i], self.x[o], self.q[i].main, self.q[i].nyq, self.q[o].main,
+                                 self.q[o].nyq, self.mag.main, self.mag.nyq), self.lr, n, iter0, eva_iter, sums,
+                    self._resident_ws)
         if sums is not None:
             self.sums.copy_(sums[-2:])
         self.cur ^= 1
@@ -269,12 +257,9 @@ class GriffinLimSolver(_Solver):
         """Raise if a CTA of the last persistent run timed out waiting for a neighbour (synchronises)."""
         if self._resident_ws is None:
             return
-        status = _lib.C.c_uint32(0)
-        with torch.cuda.device(self.plan.device):
-            _ops._ok(_lib.lib().specinv_gl_run_status(self.plan.desc_ref, self._resident_ws.data_ptr(), _lib.C.byref(status),
-                                                      torch.cuda.current_stream(self.plan.device).cuda_stream), "gl_run_status", 0)
-        if status.value:
-            raise RuntimeError(f"persistent Griffin-Lim kernel: neighbour wait timed out at iteration {status.value}")
+        status = _ops.gl_run_status(self.plan.desc_ref, self._resident_ws)
+        if status:
+            raise RuntimeError(f"persistent Griffin-Lim kernel: neighbour wait timed out at iteration {status}")
 
     def _launch(self, sums: torch.Tensor) -> None:
         p, i, o = self.plan, self.cur, self.cur ^ 1
@@ -296,7 +281,6 @@ class ADMMSolver(_Solver):
         self.rho = float(rho)
         self.X = [C, C.like()]
         self.U = [C.zeros_like(), C.like()]
-        self._fn = _lib.lib().specinv_admm_iter
         plan.istft(C, self.x[0])                          # methods.py:453
 
     def _launch(self, sums: torch.Tensor) -> None:

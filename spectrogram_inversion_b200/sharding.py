@@ -15,6 +15,7 @@ from typing import List, Optional, Tuple
 import torch
 import torch.distributed as dist
 
+from . import _ops
 from .engine import ADMMSolver, GriffinLimSolver, METRIC_NAMES, StftPlan, training_loop
 
 
@@ -94,29 +95,14 @@ class CudaRangeEngine:
     already divided by the global envelope -- partial sums of neighbouring ranks just add up."""
 
     def __init__(self, args, n_frames_local: int, batch: int, dtype, device, frame_offset: int, total_frames: int):
-        from dataclasses import replace
-        from . import _lib, _ops
-        self._ops = _ops
         self.args_global = args
-        local_args = replace(args, center=False)
-        self.plan = StftPlan(local_args, n_frames_local, batch, dtype, device, tables=False)
-        p = self.plan
-        d = _lib.make_desc(args.n_fft, args.hop_length, n_frames_local, batch, False, 0, args.normalized,
-                           args.onesided, _ops._DT[dtype])
-        nbytes = _lib.C.c_size_t(0)
-        _lib.check(_lib.lib().specinv_plan_bytes(_lib.C.byref(d), _lib.C.byref(nbytes)), "plan_bytes")
-        p.buf = torch.empty(nbytes.value, dtype=torch.uint8, device=device)
-        window = args.window.detach().to(device=device, dtype=dtype).contiguous()
-        _ops.plan_init_ranged(p.buf, window, args.n_fft, args.hop_length, n_frames_local, batch, args.normalized,
-                              args.onesided, frame_offset, total_frames)
+        self.plan = StftPlan(args, n_frames_local, batch, dtype, device, frame_offset=frame_offset,
+                             total_frames=total_frames)
         self.device, self.dtype = device, dtype
-        self.local_len = p.length
+        self.local_len = self.plan.length
         self.pad = args.pad
-        self.pad_mode = _lib.PAD_MODES[args.pad_mode]
         self.padded_offset = frame_offset * args.hop_length
         self.signal_len = args.signal_length(total_frames)
-        self._nosums = torch.empty(0, dtype=torch.float64, device=device)
-        self._gl_fn = _lib.lib().specinv_gl_iter
 
     # -- state -------------------------------------------------------------------------------------
     def pack(self, spec_local):
@@ -134,7 +120,7 @@ class CudaRangeEngine:
         F = p.n_bins
         pin = phase_in if phase_in is not None else torch.empty(0, dtype=torch.float64, device=self.device)
         pout = torch.empty(p.B, F, dtype=torch.float64, device=self.device)
-        self._ops.phase_init_ex(mag.main, mag.nyq, out.main, out.nyq, pin, pout, a.n_fft, a.hop_length, a.onesided)
+        _ops.phase_init_ex(mag.main, mag.nyq, out.main, out.nyq, pin, pout, a.n_fft, a.hop_length, a.onesided)
         return out, pout
 
     def mag_sum_sq(self, mag) -> float:
@@ -155,24 +141,18 @@ class CudaRangeEngine:
         # straight through ctypes like the single-GPU solvers (engine._Solver._launch_direct): at 8 ranks an iteration
         # is ~0.2 ms of kernel time, a torch.library dispatch (~45 us) per launch would show
         p = self.plan
-        ptrs = self._ops.pointers((p.buf, x_in, x_out, q_in.main, q_in.nyq, q_out.main, q_out.nyq, mag.main, mag.nyq))
-        self._ops.iter_direct(self._gl_fn, "gl_iter", self.device, p.desc_ref, ptrs, lr,
-                              sums.data_ptr() if sums is not None else None)
+        ptrs = _ops.pointers((p.buf, x_in, x_out, q_in.main, q_in.nyq, q_out.main, q_out.nyq, mag.main, mag.nyq))
+        _ops.iter_direct("gl_iter", "gl_iter", self.device, p.desc_ref, ptrs, lr,
+                         sums.data_ptr() if sums is not None else None)
 
     def new_sums(self):
         return torch.zeros(2, dtype=torch.float64, device=self.device)
 
     def halo_sum(self, left, right, out):
-        self._ops.halo_sum(left, right, out)
+        _ops.halo_sum(left, right, out)
 
     def fill_padding(self, x):
-        from . import _lib
-        C = _lib.C
-        with torch.cuda.device(self.device):
-            self._ops._ok(_lib.lib().specinv_fill_padding(
-                self._ops._DT[x.dtype], C.c_void_p(x.data_ptr()), x.stride(0), x.shape[0], int(self.padded_offset),
-                x.shape[1], int(self.pad), int(self.signal_len), int(self.pad_mode),
-                C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)), "fill_padding")
+        _ops.fill_padding_direct(x, self.padded_offset, self.pad, self.signal_len, self.plan.pad_mode)
 
 
 PEER_EXCHANGES = [0]      # halo exchanges done by the peer-memory kernel in this process (tests / bench look at it)
@@ -188,25 +168,17 @@ class PeerHalo:
     falls back to the NCCL send/recv exchange -- no rank is left waiting on a peer that took the other path."""
 
     def __init__(self, rows: int, ov: int, dtype, device, group, rank: int, world: int):
-        import ctypes as C
-        from . import _lib, _ops
-        self._lib, self._C = _lib, C
-        self.dt = _ops._DT[dtype]
-        self.rows, self.ov, self.device, self.seq = rows, ov, device, 0
-        self.area, self.peers = None, [C.c_void_p(), C.c_void_p()]
+        self.dtype, self.rows, self.ov, self.device, self.seq = dtype, rows, ov, device, 0
+        self.area, self.peers = None, [None, None]
         self.error = None
-        L = _lib.lib()
-        handle = C.create_string_buffer(64)
+        handle = bytes(64)
         try:
             with torch.cuda.device(device):
-                nbytes = L.specinv_halo_area_bytes(self.dt, rows, ov)
-                area = C.c_void_p()
-                _lib.check(L.specinv_ipc_alloc(nbytes, C.byref(area), handle), "ipc_alloc")
-                self.area = area
+                self.area, handle = _ops.ipc_alloc_halo_area(dtype, rows, ov)
         except Exception as ex:            # keep going: the other ranks are waiting in the all_gather below
             self.error = ex
         infos = [None] * world
-        dist.all_gather_object(infos, (bytes(handle.raw), torch.cuda.current_device(), self.error is None), group=group)
+        dist.all_gather_object(infos, (handle, torch.cuda.current_device(), self.error is None), group=group)
         if self.error is None and not all(ok for _, _, ok in infos):
             self.error = RuntimeError("a peer rank could not allocate its halo area")
         if self.error is None:
@@ -221,8 +193,7 @@ class PeerHalo:
                         # cudaIpcOpenMemHandle then decides)
                         if peer_dev != me and not torch.cuda.can_device_access_peer(me, peer_dev):
                             raise RuntimeError(f"cuda:{me} cannot access its neighbour cuda:{peer_dev} (no P2P)")
-                        _lib.check(L.specinv_ipc_open(C.create_string_buffer(infos[r][0], 64), C.byref(self.peers[side])),
-                                   "ipc_open")
+                        self.peers[side] = _ops.ipc_open(infos[r][0])
             except Exception as ex:
                 self.error = ex
 
@@ -241,42 +212,26 @@ class PeerHalo:
         return None
 
     def exchange(self, x: torch.Tensor) -> None:
-        C, L = self._C, self._lib.lib()
         self.seq += 1
         PEER_EXCHANGES[0] += 1
-        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        with torch.cuda.device(self.device):
-            self._lib.check(L.specinv_halo_exchange(self.dt, C.c_void_p(x.data_ptr()), x.stride(0), self.rows, x.shape[1],
-                                                    self.ov, self.area, self.peers[0], self.peers[1], self.seq, stream),
-                            "halo_exchange")
+        _ops.halo_exchange(x, self.rows, self.ov, self.area, self.peers[0], self.peers[1], self.seq)
 
     def check(self) -> None:
         """Raise when an exchange timed out waiting for a neighbour (synchronises the current stream; called where
         the host waits anyway: evaluations and the end of the run)."""
-        C, L = self._C, self._lib.lib()
         if self.area is None:
             return
-        status = C.c_uint32(0)
-        stream = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-        with torch.cuda.device(self.device):
-            self._lib.check(L.specinv_halo_status(self.dt, self.area, self.rows, self.ov, C.byref(status), stream),
-                            "halo_status")
-        if status.value:
-            raise RuntimeError(f"halo exchange {status.value} timed out waiting for a neighbouring rank "
+        status = _ops.halo_status(self.device, self.dtype, self.area, self.rows, self.ov)
+        if status:
+            raise RuntimeError(f"halo exchange {status} timed out waiting for a neighbouring rank "
                                "(SPECINV_P2P_TIMEOUT_MS); the result is incomplete")
 
     def close(self) -> None:
         if getattr(self, "area", None) is None and not any(bool(p) for p in getattr(self, "peers", [])):
             return
-        L = self._lib.lib()
         torch.cuda.synchronize(self.device)
-        for i, p in enumerate(self.peers):
-            if p:
-                L.specinv_ipc_close(p)
-                self.peers[i] = self._C.c_void_p()
-        if self.area is not None:
-            L.specinv_ipc_free(self.area)
-        self.area = None
+        _ops.ipc_release(self.peers, self.area)
+        self.area, self.peers = None, [None, None]
 
     def __del__(self):
         try:

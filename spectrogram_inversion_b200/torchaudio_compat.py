@@ -26,7 +26,7 @@ from typing import Callable, Optional, Tuple
 import torch
 from torch import Tensor
 
-from . import _lib, _ops
+from . import _ops
 from .engine import SplitSpec, StftPlan, compute_device, host_copy
 from .stft_args import StftArgs
 
@@ -67,26 +67,17 @@ def _check(shape, window: Optional[Tensor], n_fft: int, hop_length: int, win_len
 
 
 class _Runner:
-    """Buffers and launches of one call: the centred plan (``length`` None), or one un-centred frame range that holds
-    the whole reflect-padded signal (``sharding.CudaRangeEngine`` with frame_offset 0, total_frames T) whose padding
-    is re-created from ``length`` before every STFT."""
+    """Buffers and launches of one call: the centred plan (``length`` None), or the un-centred frame range (0, T) that
+    holds the whole reflect-padded signal, whose padding is re-created around ``length`` samples before every STFT."""
 
     def __init__(self, args: StftArgs, B: int, T: int, dtype: torch.dtype, dev: torch.device, length: Optional[int]):
         self.args, self.length, self.device = args, length, dev
-        if length is None:
-            self.engine = None
-            self.plan = StftPlan(args, T, B, dtype, dev)
-        else:
-            from .sharding import CudaRangeEngine
-            self.engine = CudaRangeEngine(args, T, B, dtype, dev, 0, T)
-            self.engine.signal_len = length        # fill_padding mirrors around the caller's length
-            self.plan = self.engine.plan
+        self.plan = StftPlan(args, T, B, dtype, dev, total_frames=None if length is None else T)
         self.P = 0 if length is None else args.pad      # buffer position of output sample 0
         # output samples [0, n_valid) come from the overlap-add; torch.istft zero-pads the rest (length > L0 + n_fft/2)
         L = self.plan.length
         self.out_len = L if length is None else length
         self.n_valid = min(self.out_len, L - self.P)
-        self._fn = _lib.lib().specinv_gl_rebuilt_iter
 
     def check_envelope(self) -> None:
         """torch.istft's check: the window envelope over the output must not fall below 1e-11 (one host sync)."""
@@ -107,15 +98,15 @@ class _Runner:
         ``s_in`` / ``s_out`` None (m == 0): plain Griffin-Lim, no state."""
         st = (None,) * 4 if s_in is None else (s_in.main, s_in.nyq, s_out.main, s_out.nyq)
         ptrs = _ops.pointers((self.plan.buf, x_in, x_out, *st, mag.main, mag.nyq))
-        _ops.iter_direct(self._fn, "gl_rebuilt_iter", self.device, self.plan.desc_ref, ptrs, float(m),
+        _ops.iter_direct("gl_rebuilt_iter", "gl_rebuilt_iter", self.device, self.plan.desc_ref, ptrs, float(m),
                          sums.data_ptr() if sums is not None else None)
 
     def restore_padding(self, x: Tensor) -> None:
-        if self.engine is not None:
-            self.engine.fill_padding(x)
+        if self.length is not None:
+            _ops.fill_padding_direct(x, 0, self.P, self.length, self.plan.pad_mode)
 
     def output(self, x: Tensor) -> Tensor:
-        if self.engine is None:
+        if self.length is None:
             return x
         out = torch.zeros(x.shape[0], self.out_len, dtype=x.dtype, device=x.device)
         if self.n_valid > 0:

@@ -40,6 +40,43 @@ def test_library_exports_every_declared_symbol(lib):
     assert handle.specinv_error_string(-2).decode().startswith("configuration not supported")
 
 
+def test_binding_signatures_match_the_header():
+    """Every prototype of include/specinv_b200.h against the restype / argtypes that _lib._declare gives it, type by
+    type: ctypes passes a wrongly declared argument without complaint, so only this check catches one."""
+    import ctypes as C
+    from types import SimpleNamespace
+    from spectrogram_inversion_b200 import _lib
+
+    class Stub:
+        def __getattr__(self, name):
+            fn = SimpleNamespace()
+            setattr(self, name, fn)
+            return fn
+
+    stub = Stub()
+    _lib._declare(stub)
+    types = {"int": C.c_int, "int64_t": C.c_int64, "size_t": C.c_size_t, "uint32_t": C.c_uint32, "double": C.c_double,
+             "const char*": C.c_char_p, "const specinv_desc*": C.POINTER(_lib.Desc), "void**": C.POINTER(C.c_void_p),
+             "int64_t*": C.POINTER(C.c_int64), "size_t*": C.POINTER(C.c_size_t), "uint32_t*": C.POINTER(C.c_uint32)}
+
+    def ctype(decl):
+        t = re.sub(r"\s*\*\s*", "*", " ".join(decl.split()))
+        return types[t] if t in types else C.c_void_p if t.endswith("*") else t
+
+    text = re.sub(r"/\*.*?\*/", "", open(os.path.join(ROOT, "include", "specinv_b200.h")).read(), flags=re.S)
+    protos = re.findall(r"([\w\s*]+?)\b(specinv_\w+)\s*\(([^)]*)\)\s*;", text)
+    assert sorted(name for _, name, _ in protos) == header_symbols()
+    for ret, name, params in protos:
+        fn = stub.__dict__.get(name)
+        assert fn is not None, f"{name} is not declared"
+        params = [p for p in (p.strip() for p in params.split(",")) if p and p != "void"]
+        want = [ctype(re.sub(r"\s*\b\w+$", "", p)) for p in params]
+        assert fn.restype is ctype(ret), (name, fn.restype, ret)
+        assert len(fn.argtypes) == len(want), (name, fn.argtypes, params)
+        for i, (got, w) in enumerate(zip(fn.argtypes, want)):
+            assert got is w, (name, i, params[i], got, w)
+
+
 def test_host_only_entry_points(lib):
     """specinv_signal_length / specinv_plan_bytes are pure host arithmetic: callable without a GPU."""
     import ctypes as C
